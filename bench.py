@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """PRMF hot-path benchmark (contract: see the task statement / DESIGN.md "Measurement").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|4|5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|4|5] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 One *step* = one outer iteration of `nmf_pathway` (reference script/prmf_runner.py:715-774) on the
@@ -19,6 +19,10 @@ the GPU path in this run and compared on rank 0 with the CPU reference on the sa
 across N.  `--impl reference` times the reference's own CPU implementation (the unmodified
 `prmf_runner.py` functions from `baseline/_ref` when that install travelled with the repo, else the oracle
 port) on all host cores.
+
+`--dump-outputs DIR` writes what the last timed step computed (objective parts, U, V, score tables, the
+candidates `restrict` kept, in order) as float64 .npy files; the inputs depend only on the arguments, so two
+builds can be compared output for output.
 """
 import os
 import sys
@@ -80,7 +84,14 @@ def parse_args():
     ap.add_argument("--cpu-inner-steps", type=int, default=2)
     ap.add_argument("--ref-budget-s", type=float, default=150.0,
                     help="--impl reference: wall-clock budget that sizes the bounded sample of each step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float64, "
+                         "at most 64 MB; U as a fixed, seeded row sample when it does not fit)")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     for key, val in CONFIGS[a.config].items():
         if getattr(a, key) is None:
             setattr(a, key, val)
@@ -166,6 +177,57 @@ def plant_signal(X, Gs, lo, m_global, n_plant=10):
 
 def digest(arr):
     return hashlib.sha256(np.ascontiguousarray(arr).tobytes()).hexdigest()[:16]
+
+
+# ------------------------------------------------------------------------------------------------
+# --dump-outputs: what the last timed step computed, so that two builds can be compared output for output
+# ------------------------------------------------------------------------------------------------
+DUMP_BYTES = 60 << 20             # below 64 MB with room for the .npy headers
+DUMP_SEED = 4321
+
+
+def dump_rows(m, k, other_bytes):
+    """Global rows of U (m x k, float64) to write beside `other_bytes` of other outputs: None for all of them, else a
+    sorted sample drawn from a fixed seed (the same rows for the same shape, whatever the number of ranks)."""
+    budget = DUMP_BYTES - other_bytes
+    row_bytes = 8 * k + 8                          # a row of U and its index in U_rows
+    if budget < row_bytes:
+        raise SystemExit("bench.py: --dump-outputs: V and the score tables alone exceed %d bytes" % DUMP_BYTES)
+    if m * 8 * k <= budget:
+        return None
+    rng = np.random.Generator(np.random.PCG64(DUMP_SEED))
+    return np.sort(rng.choice(m, size=budget // row_bytes, replace=False))
+
+
+def restrict_arrays(surv, k, P):
+    """`restrict`'s result {factor: [(pathway, score), ...]} as two k x P arrays: the 1-based position of each surviving
+    candidate in its factor's list (0: dropped), and its score.  The order counts: the next multinomial draw picks
+    from the list by position."""
+    position, scores = np.zeros((k, P)), np.zeros((k, P))
+    for kk, cands in surv.items():
+        for i, (p, s) in enumerate(cands):
+            position[kk, int(p)] = i + 1
+            scores[kk, int(p)] = s
+    return position, scores
+
+
+def dump_outputs(a, ctx, eng, lo, hi, last, P):
+    """The last timed outer iteration's outputs: the objective parts of its 10 inner steps, U and V after them, the
+    score tables and the candidates `restrict` kept.  Every rank takes part (U is gathered); rank 0 writes."""
+    parts, mass, qn, surv = last
+    U_local, V = eng.get_UV()
+    position, scores = restrict_arrays(surv, a.k, P)
+    out = {"obj_parts": parts[:, :5], "V": V, "score_mass": mass, "score_quad_norm": qn,
+           "restrict_position": position, "restrict_scores": scores}
+    rows = dump_rows(a.m, a.k, sum(np.asarray(v).nbytes for v in out.values()))
+    sel = np.arange(a.m) if rows is None else rows
+    out["U"] = ctx.all_gather_rows(U_local[sel[(sel >= lo) & (sel < hi)] - lo], len(sel))
+    if rows is not None:
+        out["U_rows"] = rows.astype(np.float64)
+    if ctx.rank == 0:
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        for name, arr in out.items():
+            np.save(os.path.join(a.dump_outputs, name + ".npy"), np.ascontiguousarray(arr, dtype=np.float64))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -467,9 +529,9 @@ def run_ours(a):
         # streaming while the host runs restrict and the multinomial draws (as prmf_b200.nmf_pathway does)
         parts, _, _, (mass, qn, _) = eng.block_end(MODULUS, want_scores=True, prefetch=True)
         t2 = time.perf_counter()
-        restrict_from_tables(mass, qn, full_cands)
+        surv = restrict_from_tables(mass, qn, full_cands)
         host_t[0] += (t1 - t0) + (time.perf_counter() - t2)
-        return parts
+        return parts, mass, qn, surv
 
     def sync_all():
         if ctx.world > 1:
@@ -496,13 +558,15 @@ def run_ours(a):
     host_t[0] = 0.0
     e0.record(stream)
     for _ in range(a.steps):
-        parts = outer_iteration()
+        last = outer_iteration()
     e1.record(stream)
     sync_all()
     host_ms = host_t[0] * 1e3 / a.steps      # sampling + set_active + scores + restrict per outer iteration
     ms = e0.elapsed_time(e1)
     launches = eng.launch_count - launches0
-    final_obj = float(parts[-1, 4])
+    final_obj = float(last[0][-1, 4])
+    if a.dump_outputs:
+        dump_outputs(a, ctx, eng, lo, hi, last, packed.P)
     # ---- the same K steps again with an event pair around every phase of every inner step (the per-kernel
     #      durations of the roofline; the event records cost a few %, so they are kept out of `value`) ----
     eng.kernel_times(reset=True)

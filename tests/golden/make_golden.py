@@ -197,6 +197,7 @@ def main():
     save_case("small_tradeoff", X4, nodelist4, Gs4, 3, tradeoff=0.5, max_iter=120)
     save_bigk()
     save_kernel_vectors()
+    save_side_by_side()
 
 
 def save_bigk():
@@ -204,6 +205,23 @@ def save_bigk():
     grid-wide Gram fold, separate objective launch) to the reference itself."""
     X5, nodelist5, Gs5 = synth.small_instance(m=120, n=400, k_true=3, n_pathways=30, pathway_size=16, seed=7)
     save_case("small_bigk", X5, nodelist5, Gs5, 20, max_iter=60)
+
+
+def save_side_by_side():
+    """What the reference's `nmf_pathway` returns (U, V, final objective, factor -> pathway map) on the instances of
+    tests/test_oracle_golden.py::test_oracle_vs_live_reference: k = 3, max_iter = 300, default gamma / delta."""
+    from make_golden_io import side_by_side_instance
+    R = ref_shim.load_reference()
+    for seed in (0, 1):
+        X, nodelist, Gs = side_by_side_instance(seed)
+        ref_shim.reset_globals(R)
+        np.random.seed(seed); random.seed(seed)
+        with contextlib.redirect_stdout(io.StringIO()), contextlib.redirect_stderr(io.StringIO()):
+            U, V, od = R.nmf_pathway(X.copy(), [G.copy() for G in Gs], nodelist=list(nodelist), k_latent=3, max_iter=300)
+        fmap = {str(k): [int(p) for p, _ in v] for k, v in od["latent_to_pathway_data"].items()}
+        np.savez_compressed(os.path.join(HERE, "side_by_side_seed%d.npz" % seed), U=U, V=V, obj=np.array(float(od["obj"])),
+                            final_map=np.array(json.dumps(fmap)))
+        print("side_by_side_seed%d          obj=%.10g map=%s" % (seed, od["obj"], fmap))
 
 
 
@@ -253,6 +271,10 @@ def save_cli_case():
 
 if __name__ == "__main__" and "--only-bigk" in sys.argv:
     save_bigk()
+    sys.exit(0)
+
+if __name__ == "__main__" and "--only-side-by-side" in sys.argv:
+    save_side_by_side()
     sys.exit(0)
 
 if __name__ == "__main__":

@@ -1,5 +1,12 @@
-"""Input-file writer shared by make_golden.py and tests/test_cli.py (no reference import)."""
+"""Inputs shared by make_golden.py and the tests (no reference import)."""
 import os
+
+
+def side_by_side_instance(seed):
+    """The instances tests/test_oracle_golden.py::test_oracle_vs_live_reference runs (seed 1 has weighted edges)."""
+    from prmf_b200 import synth
+    return synth.small_instance(m=30, n=150, k_true=3, n_pathways=14, pathway_size=16, seed=20 + seed,
+                                weighted=bool(seed))
 
 
 def write_cli_inputs(outdir, X, nodelist, Gs, header=False):

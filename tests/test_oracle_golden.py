@@ -8,7 +8,7 @@ import random
 import numpy as np
 import pytest
 
-from conftest import GOLDEN_CASES, load_golden
+from conftest import GOLDEN, GOLDEN_CASES, load_golden
 from oracle import prmf_oracle as O
 
 RTOL_OBJ = 1e-10      # per-inner-step objective parts
@@ -103,23 +103,31 @@ def _ref():
 
 @pytest.mark.parametrize("seed", [0, 1])
 def test_oracle_vs_live_reference(seed):
-    ref_shim = _ref()
-    import contextlib, io
-    from prmf_b200 import synth
-    R = ref_shim.load_reference()
-    X, nodelist, Gs = synth.small_instance(m=30, n=150, k_true=3, n_pathways=14, pathway_size=16,
-                                           seed=20 + seed, weighted=bool(seed))
-    ref_shim.reset_globals(R)
-    np.random.seed(seed); random.seed(seed)
-    with contextlib.redirect_stdout(io.StringIO()), contextlib.redirect_stderr(io.StringIO()):
-        Ur, Vr, odr = R.nmf_pathway(X.copy(), [G.copy() for G in Gs], nodelist=list(nodelist),
-                                    k_latent=3, max_iter=300)
-    ref_shim.reset_globals(R)
+    """The oracle against what the reference returns on two more instances (the weighted one without a tradeoff):
+    the fixture `make_golden.py --only-side-by-side` records from the reference, else the reference run here."""
+    import contextlib, io, json, os, sys
+    sys.path.insert(0, GOLDEN)
+    from make_golden_io import side_by_side_instance
+    X, nodelist, Gs = side_by_side_instance(seed)
+    fixture = os.path.join(GOLDEN, "side_by_side_seed%d.npz" % seed)
+    if os.path.exists(fixture):
+        z = np.load(fixture, allow_pickle=False)
+        Ur, Vr, obj_r, map_r = z["U"], z["V"], float(z["obj"]), json.loads(str(z["final_map"]))
+    else:
+        ref_shim = _ref()
+        R = ref_shim.load_reference()
+        ref_shim.reset_globals(R)
+        np.random.seed(seed); random.seed(seed)
+        with contextlib.redirect_stdout(io.StringIO()), contextlib.redirect_stderr(io.StringIO()):
+            Ur, Vr, odr = R.nmf_pathway(X.copy(), [G.copy() for G in Gs], nodelist=list(nodelist),
+                                        k_latent=3, max_iter=300)
+        ref_shim.reset_globals(R)
+        obj_r = odr["obj"]
+        map_r = {str(k): [int(p) for p, _ in v] for k, v in odr["latent_to_pathway_data"].items()}
     np.random.seed(seed); random.seed(seed)
     Uo, Vo, odo = O.nmf_pathway(X.copy(), [G.copy() for G in Gs], nodelist=list(nodelist),
                                 k_latent=3, max_iter=300)
     np.testing.assert_allclose(Uo, Ur, rtol=1e-7, atol=1e-12)
     np.testing.assert_allclose(Vo, Vr, rtol=1e-7, atol=1e-12)
-    np.testing.assert_allclose(odo["obj"], odr["obj"], rtol=1e-10)
-    assert ({k: [p for p, _ in v] for k, v in odo["latent_to_pathway_data"].items()} ==
-            {k: [p for p, _ in v] for k, v in odr["latent_to_pathway_data"].items()})
+    np.testing.assert_allclose(odo["obj"], obj_r, rtol=1e-10)
+    assert {str(k): [int(p) for p, _ in v] for k, v in odo["latent_to_pathway_data"].items()} == map_r
