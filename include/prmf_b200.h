@@ -190,6 +190,21 @@ int prmf_set_profiling(prmf_handle* h, int on);
  * of a fitted V to new samples (reference script/transfer_learning.R:108, B^T = Y^T Z (Z^T Z + l I)^-1) needs exactly
  * Y^T Z.  Sharded handles return their own row block. */
 int prmf_project(prmf_handle* h, double* A_local);
+/* X^T . U for the U last given to prmf_set_UV (n x k, row-major): the pass-2 stream of the inner step on its own.
+ * With U = ones it gives the column sums of X.  Single-rank handles only (PRMF_ERR_STATE otherwise). */
+int prmf_project_t(prmf_handle* h, double* B_out);
+/* For every column c of B: x_c = argmin_{x >= 0} || op(X) x - b_c ||_2 with op(X) = X^T (transpose != 0; b: n, x: m)
+ * or X (transpose == 0; b: m, x: n) -- scipy.optimize.nnls(op(X), b_c) for all k columns at once, sharing each pass
+ * over X (Lawson & Hanson's active-set method, the duals A^T (b - A x) from the X streams of the inner step).
+ * B_host / x_out row-major (rows x k), rnorm_out[k] = || op(X) x_c - b_c ||, status_out[k]: 1 converged, -1 maxiter
+ * reached (counted as scipy counts, default 3 * #unknowns when maxiter <= 0), -2 the passive set outgrew the device
+ * capacity (min(#equations, #unknowns, 1024) columns), -3 the Gram matrix of the passive columns lost positive
+ * definiteness.  iter_out[k] (may be NULL): the iterations of each problem as scipy counts them (one per outer
+ * iteration, including the last one that finds the optimum, and one per step back).  A problem with status -2 or -3 leaves a message in prmf_last_error; the call still returns PRMF_OK.
+ * Repeated calls return bitwise-identical results.  Needs X; fp64, single-rank handles only (PRMF_ERR_STATE otherwise).
+ * U and V of the handle are undefined afterwards: set them again before the next step. */
+int prmf_nnls_x(prmf_handle* h, int transpose, const double* B_host, int maxiter, double* x_out, double* rnorm_out,
+                int32_t* status_out, int32_t* iter_out);
 /* The library keeps the two large buffers of a destroyed handle (X and its transposed copy) for the next handle of the
  * same shape on the same device (allocating and freeing multi-GB buffers dominates a short solve otherwise); at most
  * 4 buffers / 24 GB are held.  PRMF_POOL=0 (environment) disables the cache; this call frees what is held. */

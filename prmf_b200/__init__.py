@@ -11,5 +11,6 @@ from .pathways import PackedPathways, pack_pathways  # noqa: F401
 from .engine import CudaEngine  # noqa: F401
 from .preprocess import quantile_transform  # noqa: F401
 from .cv import measure_cv_performance, nnls_rows  # noqa: F401
+from .manifold_init import nnls_x, pathway_init  # noqa: F401
 
 __version__ = "0.1.0"

@@ -50,6 +50,8 @@ SYMBOLS = {
     "prmf_kernel_times": (c_int, [_P, c_int, POINTER(c_double), POINTER(c_int64)]),
     "prmf_set_profiling": (c_int, [_P, c_int]),
     "prmf_project": (c_int, [_P, _P]),
+    "prmf_project_t": (c_int, [_P, _P]),
+    "prmf_nnls_x": (c_int, [_P, c_int, _P, c_int, _P, _P, _P, _P]),
     "prmf_release_pool": (c_int, []),
     "prmf_debug_inject_fault": (c_int, [_P, c_int]),
     "prmf_stream": (_P, [_P]),

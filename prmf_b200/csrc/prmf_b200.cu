@@ -25,6 +25,7 @@
 #include "fused.cuh"
 #include "tf32.cuh"
 #include "nccl_dyn.h"
+#include "nnls_init.cuh"
 
 using namespace prmf;
 
@@ -1276,6 +1277,36 @@ int store_tf32(prmf_handle* h, const T* X, int64_t ld, bool on_host) {
     return PRMF_OK;
 }
 
+// The Lawson-Hanson loop of prmf_nnls_x over a workspace laid out by the caller (wk).  W: the operand of the X stream
+// that computes the duals (V for A = X^T, pass 1; U for A = X, pass 2); its zero pad rows are left as they are.
+int nnls_loop(prmf_handle* h, int transpose, NnlsWork& wk, double* rnorm_dev, std::vector<int32_t>& status) {
+    const int k = wk.k;
+    double* W = transpose ? h->Vbuf[h->vcur] : h->U;
+    const double* part = transpose ? h->Apart : h->Bpart;
+    const int chunks = transpose ? a_chunks(h) : (h->use_tma ? h->tchunks : h->chunks);
+    const int64_t wcount = wk.nun * k;
+    const dim3 rgrid((unsigned)((wk.neq + kNnlsThreads - 1) / kNnlsThreads), (unsigned)k);
+    // every launch of nnls_step_kernel counts one iteration of each running problem, so the loop ends by maxiter + 1
+    for (int64_t round = 0; round <= (int64_t)wk.maxiter; ++round) {
+        nnls_resid_kernel<<<rgrid, kNnlsThreads, 0, h->stream>>>(wk, W, 0);
+        LAUNCH_CHECK("nnls_resid_kernel");
+        int rc = transpose ? launch_xv(h) : launch_xtu(h);
+        if (rc) return rc;
+        sum_chunks_kernel<<<(unsigned)((wcount + 255) / 256), 256, 0, h->stream>>>(part, chunks, wcount, wk.w);
+        LAUNCH_CHECK("sum_chunks_kernel");
+        nnls_step_kernel<<<(unsigned)k, kNnlsThreads, 0, h->stream>>>(wk);
+        LAUNCH_CHECK("nnls_step_kernel");
+        CU(cudaMemcpyAsync(status.data(), wk.status, sizeof(int32_t) * k, cudaMemcpyDeviceToHost, h->stream));
+        CU(cudaStreamSynchronize(h->stream));
+        if (std::none_of(status.begin(), status.end(), [](int32_t s) { return s == kNnlsRunning; })) break;
+    }
+    nnls_resid_kernel<<<rgrid, kNnlsThreads, 0, h->stream>>>(wk, W, 1);
+    LAUNCH_CHECK("nnls_resid_kernel");
+    nnls_rnorm_kernel<<<(unsigned)k, kNnlsThreads, 0, h->stream>>>(W, wk.neq, k, rnorm_dev);
+    LAUNCH_CHECK("nnls_rnorm_kernel");
+    return PRMF_OK;
+}
+
 int finish_X(prmf_handle* h) {
     cancel_ahead(h);
     // transposed copy for pass 1, then ||X||^2 partial of this rank, all-reduced once
@@ -2144,6 +2175,116 @@ int prmf_project(prmf_handle* h, double* A_local) {
     LAUNCH_CHECK("sum_chunks_kernel");
     CU(cudaMemcpyAsync(A_local, dst, sizeof(double) * cnt, cudaMemcpyDeviceToHost, h->stream));
     CU(cudaStreamSynchronize(h->stream));
+    return PRMF_OK;
+}
+
+int prmf_project_t(prmf_handle* h, double* B_out) {
+    if (!h || !B_out) return PRMF_ERR_ARG;
+    if (!h->have_X) return fail(h, PRMF_ERR_STATE, "prmf_project_t needs X");
+    if (h->failed) return fail(h, PRMF_ERR_STATE, "the handle is in a failed state");
+    if (h->m != h->m_global) return fail(h, PRMF_ERR_STATE, "prmf_project_t needs a single-rank handle (m_local != m_global)");
+    CU(cudaSetDevice(h->device));
+    cancel_ahead(h);
+    int rc = launch_xtu(h);                            // the pass-2 stream of the inner step, without its V update
+    if (rc) return rc;
+    const int64_t cnt = h->n * h->k;
+    double* dst = h->Vbuf[h->vcur ^ 1];                // scratch: the second V buffer is free between steps
+    sum_chunks_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, h->stream>>>(
+        h->Bpart, h->x_tf32 ? h->tc_chunks2 : h->use_tma ? h->tchunks : h->chunks, cnt, dst);
+    LAUNCH_CHECK("sum_chunks_kernel");
+    CU(cudaMemcpyAsync(B_out, dst, sizeof(double) * cnt, cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    return PRMF_OK;
+}
+
+int prmf_nnls_x(prmf_handle* h, int transpose, const double* B_host, int maxiter, double* x_out, double* rnorm_out,
+                int32_t* status_out, int32_t* iter_out) {
+    if (!h || !B_host || !x_out || !rnorm_out || !status_out) return PRMF_ERR_ARG;
+    if (h->x_tf32) return fail(h, PRMF_ERR_STATE, "prmf_nnls_x needs an fp64 handle (X is stored as tf32)");
+    if (h->m != h->m_global) return fail(h, PRMF_ERR_STATE, "prmf_nnls_x needs a single-rank handle (m_local != m_global)");
+    if (!h->have_X) return fail(h, PRMF_ERR_STATE, "prmf_nnls_x needs X");
+    if (h->failed) return fail(h, PRMF_ERR_STATE, "the handle is in a failed state");
+    if (h->m == 0) return fail(h, PRMF_ERR_ARG, "prmf_nnls_x needs at least one sample");
+    CU(cudaSetDevice(h->device));
+    cancel_ahead(h);
+    h->have_UV = false;                                // U and V serve as the residual operand from here on
+
+    NnlsWork wk;
+    wk.k = h->k;
+    wk.neq = transpose ? h->n : h->m;
+    wk.nun = transpose ? h->m : h->n;
+    wk.Arows = transpose ? h->X : h->Xt;
+    wk.lda = transpose ? h->ldx : h->ldxt;
+    wk.cap = (int)std::min<int64_t>({wk.neq, wk.nun, (int64_t)kNnlsMaxPassive});
+    wk.maxiter = maxiter > 0 ? maxiter : (int)std::min<int64_t>(3 * wk.nun, INT32_MAX - 1);   // scipy: 3 * #unknowns
+    wk.tol = 10.0 * (double)std::max(wk.neq, wk.nun) * DBL_EPSILON;                          // 10 max(m, n) eps
+    const int k = wk.k;
+    const size_t cap = (size_t)wk.cap, kk = (size_t)k;
+    auto pad = [](size_t bytes) { return (bytes + 255) & ~(size_t)255; };
+    const size_t d = sizeof(double);
+    const size_t b_bt = pad(d * kk * wk.neq), b_w = pad(d * kk * wk.nun), b_g = pad(d * kk * cap * cap);
+    const size_t b_vec = pad(d * kk * cap), b_idx = pad(sizeof(int) * kk * cap), b_flag = pad(kk * wk.nun);
+    const size_t b_small = pad(sizeof(int) * kk), b_rn = pad(d * kk);
+    const size_t total = b_bt + b_w + 2 * b_g + 2 * b_vec + b_idx + b_flag + 3 * b_small + b_rn;
+    unsigned char* ws = nullptr;
+    cudaError_t ea = g_pool.alloc((void**)&ws, total, h->device);
+    if (ea != cudaSuccess) return fail(h, PRMF_ERR_NOMEM, "cudaMalloc of %zu bytes failed: %s", total, cudaGetErrorString(ea));
+    size_t off = 0;
+    auto take = [&](size_t bytes) { unsigned char* p = ws + off; off += bytes; return p; };
+    wk.Bt = (const double*)take(b_bt);
+    wk.w = (double*)take(b_w);
+    wk.G = (double*)take(b_g);
+    wk.L = (double*)take(b_g);
+    wk.atb = (double*)take(b_vec);
+    unsigned char* zero_from = ws + off;               // everything from here on starts at zero
+    wk.xP = (double*)take(b_vec);
+    wk.pidx = (int*)take(b_idx);
+    wk.flag = (int8_t*)take(b_flag);
+    wk.np = (int*)take(b_small);
+    wk.iter = (int*)take(b_small);
+    wk.status = (int*)take(b_small);
+    double* rnorm_dev = (double*)take(b_rn);
+
+    std::vector<double> Bt((size_t)k * wk.neq);
+    for (int64_t e = 0; e < wk.neq; ++e)
+        for (int c = 0; c < k; ++c) Bt[(size_t)c * wk.neq + e] = B_host[e * k + c];
+    std::vector<int32_t> status(k, kNnlsRunning), np_h(k), pidx_h(kk * cap);
+    std::vector<double> xP_h(kk * cap);
+    int rc = PRMF_OK;
+    cudaError_t e = cudaMemcpyAsync((void*)wk.Bt, Bt.data(), sizeof(double) * Bt.size(), cudaMemcpyHostToDevice, h->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(zero_from, 0, (size_t)(ws + total - zero_from), h->stream);
+    if (e != cudaSuccess) rc = fail(h, PRMF_ERR_CUDA, "prmf_nnls_x upload: %s", cudaGetErrorString(e));
+    if (!rc) rc = nnls_loop(h, transpose, wk, rnorm_dev, status);
+    if (!rc) {
+        e = cudaMemcpyAsync(np_h.data(), wk.np, sizeof(int32_t) * k, cudaMemcpyDeviceToHost, h->stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(pidx_h.data(), wk.pidx, sizeof(int32_t) * kk * cap, cudaMemcpyDeviceToHost, h->stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(xP_h.data(), wk.xP, sizeof(double) * kk * cap, cudaMemcpyDeviceToHost, h->stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(status_out, wk.status, sizeof(int32_t) * k, cudaMemcpyDeviceToHost, h->stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(rnorm_out, rnorm_dev, sizeof(double) * k, cudaMemcpyDeviceToHost, h->stream);
+        if (e == cudaSuccess && iter_out)
+            e = cudaMemcpyAsync(iter_out, wk.iter, sizeof(int32_t) * k, cudaMemcpyDeviceToHost, h->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+        if (e != cudaSuccess) rc = fail(h, PRMF_ERR_CUDA, "prmf_nnls_x read-back: %s", cudaGetErrorString(e));
+    } else {
+        cudaStreamSynchronize(h->stream);
+    }
+    g_pool.release(ws, total, h->device);
+    if (rc) return rc;
+    std::fill(x_out, x_out + wk.nun * k, 0.0);
+    for (int c = 0; c < k; ++c)
+        for (int q = 0; q < np_h[c]; ++q) x_out[(int64_t)pidx_h[c * cap + q] * k + c] = xP_h[c * cap + q];
+    h->err.clear();
+    for (int c = 0; c < k; ++c) {
+        if (status_out[c] == kNnlsCapacity) {
+            fail(h, PRMF_OK, "prmf_nnls_x: problem %d needs more than %d passive columns (the workspace capacity)", c,
+                 wk.cap);
+            break;
+        }
+        if (status_out[c] == kNnlsSingular) {
+            fail(h, PRMF_OK, "prmf_nnls_x: problem %d: the Gram matrix of its passive columns lost positive definiteness", c);
+            break;
+        }
+    }
     return PRMF_OK;
 }
 

@@ -175,6 +175,34 @@ class CudaEngine:
         self._ck(self.lib.prmf_project(self.h, _ptr(A)))
         return A
 
+    def project_t(self):
+        """X^T . U for the U last set (n x k): the pass-2 stream on its own (prmf_project_t)."""
+        B = np.empty((self.n, self.k))
+        self._ck(self.lib.prmf_project_t(self.h, _ptr(B)))
+        return B
+
+    def nnls(self, B, transpose, maxiter=None):
+        """scipy.optimize.nnls(op(X), B[:, c]) for every column c at once (prmf_nnls_x), op(X) = X^T when `transpose`
+        (B: n x k, x: m x k) and X otherwise (B: m x k, x: n x k).  Returns (x, rnorm[k], status[k]) with status 1
+        converged, -1 iteration limit, -2 passive-set capacity, -3 loss of positive definiteness, and iters[k], the
+        iterations of each problem as scipy counts them.  U and V of the engine are undefined afterwards."""
+        rows, cols = (self.n, self.m) if transpose else (self.m, self.n)
+        B = _f64(B)
+        if B.shape != (rows, self.k):
+            raise ValueError("B has shape %s, expected %s" % (B.shape, (rows, self.k)))
+        x = np.empty((cols, self.k))
+        rnorm = np.empty(self.k)
+        status = np.empty(self.k, dtype=np.int32)
+        iters = np.empty(self.k, dtype=np.int32)
+        self._ck(self.lib.prmf_nnls_x(self.h, 1 if transpose else 0, _ptr(B), int(maxiter or 0), _ptr(x), _ptr(rnorm),
+                                      _ptr(status), _ptr(iters)))
+        return x, rnorm, status, iters
+
+    @property
+    def last_error(self):
+        msg = self.lib.prmf_last_error(self.h)
+        return msg.decode() if msg else ""
+
     def snapshot_best(self):
         self._ck(self.lib.prmf_snapshot_best(self.h))
 

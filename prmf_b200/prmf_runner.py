@@ -22,6 +22,7 @@ from argparse import RawTextHelpFormatter
 import numpy as np
 
 from . import prmf_args
+from .manifold_init import pathway_init
 from .solver import nmf_pathway
 
 
@@ -100,33 +101,6 @@ def parse_pathways(manifold_fps, node_attribute="name"):
         G = nx.read_graphml(fp).to_undirected()
         pairs.append((relabel_nodes(G, node_attribute), fp))
     return pairs
-
-
-# ---- pathway-seeded initialisation (:272-334, :1023-1064) -------------------------------------------
-def pathway_to_vec(X, G, nodelist, rel_weight=5):
-    n_genes = len(nodelist)
-    v = np.zeros((n_genes,))
-    index = {node: i for i, node in enumerate(nodelist)}
-    for node in G.nodes():
-        v[index[node]] = 1
-    on = (v == 1)
-    off = np.invert(on)
-    v[off] = np.mean(X.transpose()[off], axis=1)
-    v[on] = (np.sum(v[off]) * rel_weight) / np.sum(on)
-    v = v.reshape((n_genes, 1))
-    return v / np.linalg.norm(v), on
-
-
-def nmf_init_u(X, v):
-    import scipy.optimize
-    u, residual = scipy.optimize.nnls(X.transpose(), v.flatten())
-    return (u / np.linalg.norm(u) ** 2).reshape((X.shape[0], 1)), residual
-
-
-def nmf_init_v(X, u):
-    import scipy.optimize
-    v, residual = scipy.optimize.nnls(X, u.flatten())
-    return (v / np.linalg.norm(v) ** 2).reshape(X.shape[1], 1), residual
 
 
 DESCRIPTION = """
@@ -233,7 +207,6 @@ def main(argv=None):
 
     U_init = V_init = None                                                       # :1023-1064
     if args.manifolds_init is not None:
-        X_dev, X = X, (X.cpu().numpy() if hasattr(X, "is_cuda") else X)          # the NNLS seeding runs on the host
         Gs_init = [fp_to_G[fp] for fp in args.manifolds_init]
         if len(args.manifolds_init) < args.k_latent:
             non_init = list(set(manifold_fps) - set(args.manifolds_init))
@@ -248,21 +221,12 @@ def main(argv=None):
             inds = np.random.choice(len(Gs_init), args.k_latent)
             init_fps = [args.manifolds_init[i] for i in inds]
             Gs_init = [Gs_init[i] for i in inds]
-        us, vs = [], []
-        for G in Gs_init:
-            v, on = pathway_to_vec(X, G, nodelist)
-            signal = v[on]
-            u, _ = nmf_init_u(X, v)
-            v_new, _ = nmf_init_v(X, u)
-            v_new[on] = signal
-            vs.append(v_new)
-            us.append(u)
-        V_init = np.concatenate(vs, axis=1)
-        U_init = np.concatenate(us, axis=1)
+        # pathway_to_vec -> nmf_init_u -> nmf_init_v for every init pathway (:272-334, :1023-1064), batched on the GPU
+        # against X where it already lives
+        U_init, V_init = pathway_init(X, Gs_init, nodelist)
         sys.stdout.write("Using the following manifolds for initialization:\n{}\n".format("\n".join(init_fps)))
         with open(os.path.join(args.outdir, "init_pathways.txt"), "w") as fh:
             fh.write("\n".join(init_fps))
-        X = X_dev
 
     # :1067 -- like the reference only gamma, tradeoff, k_latent, U_init, V_init and verbose are forwarded
     U, V, obj_data = nmf_pathway(X, Gs, nodelist=nodelist, gamma=args.gamma, tradeoff=tradeoff,
