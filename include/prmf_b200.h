@@ -88,7 +88,9 @@ int prmf_set_pathways(prmf_handle* h, int32_t P, const int64_t* path_ptr, const 
                       const int64_t* row_ptr, const int32_t* col_local, const double* w);
 
 /* Initial / current factors.  U is this rank's m_local x k block, V is n x k (replicated).  Either
- * pointer may be NULL to skip it.  U_init / V_init of nmf_pathway (:650-655) and its return value. */
+ * pointer may be NULL to skip it.  U_init / V_init of nmf_pathway (:650-655) and its return value.
+ * The library tracks U and V separately: calls that read one fail with PRMF_ERR_STATE until it has been set (again,
+ * after prmf_nnls_x). */
 int prmf_set_UV(prmf_handle* h, const double* U_local, const double* V);
 int prmf_get_UV(prmf_handle* h, double* U_local, double* V);
 
@@ -190,8 +192,9 @@ int prmf_set_profiling(prmf_handle* h, int on);
  * of a fitted V to new samples (reference script/transfer_learning.R:108, B^T = Y^T Z (Z^T Z + l I)^-1) needs exactly
  * Y^T Z.  Sharded handles return their own row block. */
 int prmf_project(prmf_handle* h, double* A_local);
-/* X^T . U for the U last given to prmf_set_UV (n x k, row-major): the pass-2 stream of the inner step on its own.
- * With U = ones it gives the column sums of X.  Single-rank handles only (PRMF_ERR_STATE otherwise). */
+/* X^T . U for the current U (n x k, row-major): the pass-2 stream of the inner step on its own.  The current U is the
+ * one last given to prmf_set_UV, or the result of the steps since.  With U = ones it gives the column sums of X.
+ * Single-rank handles only; PRMF_ERR_STATE as well when U was never set or prmf_nnls_x has used it since. */
 int prmf_project_t(prmf_handle* h, double* B_out);
 /* For every column c of B: x_c = argmin_{x >= 0} || op(X) x - b_c ||_2 with op(X) = X^T (transpose != 0; b: n, x: m)
  * or X (transpose == 0; b: m, x: n) -- scipy.optimize.nnls(op(X), b_c) for all k columns at once, sharing each pass
@@ -202,7 +205,8 @@ int prmf_project_t(prmf_handle* h, double* B_out);
  * definiteness.  iter_out[k] (may be NULL): the iterations of each problem as scipy counts them (one per outer
  * iteration, including the last one that finds the optimum, and one per step back).  A problem with status -2 or -3 leaves a message in prmf_last_error; the call still returns PRMF_OK.
  * Repeated calls return bitwise-identical results.  Needs X; fp64, single-rank handles only (PRMF_ERR_STATE otherwise).
- * U and V of the handle are undefined afterwards: set them again before the next step. */
+ * U and V of the handle are unset afterwards: calls that read them fail with PRMF_ERR_STATE until prmf_set_UV gives
+ * them again. */
 int prmf_nnls_x(prmf_handle* h, int transpose, const double* B_host, int maxiter, double* x_out, double* rnorm_out,
                 int32_t* status_out, int32_t* iter_out);
 /* The library keeps the two large buffers of a destroyed handle (X and its transposed copy) for the next handle of the

@@ -1067,8 +1067,9 @@ skinny_tma_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_total,
 // 256 consumer threads are split into FG factor groups of 256/FG threads.  A thread owns 4 columns of a
 // (1024/FG)-column panel and KT consecutive factors of its group, so the X tile is fetched from HBM once and
 // re-read from shared memory by every group -- at k = 64 the kernel is FP64-FMA bound (16 flop per byte of X),
-// not HBM bound.  k is a run-time value; factors >= k of the last group are computed on in-bounds garbage
-// and never written.
+// not HBM bound.  k is a run-time value: factors >= k are computed on in-bounds garbage and never written.  A group
+// reads W indices up to f0 + (RS-1) k + KT - 1, which for f0 < k is <= RS k + KT - 2, inside the RS k + KT doubles
+// of the W slot; groups with f0 >= k read group 0's columns instead.
 // ----------------------------------------------------------------------------------------------------
 template <int KT, int FG, int RS>
 __global__ void __launch_bounds__(kTmaThreads, 1)
@@ -1131,6 +1132,10 @@ skinny_tma_gen_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_to
     const int H = panel_w >> 2;
     const int fg = threadIdx.x / TG, t = threadIdx.x % TG;
     const int f0 = fg * KT;                                               // first factor of this thread
+    // groups whose factors all lie at or beyond k (k = 33..36, 65..84, 97..112) read group 0's columns, since their
+    // own can lie past the W slot; what they compute is never written.  A branch around their loop instead measured
+    // 1 % slower on the k = 64 stream, where no group is idle (B200, 1000 W).
+    const int fr = f0 < k ? f0 : 0;
     const bool active = t < H && (2 * t) < width;
     const bool active2 = t < H && (2 * (t + H)) < width;
     double acc[4][KT];
@@ -1144,7 +1149,7 @@ skinny_tma_gen_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_to
         const int rows = (int)min((int64_t)RS, rend - (rbeg + (int64_t)it * RS));
         mbar_wait(&full_bar[s2], phase);
         const unsigned char* sx = smem_raw + (size_t)s2 * stage_bytes;
-        const double* sw = reinterpret_cast<const double*>(sx + x_stage_bytes) + f0;
+        const double* sw = reinterpret_cast<const double*>(sx + x_stage_bytes) + fr;
         for (int r = 0; r < rows; ++r) {
             const double2* xrow = reinterpret_cast<const double2*>(sx + (size_t)r * panel_w * 8);
             const double2 xa = active ? xrow[t] : make_double2(0.0, 0.0);

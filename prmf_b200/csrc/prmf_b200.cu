@@ -151,7 +151,7 @@ struct prmf_handle {
     double* as_f64 = nullptr;                 // [diag_coef | off_coef]
     int64_t* as_off = nullptr;                // doff[k+1] | eoff[k+1] on the device
     std::vector<int64_t> row_ptr_host;
-    bool have_X = false, have_UV = false, have_pw = false, have_active = false, pos_dirty = true;
+    bool have_X = false, have_U = false, have_V = false, have_pw = false, have_active = false, pos_dirty = true;
     std::vector<int32_t> active_host;
 
     // pathways
@@ -936,7 +936,7 @@ void cancel_ahead(prmf_handle* h) {
 
 int prefetch_pass1(prmf_handle* h) {
     if (h->ahead || h->profiling || h->use_fused || h->m == 0) return PRMF_OK;
-    if (!h->have_X || !h->have_UV) return PRMF_OK;
+    if (!h->have_X || !h->have_U || !h->have_V) return PRMF_OK;
     int rc = 0;
     if (h->failed) return PRMF_OK;
     if (block_path(h)) {
@@ -1001,7 +1001,7 @@ void harvest_events(prmf_handle* h) {
 }
 
 int enqueue_steps(prmf_handle* h, int n_steps, double gamma, double delta, double tradeoff) {
-    if (!h->have_X || !h->have_UV || !h->have_pw || !h->have_active)
+    if (!h->have_X || !h->have_U || !h->have_V || !h->have_pw || !h->have_active)
         return fail(h, PRMF_ERR_STATE, "prmf_step needs X, U/V, pathways and the active set first");
     if (n_steps <= 0) return fail(h, PRMF_ERR_ARG, "n_steps must be positive");
     if (h->failed) return fail(h, PRMF_ERR_STATE, "the handle is in a failed state (an earlier launch failed or a device wait expired)");
@@ -1841,7 +1841,8 @@ int prmf_set_UV(prmf_handle* h, const double* U_local, const double* V) {
         if (h->x_tf32 && (rc = refresh_wt(h, h->Vbuf[h->vcur], h->n, h->Vt32, h->ldx32))) return rc;
     }
     CU(cudaStreamSynchronize(h->stream));
-    if (V) h->have_UV = true;
+    if (U_local || h->m == 0) h->have_U = true;          // a handle without rows has no U to set
+    if (V) h->have_V = true;
     return PRMF_OK;
 }
 
@@ -1889,7 +1890,7 @@ int prmf_step(prmf_handle* h, int n_steps, double gamma, double delta, double tr
 
 int prmf_scores(prmf_handle* h, double* mass, double* quad_norm, double* quad_raw) {
     if (!h) return PRMF_ERR_ARG;
-    if (!h->have_pw || !h->have_UV) return fail(h, PRMF_ERR_STATE, "prmf_scores needs pathways and V");
+    if (!h->have_pw || !h->have_V) return fail(h, PRMF_ERR_STATE, "prmf_scores needs pathways and V");
     CU(cudaSetDevice(h->device));
     const size_t cnt = (size_t)h->k * h->pw.P;
     double* d = h->scores_buf;
@@ -1908,7 +1909,7 @@ int prmf_block_end(prmf_handle* h, int n_steps, double* obj_parts, double* gamma
     CU(cudaSetDevice(h->device));
     if (n_steps > h->obj_capacity) return fail(h, PRMF_ERR_ARG, "prmf_block_end: more steps than were run");
     if (want_scores) {
-        if (!h->have_pw || !h->have_UV) return fail(h, PRMF_ERR_STATE, "prmf_block_end needs pathways and V for the scores");
+        if (!h->have_pw || !h->have_V) return fail(h, PRMF_ERR_STATE, "prmf_block_end needs pathways and V for the scores");
         const size_t cnt = (size_t)h->k * h->pw.P;
         double* d = h->scores_buf;
         int rc_s = launch_scores(h);
@@ -1965,7 +1966,7 @@ int prmf_restore_best(prmf_handle* h) {
 
 int prmf_residual_sq(prmf_handle* h, double* out) {
     if (!h || !out) return PRMF_ERR_ARG;
-    if (!h->have_X || !h->have_UV) return fail(h, PRMF_ERR_STATE, "prmf_residual_sq needs X and U/V");
+    if (!h->have_X || !h->have_U || !h->have_V) return fail(h, PRMF_ERR_STATE, "prmf_residual_sq needs X and U/V");
     CU(cudaSetDevice(h->device));
     const int blocks = h->sm_count * 4;
     double* d = nullptr;
@@ -1995,7 +1996,7 @@ int prmf_residual_sq(prmf_handle* h, double* out) {
 
 int prmf_objective(prmf_handle* h, double gamma, double delta, double* out) {
     if (!h || !out) return PRMF_ERR_ARG;
-    if (!h->have_X || !h->have_UV || !h->have_pw || !h->have_active)
+    if (!h->have_X || !h->have_U || !h->have_V || !h->have_pw || !h->have_active)
         return fail(h, PRMF_ERR_STATE, "prmf_objective needs X, U/V, pathways and the active set");
     CU(cudaSetDevice(h->device));
     int rc = ensure_pos(h);
@@ -2162,7 +2163,7 @@ int prmf_kernel_times(prmf_handle* h, int reset, double* phase_ms, int64_t* phas
 
 int prmf_project(prmf_handle* h, double* A_local) {
     if (!h || (!A_local && h->m > 0)) return PRMF_ERR_ARG;
-    if (!h->have_X || !h->have_UV) return fail(h, PRMF_ERR_STATE, "prmf_project needs X and V");
+    if (!h->have_X || !h->have_V) return fail(h, PRMF_ERR_STATE, "prmf_project needs X and V");
     if (h->failed) return fail(h, PRMF_ERR_STATE, "the handle is in a failed state");
     CU(cudaSetDevice(h->device));
     if (h->m == 0) return PRMF_OK;
@@ -2180,7 +2181,7 @@ int prmf_project(prmf_handle* h, double* A_local) {
 
 int prmf_project_t(prmf_handle* h, double* B_out) {
     if (!h || !B_out) return PRMF_ERR_ARG;
-    if (!h->have_X) return fail(h, PRMF_ERR_STATE, "prmf_project_t needs X");
+    if (!h->have_X || !h->have_U) return fail(h, PRMF_ERR_STATE, "prmf_project_t needs X and U");
     if (h->failed) return fail(h, PRMF_ERR_STATE, "the handle is in a failed state");
     if (h->m != h->m_global) return fail(h, PRMF_ERR_STATE, "prmf_project_t needs a single-rank handle (m_local != m_global)");
     CU(cudaSetDevice(h->device));
@@ -2207,7 +2208,7 @@ int prmf_nnls_x(prmf_handle* h, int transpose, const double* B_host, int maxiter
     if (h->m == 0) return fail(h, PRMF_ERR_ARG, "prmf_nnls_x needs at least one sample");
     CU(cudaSetDevice(h->device));
     cancel_ahead(h);
-    h->have_UV = false;                                // U and V serve as the residual operand from here on
+    h->have_U = h->have_V = false;                     // U and V serve as the residual operand from here on
 
     NnlsWork wk;
     wk.k = h->k;

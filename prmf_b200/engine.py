@@ -176,7 +176,7 @@ class CudaEngine:
         return A
 
     def project_t(self):
-        """X^T . U for the U last set (n x k): the pass-2 stream on its own (prmf_project_t)."""
+        """X^T . U for the current U (n x k): the pass-2 stream on its own (prmf_project_t)."""
         B = np.empty((self.n, self.k))
         self._ck(self.lib.prmf_project_t(self.h, _ptr(B)))
         return B
@@ -185,7 +185,8 @@ class CudaEngine:
         """scipy.optimize.nnls(op(X), B[:, c]) for every column c at once (prmf_nnls_x), op(X) = X^T when `transpose`
         (B: n x k, x: m x k) and X otherwise (B: m x k, x: n x k).  Returns (x, rnorm[k], status[k]) with status 1
         converged, -1 iteration limit, -2 passive-set capacity, -3 loss of positive definiteness, and iters[k], the
-        iterations of each problem as scipy counts them.  U and V of the engine are undefined afterwards."""
+        iterations of each problem as scipy counts them.  U and V of the engine are unset afterwards: steps and
+        projections raise until `set_UV` gives them again."""
         rows, cols = (self.n, self.m) if transpose else (self.m, self.n)
         B = _f64(B)
         if B.shape != (rows, self.k):

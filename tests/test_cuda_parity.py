@@ -51,6 +51,13 @@ def _instance(m, n, k, P, seed, weighted=False, psize=12):
     (64, 2100, 64, 6),     # BASELINE config 4's k: 4 groups x 16, several panels
     (33, 150, 100, 4),     # 8 groups, ragged last group
     (24, 140, 128, 3),     # BASELINE config 5's k
+    (45, 190, 2, 4),       # k = 2, 4, 5, 8, 9: the fused tails of those K
+    (80, 333, 4, 6),
+    (51, 260, 5, 7),
+    (150, 700, 8, 9),
+    (66, 1100, 9, 8),
+    (90, 400, 27, 6),      # skinny_tma_gen_kernel<16,2>, tiled tails at 2 columns per thread
+    (60, 500, 80, 5),      # skinny_tma_gen_kernel<12,8> with two idle factor groups, tiled tails at 8
 ])
 @pytest.mark.parametrize("weighted", [False, True])
 def test_inner_steps_match_oracle(m, n, k, P, weighted):
@@ -276,7 +283,8 @@ def test_speculative_pass_is_bitwise_neutral(k):
 
 # ---- the launch-structure switches must not change results ----------------------------------------------
 @pytest.mark.parametrize("env", [{"PRMF_EPI": "0"}, {"PRMF_BLOCK": "1"}, {"PRMF_TMA": "0"}])
-@pytest.mark.parametrize("m,n,k,P", [(200, 517, 10, 12), (1000, 6750, 10, 20), (37, 131, 3, 5)])
+@pytest.mark.parametrize("m,n,k,P", [(200, 517, 10, 12), (1000, 6750, 10, 20), (37, 131, 3, 5)] +
+                         [(48, 97 + 10 * k, k, 6) for k in (1, 2, 4, 5, 6, 7, 8, 9)])    # every K of the three paths
 def test_launch_structure_switches(monkeypatch, env, m, n, k, P):
     """PRMF_EPI=0: separate U / V-update launches instead of the fused tails (the path of ranks without rows);
     PRMF_BLOCK=1: the persistent step kernel (the default of sharded runs) on one GPU instead of two fused-tail launches
