@@ -15,7 +15,7 @@ LIB = os.path.join(HERE, "libprmf_b200.so")
 HEADER = os.path.join(HERE, "..", "include", "prmf_b200.h")
 # translation unit -> headers it depends on
 SOURCES = {
-    "prmf_b200.cu": ["kernels.cuh", "block_params.h", "fused.cuh", "tf32.cuh", "nccl_dyn.h", "nnls_init.cuh"],
+    "prmf_b200.cu": ["kernels.cuh", "block_params.h", "tf32.cuh", "nccl_dyn.h", "nnls_init.cuh"],
     "block.cu": ["kernels.cuh", "block_params.h", "block.cuh"],
     "preprocess.cu": [],
     "cv.cu": [],

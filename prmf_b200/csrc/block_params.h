@@ -6,7 +6,7 @@
 
 namespace prmf {
 
-constexpr int kBlkRS = 8;            // rows of M per ring stage (as skinny_tma_kernel<.,8,.>)
+constexpr int kBlkRS = kTmaRS;       // rows of M per ring stage, as in the X-stream kernels
 constexpr int kBlkRowsCap = 256;     // large shares (few chunks): rows per tile, K entries per thread, one staged array
 constexpr int kBlkTile = 85;         // small shares (many chunks): rows per tile, three staged arrays share the same scratch
 constexpr int kBlkPre = 51;          // largest pass-2 share the helper warp prefetches (five staged arrays share that scratch)

@@ -307,103 +307,21 @@ struct ActiveSet {
 };
 
 // ----------------------------------------------------------------------------------------------------
-// The X-stream kernel, used for BOTH passes:   Out[chunk][j][k0:k0+KT] = sum_{i in chunk} M[i][j] * W[i][k0:k0+KT]
+// The X-stream kernel, used for BOTH passes:   Out[chunk][j][0:KT] = sum_{i in chunk} M[i][j] * W[i][0:KT]   (KT == k)
 //   pass 1  (U_up_num = X.V, :420):        M = Xt (genes x samples, the transposed copy), W = V -> A partials
 //   pass 2  (V_up_num_recon = X^T.U, :424): M = X  (samples x genes),                     W = U -> B partials
-// M is row-major with leading dimension ldm (a multiple of 16 doubles, pad columns zero).  A thread owns 4
-// consecutive columns of M (two 128-bit streaming loads per row, 8 rows in flight) and KT accumulators for
-// each; the W row is the same for the whole block and is read from shared memory as a broadcast.  The grid
-// is (column panels) x (row chunks); per-chunk partials are summed in a fixed order by the consumer.
-// ----------------------------------------------------------------------------------------------------
-constexpr int kSkinnyRowsPerStage = 32;
-
-template <int KT>
-__global__ void __launch_bounds__(256, 2)
-skinny_tn_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_total, int64_t cols,
-                 const double* __restrict__ W, int k, int k0, int panel_w, int64_t rows_per_chunk,
-                 double* __restrict__ OutPart) {
-    __shared__ double sW[kSkinnyRowsPerStage][KT];
-    const int panel = blockIdx.x;
-    const int64_t chunk = blockIdx.y;
-    const int jl = threadIdx.x * 4;
-    const int64_t j0 = (int64_t)panel * panel_w + jl;
-    const bool active = (jl < panel_w) && (j0 < ldm);
-    const int64_t rbeg = chunk * rows_per_chunk;
-    const int64_t rend = min(rows_total, rbeg + rows_per_chunk);
-    double acc[4][KT];
-#pragma unroll
-    for (int g = 0; g < 4; ++g)
-#pragma unroll
-        for (int c = 0; c < KT; ++c) acc[g][c] = 0.0;
-    const double* xp = M + j0;
-    for (int64_t r0 = rbeg; r0 < rend; r0 += kSkinnyRowsPerStage) {
-        const int rows = (int)min((int64_t)kSkinnyRowsPerStage, rend - r0);
-        __syncthreads();
-        for (int e = threadIdx.x; e < rows * KT; e += blockDim.x) {
-            const int r = e / KT, c = e - r * KT;
-            sW[r][c] = W[(r0 + r) * k + k0 + c];
-        }
-        __syncthreads();
-        if (active) {
-            int r = 0;
-            for (; r + 4 <= rows; r += 4) {
-                double2 xa[4], xb[4];
-#pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    const double* p = xp + (r0 + r + q) * ldm;
-                    xa[q] = ld_stream(p);
-                    xb[q] = ld_stream(p + 2);
-                }
-#pragma unroll
-                for (int q = 0; q < 4; ++q)
-#pragma unroll
-                    for (int c = 0; c < KT; ++c) {
-                        const double u = sW[r + q][c];
-                        acc[0][c] = fma(xa[q].x, u, acc[0][c]);
-                        acc[1][c] = fma(xa[q].y, u, acc[1][c]);
-                        acc[2][c] = fma(xb[q].x, u, acc[2][c]);
-                        acc[3][c] = fma(xb[q].y, u, acc[3][c]);
-                    }
-            }
-            for (; r < rows; ++r) {
-                const double* p = xp + (r0 + r) * ldm;
-                const double2 xa = ld_stream(p), xb = ld_stream(p + 2);
-#pragma unroll
-                for (int c = 0; c < KT; ++c) {
-                    const double u = sW[r][c];
-                    acc[0][c] = fma(xa.x, u, acc[0][c]);
-                    acc[1][c] = fma(xa.y, u, acc[1][c]);
-                    acc[2][c] = fma(xb.x, u, acc[2][c]);
-                    acc[3][c] = fma(xb.y, u, acc[3][c]);
-                }
-            }
-        }
-    }
-    if (active) {
-#pragma unroll
-        for (int g = 0; g < 4; ++g) {
-            const int64_t j = j0 + g;
-            if (j < cols) {
-                double* out = OutPart + ((int64_t)chunk * cols + j) * k + k0;
-#pragma unroll
-                for (int c = 0; c < KT; ++c) out[c] = acc[g][c];
-            }
-        }
-    }
-}
-
-// ----------------------------------------------------------------------------------------------------
-// TMA version of the X-stream kernel (single factor tile, KT == k).  Same math and same output layout as
-// skinny_tn_kernel; the difference is how bytes move: a producer warp issues 1-D bulk async copies
-// (cp.async.bulk, SASS UBLKCP) of RS row pieces of M (<= 8 KB each, contiguous) plus the RS matching rows
-// of W per stage into a ring of `stages` shared-memory buffers; completion is tracked with mbarrier
-// transaction counts, and the 8 consumer warps release a buffer through an "empty" mbarrier.  Bytes in
-// flight per SM are set by the ring (>= 100 KB), not by registers, which is what the LDG version lacked
-// (ncu: long_scoreboard stalls, 24 % warps active, 84 % of the measured copy bandwidth).
+// M is row-major with leading dimension ldm (a multiple of 16 doubles, pad columns zero).  The grid is (column panels)
+// x (row chunks); per-chunk partials are summed in a fixed order by the consumer.  A producer warp issues 1-D bulk
+// async copies (cp.async.bulk, SASS UBLKCP) of RS row pieces of M (<= 8 KB each, contiguous) plus the RS matching rows
+// of W per stage into a ring of `stages` shared-memory buffers; completion is tracked with mbarrier transaction
+// counts, and the 8 consumer warps release a buffer through an "empty" mbarrier.  Bytes in flight per SM are set by
+// the ring (>= 100 KB), not by registers: a version that streamed M with ld.global stalled on long_scoreboard (ncu:
+// 24 % warps active) and reached 84 % of the measured copy bandwidth.
 // Thread t owns the double2 columns t and t + H of the panel (H = panel_w / 4), so shared-memory reads of a
 // warp are contiguous 512-byte runs (conflict free); W rows are broadcast reads.
 // W must be readable for RS rows past the last row of the chunk (the host pads U and V allocations).
 // ----------------------------------------------------------------------------------------------------
+constexpr int kTmaRS = 8;                  // rows of M per ring stage (the RS of every launched instantiation)
 constexpr int kTmaConsumerWarps = 8;
 constexpr int kTmaThreads = (kTmaConsumerWarps + 1) * 32;
 

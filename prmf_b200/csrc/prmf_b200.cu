@@ -1,13 +1,22 @@
-// libprmf_b200.so -- C ABI (include/prmf_b200.h) over the sm_100a kernels in kernels.cuh.
-// Host orchestration of one PRMF inner step (reference prmf_runner.py:419-449):
+// libprmf_b200.so -- C ABI (include/prmf_b200.h) over the sm_100a kernels in kernels.cuh, block.cuh and tf32.cuh.
+// Host orchestration of one PRMF inner step (reference prmf_runner.py:419-449).  Both passes over X are TMA X-stream
+// launches: skinny_tma_kernel<k,kTmaRS,EPI> at k <= 10, skinny_tma_gen_kernel<KT,FG,kTmaRS> at k > 10, or
+// tc_rowdot_kernel in tf32 mode.
 //
-//   skinny_tn_kernel    A partials = Xt^T.V            pass 1 over X (transposed copy)   (:420)
-//   u_update_kernel     U <- U*A/(U.Gv+U), Gu partials                                   (:421-422,:425)
-//   skinny_tn_kernel    B partials = X^T.U_new         pass 2 over X                     (:424)
-//   reduce_pack_kernel  red = [B | Gu | .]  (fixed-order sums)
-//   ncclAllReduce(red)                                 only with a communicator
-//   v_update_kernel     V_new (double-buffered), Gv/VB partials                          (:425-444)
-//   objective_kernel    Gv_new, recon/manifold/ignore/fro/obj, tradeoff                  (:336-372,:542-548)
+// k <= 10, fp64 (fused tails, launch_xv_epi / launch_xtu_epi):
+//   skinny_tma_kernel<k,8,1>   A partials = Xt^T.V, then U <- U*A/(U.Gv+U) and Gu in the last CTA of each panel   (:420-422)
+//   skinny_tma_kernel<k,8,2>   B partials = X^T.U_new, then V_new, Gv/VB partials                                 (:424-444)
+//   objective_(parts|deferred)_kernel   recon/manifold/ignore/fro/obj, per step or once per block                 (:336-372)
+//   sharded: the pass-2 tail packs for ncclAllReduce (EPI 3) or exchanges over NVLink (EPI 4); or the whole block
+//   of steps runs as one persistent launch (block_kernel<K>, block.cuh)
+//
+// otherwise (k > 10, tf32 mode, PRMF_EPI=0, ranks without rows):
+//   X-stream pass 1 (launch_xv)   A partials = Xt^T.V                                      (:420)
+//   u_update_kernel               U <- U*A/(U.Gv+U), Gu partials                          (:421-422,:425)
+//   X-stream pass 2 (launch_xtu)  B partials = X^T.U_new                                  (:424)
+//   reduce_pack_kernel + ncclAllReduce          only when sharded
+//   v_update_objective_kernel     V_new (double-buffered), Gv/VB partials, objective     (:425-444,:336-372,:542-548)
+//   (k > 16: the tiled U / V updates, gram_reduce_kernel, manifold_parts_kernel and objective_kernel instead)
 #include "../../include/prmf_b200.h"
 
 #include <algorithm>
@@ -22,7 +31,6 @@
 
 #include "kernels.cuh"
 #include "block_params.h"
-#include "fused.cuh"
 #include "tf32.cuh"
 #include "nccl_dyn.h"
 #include "nnls_init.cuh"
@@ -132,6 +140,7 @@ struct prmf_handle {
     Arena arena, pw_arena, as_arena;
     double *X = nullptr, *Xt = nullptr;       // samples x genes, and its transposed copy genes x samples
     double *U = nullptr, *Vbuf[2] = {nullptr, nullptr}, *Ub = nullptr, *Vb = nullptr, *Gvb = nullptr;
+    double* U2 = nullptr;                     // the other U buffer: the fused U update writes U_new there
     int vcur = 0;                             // Vbuf[vcur] is the current V
     double* Apart = nullptr;                  // pass-1 partials [chunks1][m][k]
     double *Gv = nullptr, *Gu_part = nullptr, *Gv_part = nullptr, *VB_part = nullptr;
@@ -163,18 +172,15 @@ struct prmf_handle {
 
     // launch geometry
     int uu_grid = 0, uu_rows = 0, vu_grid = 0, vu_rows = 0;
+    int nq = 1, ni = 1;
+    unsigned int* ticket = nullptr;
+    // fp64 X-stream kernels (TMA ring of tma_stages stages of kTmaRS rows)
+    int tma_fg = 1, tma_kt = 0;               // factor groups / factors per thread of the general-k kernel
+    int tma_stages = 3;
     int panels1 = 0, panel_w1 = 0, chunks1 = 0;      // pass 1: panels over samples, chunks over genes
     int64_t rows_per_chunk1 = 0;
     int panels = 0, panel_w = 0, chunks = 0;         // pass 2: panels over genes, chunks over samples
     int64_t rows_per_chunk = 0;
-    int ktile = 0, nq = 1, ni = 1;
-    unsigned int* ticket = nullptr;
-    // TMA (bulk-async) variant of the X-stream kernel: used when one factor tile covers k
-    bool use_tma = false;
-    int tma_fg = 1, tma_kt = 0;               // factor groups / factors per thread of the general-k kernel
-    int tma_rs = 8, tma_stages = 3;
-    int tpanels1 = 0, tpanel_w1 = 0, tchunks1 = 0, tpanels = 0, tpanel_w = 0, tchunks = 0;
-    int64_t trows_per_chunk1 = 0, trows_per_chunk = 0;
     size_t tma_smem1 = 0, tma_smem2 = 0;
 
     // large k (> 16): register-tiled U update, Gram partials folded by gram_reduce_kernel, objective as its own launch
@@ -186,7 +192,7 @@ struct prmf_handle {
 
     // fused tails (k <= 10, TMA path): the U / V updates run in the last CTA of each panel of the X-stream kernels
     bool use_epi = false;
-    unsigned long long* epi_counters = nullptr;   // arrive | done, each [tpanels1 + tpanels], monotone over launches
+    unsigned long long* epi_counters = nullptr;   // arrive | done, each [panels1 + panels], monotone over launches
     unsigned long long epi_seq1 = 0, epi_seq2 = 0;
     // deferred objective: per-step history [obj_capacity] of what the objective needs (one cudaMalloc)
     double* hist = nullptr;
@@ -212,14 +218,6 @@ struct prmf_handle {
     double* xsmall = nullptr;                 // receive slots of the small all-reduce (set-up scalars without NCCL)
     unsigned long long small_seq = 0;
     size_t xcount = 0;
-
-    // single-pass fused X kernel (opt-in: PRMF_FUSED=1)
-    bool use_fused = false;
-    FusedParams fp{};
-    size_t fused_smem = 0;
-    double* U2 = nullptr;
-    unsigned long long* fEx = nullptr;        // tagged exchange words of the fused kernel
-    unsigned long long fused_epoch = 0;
 
     // TF32 tensor-core storage mode (opt-in: prmf_create_ex with PRMF_X_TF32): X, X^T kept as fp32 rounded to tf32,
     // both passes by tc_rowdot_kernel, everything else unchanged
@@ -302,12 +300,6 @@ int dalloc(prmf_handle* h, T** p, size_t count) {
 
 int64_t round_up(int64_t a, int64_t b) { return (a + b - 1) / b * b; }
 
-int pick_ktile(int k) {
-    if (k <= 10) return k;
-    int tiles = (k + 9) / 10;
-    return (k + tiles - 1) / tiles;
-}
-
 int pick_nq(int k) {
     int pairs = k * k;
     int q = (pairs + 255) / 256;
@@ -326,42 +318,15 @@ int set_smem(prmf_handle* h, F kernel, size_t bytes) {
 
 // ---- templated launch dispatch ---------------------------------------------------------------------
 template <int KT>
-void launch_skinny_t(prmf_handle* h, const double* M, int64_t ldm, int64_t rows, int64_t cols, const double* W,
-                     int k0, int panels, int panel_w, int chunks, int64_t rows_per_chunk, double* out) {
-    dim3 grid(panels, chunks);
-    skinny_tn_kernel<KT><<<grid, 256, 0, h->stream>>>(M, ldm, rows, cols, W, h->k, k0, panel_w, rows_per_chunk, out);
-}
-
-#define KT_SWITCH(kt, FN, ...)          \
-    switch (kt) {                       \
-        case 1: FN<1>(__VA_ARGS__); break;   \
-        case 2: FN<2>(__VA_ARGS__); break;   \
-        case 3: FN<3>(__VA_ARGS__); break;   \
-        case 4: FN<4>(__VA_ARGS__); break;   \
-        case 5: FN<5>(__VA_ARGS__); break;   \
-        case 6: FN<6>(__VA_ARGS__); break;   \
-        case 7: FN<7>(__VA_ARGS__); break;   \
-        case 8: FN<8>(__VA_ARGS__); break;   \
-        case 9: FN<9>(__VA_ARGS__); break;   \
-        default: FN<10>(__VA_ARGS__); break; \
-    }
-
-template <int KT>
 int launch_skinny_tma_t(prmf_handle* h, const double* M, int64_t ldm, int64_t rows, int64_t cols, const double* W,
                         int panels, int panel_w, int chunks, int64_t rows_per_chunk, size_t smem, double* out) {
     dim3 grid(panels, chunks);
     EpiParams none{};
     none.dbg_slot = -1;
     none.err = h->err_word; none.timeout_ns = h->spin_timeout_ns;
-    if (h->tma_rs == 4) {
-        CU(cudaFuncSetAttribute(skinny_tma_kernel<KT, 4, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        skinny_tma_kernel<KT, 4, 0><<<grid, kTmaThreads, smem, h->stream>>>(M, ldm, rows, cols, W, panel_w, rows_per_chunk,
-                                                                            h->tma_stages, out, none);
-    } else {
-        CU(cudaFuncSetAttribute(skinny_tma_kernel<KT, 8, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        skinny_tma_kernel<KT, 8, 0><<<grid, kTmaThreads, smem, h->stream>>>(M, ldm, rows, cols, W, panel_w, rows_per_chunk,
-                                                                            h->tma_stages, out, none);
-    }
+    CU(cudaFuncSetAttribute(skinny_tma_kernel<KT, kTmaRS, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    skinny_tma_kernel<KT, kTmaRS, 0><<<grid, kTmaThreads, smem, h->stream>>>(M, ldm, rows, cols, W, panel_w,
+                                                                             rows_per_chunk, h->tma_stages, out, none);
     return PRMF_OK;
 }
 
@@ -378,10 +343,10 @@ int launch_skinny_epi_t(prmf_handle* h, int epi, const double* M, int64_t ldm, i
                     (void*)&rows_per_chunk, (void*)&stages, (void*)&out, (void*)&ep};
     const void* fn = nullptr;
     switch (epi) {
-        case 1: fn = (const void*)skinny_tma_kernel<KT, 8, 1>; break;
-        case 2: fn = (const void*)skinny_tma_kernel<KT, 8, 2>; break;
-        case 3: fn = (const void*)skinny_tma_kernel<KT, 8, 3>; break;
-        case 4: fn = (const void*)skinny_tma_kernel<KT, 8, 4>; break;
+        case 1: fn = (const void*)skinny_tma_kernel<KT, kTmaRS, 1>; break;
+        case 2: fn = (const void*)skinny_tma_kernel<KT, kTmaRS, 2>; break;
+        case 3: fn = (const void*)skinny_tma_kernel<KT, kTmaRS, 3>; break;
+        case 4: fn = (const void*)skinny_tma_kernel<KT, kTmaRS, 4>; break;
         default: return fail(h, PRMF_ERR_STATE, "bad fused-tail id %d", epi);
     }
     CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -394,9 +359,9 @@ template <int KT, int FG>
 int launch_skinny_gen_t(prmf_handle* h, const double* M, int64_t ldm, int64_t rows, int64_t cols, const double* W,
                         int panels, int panel_w, int chunks, int64_t rows_per_chunk, size_t smem, double* out) {
     dim3 grid(panels, chunks);
-    CU(cudaFuncSetAttribute(skinny_tma_gen_kernel<KT, FG, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    skinny_tma_gen_kernel<KT, FG, 8><<<grid, kTmaThreads, smem, h->stream>>>(M, ldm, rows, cols, W, h->k, panel_w,
-                                                                             rows_per_chunk, h->tma_stages, out);
+    CU(cudaFuncSetAttribute(skinny_tma_gen_kernel<KT, FG, kTmaRS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    skinny_tma_gen_kernel<KT, FG, kTmaRS><<<grid, kTmaThreads, smem, h->stream>>>(M, ldm, rows, cols, W, h->k, panel_w,
+                                                                                  rows_per_chunk, h->tma_stages, out);
     return PRMF_OK;
 }
 
@@ -425,41 +390,9 @@ int launch_skinny_gen(prmf_handle* h, const double* M, int64_t ldm, int64_t rows
         default: rc = FN<10>(__VA_ARGS__); break; \
     }
 
-template <int K>
-int launch_fused_t(prmf_handle* h) {
-    CU(cudaFuncSetAttribute(fused_xvu_kernel<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->fused_smem));
-    FusedParams prm = h->fp;
-    void* args[] = {&prm};
-    dim3 grid(h->fp.panels, h->fp.groups);
-    CU(cudaLaunchCooperativeKernel((void*)fused_xvu_kernel<K>, grid, dim3(kFThreads), args, h->fused_smem, h->stream));
-    return PRMF_OK;
-}
-
-// fused step: U update and B partials from ONE pass over X
-int launch_fused(prmf_handle* h) {
-    if (h->m == 0) {
-        CU(cudaMemsetAsync(h->Bpart, 0, sizeof(double) * h->fp.groups * h->n * h->k, h->stream));
-        CU(cudaMemsetAsync(h->Gu_part, 0, sizeof(double) * h->fp.groups * h->k * h->k, h->stream));
-        return PRMF_OK;
-    }
-    h->fused_epoch += (1ull << 24);
-    h->fp.Uold = h->U;
-    h->fp.Unew = h->U2;
-    h->fp.V = h->Vbuf[h->vcur];
-    h->fp.epoch = h->fused_epoch;
-    int rc = 0;
-    KT_SWITCH_RC(h->k, rc, launch_fused_t, h);
-    if (rc) return rc;
-    LAUNCH_CHECK("fused_xvu_kernel");
-    std::swap(h->U, h->U2);
-    return PRMF_OK;
-}
-
 // number of per-chunk partials the passes leave in Apart / Bpart
-int a_chunks(const prmf_handle* h) { return h->x_tf32 ? h->tc_chunks1 : h->use_tma ? h->tchunks1 : h->chunks1; }
-int b_chunks(const prmf_handle* h) {
-    return h->x_tf32 ? h->tc_chunks2 : h->use_fused ? h->fp.groups : h->use_tma ? h->tchunks : h->chunks;
-}
+int a_chunks(const prmf_handle* h) { return h->x_tf32 ? h->tc_chunks1 : h->chunks1; }
+int b_chunks(const prmf_handle* h) { return h->x_tf32 ? h->tc_chunks2 : h->chunks; }
 
 // TF32 mode: one tensor-core kernel serves both passes
 int launch_tc(prmf_handle* h, const CUtensorMap& tmM, const CUtensorMap& tmW, const TcParams& prm, int tiles, int chunks,
@@ -483,33 +416,23 @@ int refresh_wt(prmf_handle* h, const double* W, int64_t rows, float* Wt, int64_t
 int launch_xv(prmf_handle* h) {
     if (h->m == 0) return PRMF_OK;
     if (h->x_tf32) return launch_tc(h, h->tm_X, h->tm_Vt, h->tc1, h->tc_tiles1, h->tc_chunks1, "tc_rowdot_kernel(pass 1)");
-    if (h->use_tma) {
-        int rc = 0;
-        if (h->k > 10) {
-            rc = launch_skinny_gen(h, h->Xt, h->ldxt, h->n, h->m, h->Vbuf[h->vcur], h->tpanels1, h->tpanel_w1,
-                                   h->tchunks1, h->trows_per_chunk1, h->tma_smem1, h->Apart);
-        } else {
-            KT_SWITCH_RC(h->k, rc, launch_skinny_tma_t, h, h->Xt, h->ldxt, h->n, h->m, h->Vbuf[h->vcur], h->tpanels1,
-                         h->tpanel_w1, h->tchunks1, h->trows_per_chunk1, h->tma_smem1, h->Apart);
-        }
-        if (rc) return rc;
-        LAUNCH_CHECK("skinny_tma_kernel(pass 1)");
-        return PRMF_OK;
+    int rc = 0;
+    if (h->k > 10) {
+        rc = launch_skinny_gen(h, h->Xt, h->ldxt, h->n, h->m, h->Vbuf[h->vcur], h->panels1, h->panel_w1, h->chunks1,
+                               h->rows_per_chunk1, h->tma_smem1, h->Apart);
+    } else {
+        KT_SWITCH_RC(h->k, rc, launch_skinny_tma_t, h, h->Xt, h->ldxt, h->n, h->m, h->Vbuf[h->vcur], h->panels1,
+                     h->panel_w1, h->chunks1, h->rows_per_chunk1, h->tma_smem1, h->Apart);
     }
-    for (int k0 = 0; k0 < h->k; k0 += h->ktile) {
-        int kt = std::min(h->ktile, h->k - k0);
-        KT_SWITCH(kt, launch_skinny_t, h, h->Xt, h->ldxt, h->n, h->m, h->Vbuf[h->vcur], k0, h->panels1, h->panel_w1,
-                  h->chunks1, h->rows_per_chunk1, h->Apart);
-        LAUNCH_CHECK("skinny_tn_kernel(pass 1)");
-    }
+    if (rc) return rc;
+    LAUNCH_CHECK("skinny_tma_kernel(pass 1)");
     return PRMF_OK;
 }
 
 // pass 2: B partials = X^T . U_new   (M = X: m rows x n cols)
 int launch_xtu(prmf_handle* h) {
     if (h->m == 0) {
-        CU(cudaMemsetAsync(h->Bpart, 0, sizeof(double) * std::max({h->chunks, h->tchunks, h->tc_chunks2}) * h->n * h->k,
-                           h->stream));
+        CU(cudaMemsetAsync(h->Bpart, 0, sizeof(double) * b_chunks(h) * h->n * h->k, h->stream));
         return PRMF_OK;
     }
     if (h->x_tf32) {
@@ -517,25 +440,16 @@ int launch_xtu(prmf_handle* h) {
         if (rc) return rc;
         return launch_tc(h, h->tm_Xt, h->tm_Ut, h->tc2, h->tc_tiles2, h->tc_chunks2, "tc_rowdot_kernel(pass 2)");
     }
-    if (h->use_tma) {
-        int rc = 0;
-        if (h->k > 10) {
-            rc = launch_skinny_gen(h, h->X, h->ldx, h->m, h->n, h->U, h->tpanels, h->tpanel_w, h->tchunks,
-                                   h->trows_per_chunk, h->tma_smem2, h->Bpart);
-        } else {
-            KT_SWITCH_RC(h->k, rc, launch_skinny_tma_t, h, h->X, h->ldx, h->m, h->n, h->U, h->tpanels, h->tpanel_w,
-                         h->tchunks, h->trows_per_chunk, h->tma_smem2, h->Bpart);
-        }
-        if (rc) return rc;
-        LAUNCH_CHECK("skinny_tma_kernel(pass 2)");
-        return PRMF_OK;
+    int rc = 0;
+    if (h->k > 10) {
+        rc = launch_skinny_gen(h, h->X, h->ldx, h->m, h->n, h->U, h->panels, h->panel_w, h->chunks, h->rows_per_chunk,
+                               h->tma_smem2, h->Bpart);
+    } else {
+        KT_SWITCH_RC(h->k, rc, launch_skinny_tma_t, h, h->X, h->ldx, h->m, h->n, h->U, h->panels, h->panel_w, h->chunks,
+                     h->rows_per_chunk, h->tma_smem2, h->Bpart);
     }
-    for (int k0 = 0; k0 < h->k; k0 += h->ktile) {
-        int kt = std::min(h->ktile, h->k - k0);
-        KT_SWITCH(kt, launch_skinny_t, h, h->X, h->ldx, h->m, h->n, h->U, k0, h->panels, h->panel_w, h->chunks,
-                  h->rows_per_chunk, h->Bpart);
-        LAUNCH_CHECK("skinny_tn_kernel(pass 2)");
-    }
+    if (rc) return rc;
+    LAUNCH_CHECK("skinny_tma_kernel(pass 2)");
     return PRMF_OK;
 }
 
@@ -627,7 +541,7 @@ int launch_v_update_objective(prmf_handle* h, bool sharded, double tradeoff) {
     const double* Bsrc = sharded ? h->red : h->Bpart;
     const int bchunks = sharded ? 1 : b_chunks(h);
     const double* Gusrc = sharded ? h->red + nk : h->big_k ? h->Gu_glob : h->Gu_part;
-    const int gchunks = (sharded || h->big_k) ? 1 : h->use_fused ? h->fp.groups : h->uu_grid;
+    const int gchunks = (sharded || h->big_k) ? 1 : h->uu_grid;
     double* Gu_out = (h->big_k && sharded) ? h->Gu_glob : nullptr;
     if (h->big_k) {
 #define TILED_CASE(C)                                                                                                  \
@@ -743,7 +657,7 @@ int ensure_pos(prmf_handle* h) {
 int launch_xv_epi(prmf_handle* h, const double* gv_src = nullptr, int gv_parts = 1) {
     EpiParams ep{};
     ep.err = h->err_word; ep.timeout_ns = h->spin_timeout_ns;
-    const size_t np = (size_t)h->tpanels1 + h->tpanels;
+    const size_t np = (size_t)h->panels1 + h->panels;
     ep.arrive = h->epi_counters;
     ep.done = h->epi_counters + np;
     ep.seq = ++h->epi_seq1;
@@ -756,8 +670,8 @@ int launch_xv_epi(prmf_handle* h, const double* gv_src = nullptr, int gv_parts =
     ep.gv_parts = gv_src ? gv_parts : 1;
     ep.Gu_part = h->Gu_part;
     int rc = 0;
-    KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, 1, h->Xt, h->ldxt, h->n, h->m, h->Vbuf[h->vcur], h->tpanels1,
-                 h->tpanel_w1, h->tchunks1, h->trows_per_chunk1, h->tma_smem1, h->Apart, ep);
+    KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, 1, h->Xt, h->ldxt, h->n, h->m, h->Vbuf[h->vcur], h->panels1,
+                 h->panel_w1, h->chunks1, h->rows_per_chunk1, h->tma_smem1, h->Apart, ep);
     if (rc) { h->failed = true; return rc; }     // the panel counters expect this launch: no further steps on this handle
     LAUNCH_CHECK("skinny_tma_kernel(pass 1 + U update)");
     std::swap(h->U, h->U2);
@@ -768,15 +682,15 @@ int launch_xv_epi(prmf_handle* h, const double* gv_src = nullptr, int gv_parts =
 int launch_xtu_epi(prmf_handle* h, int mode, double* packed_dst, int hist_slot = -1) {
     EpiParams ep{};
     ep.err = h->err_word; ep.timeout_ns = h->spin_timeout_ns;
-    const size_t np = (size_t)h->tpanels1 + h->tpanels;
-    ep.arrive = h->epi_counters + h->tpanels1;
-    ep.done = h->epi_counters + np + h->tpanels1;
+    const size_t np = (size_t)h->panels1 + h->panels;
+    ep.arrive = h->epi_counters + h->panels1;
+    ep.done = h->epi_counters + np + h->panels1;
     ep.seq = ++h->epi_seq2;
     ep.dbg_slot = (int)((2 * (h->epi_seq2 - 1) + 1) % 64);
     ep.part2 = h->epi_part2;
     ep.vb2 = h->epi_vb2;
     ep.Gu_part_in = h->Gu_part;
-    ep.gu_parts = h->tpanels1;
+    ep.gu_parts = h->panels1;
     if (mode == 3) {
         ep.red = packed_dst;
     } else {
@@ -790,8 +704,8 @@ int launch_xtu_epi(prmf_handle* h, int mode, double* packed_dst, int hist_slot =
         ep.VB_part = h->VB_part;
         if (hist_slot >= 0) {                       // deferred objective: this step's slots
             const size_t kk2 = (size_t)h->k * h->k;
-            ep.Gv_part = h->hist_Gvp + (size_t)hist_slot * h->tpanels * kk2;
-            ep.VB_part = h->hist_VBp + (size_t)hist_slot * h->tpanels;
+            ep.Gv_part = h->hist_Gvp + (size_t)hist_slot * h->panels * kk2;
+            ep.VB_part = h->hist_VBp + (size_t)hist_slot * h->panels;
             ep.hist_Gu = h->hist_Gu + (size_t)hist_slot * kk2;
             ep.hist_vh = h->hist_vh + (size_t)hist_slot * kVhCap;
             ep.doff = h->as_off;
@@ -812,8 +726,8 @@ int launch_xtu_epi(prmf_handle* h, int mode, double* packed_dst, int hist_slot =
         ep.Gu_glob = h->Gu_glob;
     }
     int rc = 0;
-    KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, mode, h->X, h->ldx, h->m, h->n, h->U, h->tpanels, h->tpanel_w,
-                 h->tchunks, h->trows_per_chunk, h->tma_smem2, h->Bpart, ep);
+    KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, mode, h->X, h->ldx, h->m, h->n, h->U, h->panels, h->panel_w,
+                 h->chunks, h->rows_per_chunk, h->tma_smem2, h->Bpart, ep);
     if (rc) { h->failed = true; return rc; }
     LAUNCH_CHECK(mode == 3 ? "skinny_tma_kernel(pass 2 + pack)" : mode == 4 ? "skinny_tma_kernel(pass 2 + exchange + V update)"
                                                                             : "skinny_tma_kernel(pass 2 + V update)");
@@ -824,7 +738,7 @@ int launch_xtu_epi(prmf_handle* h, int mode, double* packed_dst, int hist_slot =
 // fused-tail path (k <= 10): objective of the step from the per-panel partials the pass-2 kernel left
 int launch_objective(prmf_handle* h, double tradeoff, const double* Gu_parts, int gu_parts) {
     objective_parts_kernel<<<1, kTailThreads, obj_smem(h), h->stream>>>(
-        h->Vbuf[h->vcur], h->k, Gu_parts, gu_parts, h->Gv_part, h->VB_part, h->tpanels, h->normX_sq, h->as, h->Gv, h->gd,
+        h->Vbuf[h->vcur], h->k, Gu_parts, gu_parts, h->Gv_part, h->VB_part, h->panels, h->normX_sq, h->as, h->Gv, h->gd,
         tradeoff, h->obj, h->step_counter, h->obj_capacity);
     LAUNCH_CHECK("objective_parts_kernel");
     return PRMF_OK;
@@ -881,8 +795,8 @@ int launch_block(prmf_handle* h, int h0, int nh) {
     if (nh <= 0) return PRMF_OK;
     BlockParams prm{};
     prm.X = h->X; prm.Xt = h->Xt; prm.ldx = h->ldx; prm.ldxt = h->ldxt; prm.m = h->m; prm.n = h->n;
-    prm.panels1 = h->tpanels1; prm.panel_w1 = h->tpanel_w1; prm.chunks1 = h->tchunks1; prm.rpc1 = h->trows_per_chunk1;
-    prm.panels2 = h->tpanels; prm.panel_w2 = h->tpanel_w; prm.chunks2 = h->tchunks; prm.rpc2 = h->trows_per_chunk;
+    prm.panels1 = h->panels1; prm.panel_w1 = h->panel_w1; prm.chunks1 = h->chunks1; prm.rpc1 = h->rows_per_chunk1;
+    prm.panels2 = h->panels; prm.panel_w2 = h->panel_w; prm.chunks2 = h->chunks; prm.rpc2 = h->rows_per_chunk;
     prm.stages = h->tma_stages;
     prm.ring_stage_bytes = h->blk_stage_bytes;
     prm.U[0] = h->U; prm.U[1] = h->U2;
@@ -891,10 +805,10 @@ int launch_block(prmf_handle* h, int h0, int nh) {
     prm.part2 = h->epi_part2; prm.vb2 = h->epi_vb2;
     prm.Gv0 = h->Gv;
     unsigned long long* c = h->blk_ctr;
-    prm.arrive1 = c; c += h->tpanels1;
-    prm.done1 = c; c += h->tpanels1;
-    prm.arrive2 = c; c += h->tpanels;
-    prm.done2 = c; c += h->tpanels;
+    prm.arrive1 = c; c += h->panels1;
+    prm.done1 = c; c += h->panels1;
+    prm.arrive2 = c; c += h->panels;
+    prm.done2 = c; c += h->panels;
     prm.udone = c; prm.vdone = c + 1; prm.ufold = c + 2; prm.vfold = c + 3;
     prm.base1 = h->blk_n1; prm.base2 = h->blk_n2;
     prm.h0 = h0; prm.nh = nh;
@@ -912,7 +826,7 @@ int launch_block(prmf_handle* h, int h0, int nh) {
     }
     int n_p1 = 0, n_p2 = 0;
     for (int i = 0; i < nh; ++i) (((h0 + i) & 1) == 0 ? n_p1 : n_p2)++;
-    const int grid = std::max(h->tpanels1 * h->tchunks1, h->tpanels * h->tchunks);
+    const int grid = std::max(h->panels1 * h->chunks1, h->panels * h->chunks);
     cudaError_t e_ = prmf_launch_block_kernel(h->k, prm, grid, h->blk_smem, h->stream);
     if (e_ == cudaSuccess) e_ = cudaGetLastError();
     if (e_ != cudaSuccess) {                      // the counters below only move for a launch that is really queued
@@ -935,7 +849,7 @@ void cancel_ahead(prmf_handle* h) {
 }
 
 int prefetch_pass1(prmf_handle* h) {
-    if (h->ahead || h->profiling || h->use_fused || h->m == 0) return PRMF_OK;
+    if (h->ahead || h->profiling || h->m == 0) return PRMF_OK;
     if (!h->have_X || !h->have_U || !h->have_V) return PRMF_OK;
     int rc = 0;
     if (h->failed) return PRMF_OK;
@@ -1037,7 +951,7 @@ int enqueue_steps(prmf_handle* h, int n_steps, double gamma, double delta, doubl
         h->ahead = 0;
         if ((rc = launch_block(h, h0, 2 * n_steps - h0))) return rc;
         objective_deferred_kernel<<<n_steps, kTailThreads, obj_smem(h), h->stream>>>(
-            h->k, h->hist_Gu, h->hist_Gvp, h->hist_VBp, h->tpanels, h->hist_vh, kVhCap, h->normX_sq, h->as, h->Gv,
+            h->k, h->hist_Gu, h->hist_Gvp, h->hist_VBp, h->panels, h->hist_vh, kVhCap, h->normX_sq, h->as, h->Gv,
             h->gd, h->obj, h->obj_capacity);
         LAUNCH_CHECK("objective_deferred_kernel");
         return PRMF_OK;
@@ -1052,13 +966,13 @@ int enqueue_steps(prmf_handle* h, int n_steps, double gamma, double delta, doubl
             // one GPU, fixed gamma / delta: the objective of every step is evaluated by ONE launch after the block
             if (!skip_pass1) {
                 const size_t kk2s = (size_t)h->k * h->k;
-                rc = s == 0 ? launch_xv_epi(h) : launch_xv_epi(h, h->hist_Gvp + (size_t)(s - 1) * h->tpanels * kk2s, h->tpanels);
+                rc = s == 0 ? launch_xv_epi(h) : launch_xv_epi(h, h->hist_Gvp + (size_t)(s - 1) * h->panels * kk2s, h->panels);
                 if (rc) return rc;
             }
             if ((rc = launch_xtu_epi(h, !sharded(h) ? 2 : 4, nullptr, s))) return rc;
             if (s == n_steps - 1) {
                 objective_deferred_kernel<<<n_steps, kTailThreads, obj_smem(h), h->stream>>>(
-                    h->k, h->hist_Gu, h->hist_Gvp, h->hist_VBp, h->tpanels, h->hist_vh, kVhCap, h->normX_sq, h->as, h->Gv,
+                    h->k, h->hist_Gu, h->hist_Gvp, h->hist_VBp, h->panels, h->hist_vh, kVhCap, h->normX_sq, h->as, h->Gv,
                     h->gd, h->obj, h->obj_capacity);
                 LAUNCH_CHECK("objective_deferred_kernel");
             }
@@ -1070,7 +984,7 @@ int enqueue_steps(prmf_handle* h, int n_steps, double gamma, double delta, doubl
             if (!sharded(h)) {
                 tic(2); rc = launch_xtu_epi(h, 2, nullptr); toc();               // + V update
                 if (rc) return rc;
-                tic(5); rc = launch_objective(h, tradeoff, h->Gu_part, h->tpanels1); toc();
+                tic(5); rc = launch_objective(h, tradeoff, h->Gu_part, h->panels1); toc();
                 if (rc) return rc;
             } else if (h->use_xchg) {
                 tic(2); rc = launch_xtu_epi(h, 4, nullptr); toc();               // + exchange + V update
@@ -1090,24 +1004,18 @@ int enqueue_steps(prmf_handle* h, int n_steps, double gamma, double delta, doubl
             }
             continue;
         }
-        if (h->use_fused) {
-            tic(0); rc = launch_fused(h); toc();
-            if (rc) return rc;
-        } else {
-            if (!skip_pass1) { tic(0); rc = launch_xv(h); toc(); }
-            if (rc) return rc;
-            tic(1); rc = launch_u_update(h); toc();
-            if (rc) return rc;
-            tic(2); rc = launch_xtu(h); toc();
-            if (rc) return rc;
-        }
+        if (!skip_pass1) { tic(0); rc = launch_xv(h); toc(); }
+        if (rc) return rc;
+        tic(1); rc = launch_u_update(h); toc();
+        if (rc) return rc;
+        tic(2); rc = launch_xtu(h); toc();
+        if (rc) return rc;
         const bool is_sharded = sharded(h);
         if (is_sharded) {
             tic(3);
             double* dst = h->p2p_ready ? h->p2p_buf + (size_t)h->p2p_parity * h->p2p_red_count : h->red;
             reduce_pack_kernel<<<(unsigned)((nk + kk2 + 2 + 255) / 256), 256, 0, h->stream>>>(
-                h->Bpart, b_chunks(h), nk, h->Gu_part,
-                h->use_fused ? h->fp.groups : h->uu_grid, h->k, dst);
+                h->Bpart, b_chunks(h), nk, h->Gu_part, h->uu_grid, h->k, dst);
             LAUNCH_CHECK("reduce_pack_kernel");
             if (!h->p2p_ready) rc = allreduce(h, h->red, red_count);      // else: summed inside the V update
             toc();
@@ -1283,7 +1191,7 @@ int nnls_loop(prmf_handle* h, int transpose, NnlsWork& wk, double* rnorm_dev, st
     const int k = wk.k;
     double* W = transpose ? h->Vbuf[h->vcur] : h->U;
     const double* part = transpose ? h->Apart : h->Bpart;
-    const int chunks = transpose ? a_chunks(h) : (h->use_tma ? h->tchunks : h->chunks);
+    const int chunks = transpose ? a_chunks(h) : b_chunks(h);
     const int64_t wcount = wk.nun * k;
     const dim3 rgrid((unsigned)((wk.neq + kNnlsThreads - 1) / kNnlsThreads), (unsigned)k);
     // every launch of nnls_step_kernel counts one iteration of each running problem, so the loop ends by maxiter + 1
@@ -1391,7 +1299,6 @@ int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_glo
         h->own_stream = true;
     }
     // launch geometry
-    h->ktile = pick_ktile(k);
     h->nq = pick_nq(k);
     h->ni = pick_ni(k);
     h->uu_rows = (int)std::max<int64_t>(8, std::min<int64_t>(128, 2048 / k));
@@ -1410,98 +1317,62 @@ int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_glo
         h->vu_rows = 32;
         h->vu_grid = (int)std::max<int64_t>(1, std::min<int64_t>(h->sm_count, (n + 31) / 32));
     }
-    // pass 2 (X^T.U): column panels over genes, row chunks over samples
-    h->panels = (int)((n + 1023) / 1024);
-    h->panel_w = (int)round_up((n + h->panels - 1) / h->panels, 4);
-    h->chunks = std::max(1, (h->sm_count * 2) / h->panels);
-    if (m_local > 0) h->chunks = (int)std::min<int64_t>(h->chunks, std::max<int64_t>(1, m_local / 64));
-    h->rows_per_chunk = std::max<int64_t>(1, (m_local + h->chunks - 1) / h->chunks);
-    // pass 1 (Xt^T.V): column panels over samples, row chunks over genes
-    h->panels1 = (int)std::max<int64_t>(1, (m_local + 1023) / 1024);
-    h->panel_w1 = (int)round_up((std::max<int64_t>(1, m_local) + h->panels1 - 1) / h->panels1, 4);
-    h->chunks1 = std::max(1, (h->sm_count * 2) / h->panels1);
-    h->chunks1 = (int)std::min<int64_t>(h->chunks1, std::max<int64_t>(1, n / 64));
-    h->rows_per_chunk1 = std::max<int64_t>(1, (n + h->chunks1 - 1) / h->chunks1);
-
-    // TMA variant: one CTA per SM, <= 1024-column panels, row chunks a multiple of the stage height
+    // X-stream plan: one CTA per SM, column panels of at most 1024 / FG columns, row chunks of at least 4 stages
+    if (k > 10) {                          // general-k kernel: FG factor groups x KT factors per thread
+        const int groups = (k + 15) / 16;
+        h->tma_fg = groups <= 1 ? 1 : groups <= 2 ? 2 : groups <= 4 ? 4 : 8;
+        const int per = (k + h->tma_fg - 1) / h->tma_fg;
+        h->tma_kt = per <= 8 ? 8 : per <= 12 ? 12 : 16;
+    }
     {
-        const char* e1 = getenv("PRMF_TMA");
-        const char* e2 = getenv("PRMF_TMA_RS");
-        const char* e3 = getenv("PRMF_TMA_STAGES");
-        h->use_tma = !(e1 && atoi(e1) == 0);
-        if (e2 && atoi(e2) == 4 && k <= 10) h->tma_rs = 4;
-        if (e3 && atoi(e3) >= 2 && atoi(e3) <= 12) h->tma_stages = atoi(e3);
-        if (k > 10) {                      // general-k kernel: FG factor groups x KT factors per thread
-            const int groups = (k + 15) / 16;
-            h->tma_fg = groups <= 1 ? 1 : groups <= 2 ? 2 : groups <= 4 ? 4 : 8;
-            const int per = (k + h->tma_fg - 1) / h->tma_fg;
-            h->tma_kt = per <= 8 ? 8 : per <= 12 ? 12 : 16;
-            if (!e3) h->tma_stages = h->tma_fg >= 4 ? 6 : h->tma_fg == 2 ? 4 : 3;
-        }
         const int64_t max_panel = 1024 / h->tma_fg;
         auto plan = [&](int64_t cols, int64_t rows, int* panels, int* panel_w, int* chunks, int64_t* rpc, size_t* smem) {
             *panels = (int)std::max<int64_t>(1, (cols + max_panel - 1) / max_panel);
             *panel_w = (int)round_up((std::max<int64_t>(1, cols) + *panels - 1) / *panels, 4);
             *chunks = std::max(1, h->sm_count / *panels);
-            *chunks = (int)std::min<int64_t>(*chunks, std::max<int64_t>(1, rows / (4 * h->tma_rs)));
+            *chunks = (int)std::min<int64_t>(*chunks, std::max<int64_t>(1, rows / (4 * kTmaRS)));
             // rows per chunk: even (the W rows of a chunk must start 16-byte aligned for the bulk copies), not a multiple
             // of the stage height -- a ragged last stage costs less than a last chunk that is nearly empty
             *rpc = round_up(std::max<int64_t>(1, (rows + *chunks - 1) / *chunks), 2);
-            const size_t xb = (size_t)h->tma_rs * *panel_w * 8;
-            const size_t wb = (((size_t)h->tma_rs * k + 16) * 8 + 127) & ~(size_t)127;
+            const size_t xb = (size_t)kTmaRS * *panel_w * 8;
+            const size_t wb = (((size_t)kTmaRS * k + 16) * 8 + 127) & ~(size_t)127;
             *smem = h->tma_stages * (xb + wb) + 2 * h->tma_stages * sizeof(uint64_t);
         };
-        plan(m_local, n, &h->tpanels1, &h->tpanel_w1, &h->tchunks1, &h->trows_per_chunk1, &h->tma_smem1);
-        plan(n, m_local, &h->tpanels, &h->tpanel_w, &h->tchunks, &h->trows_per_chunk, &h->tma_smem2);
-        if (h->tma_smem1 > 220 * 1024 || h->tma_smem2 > 220 * 1024) h->use_tma = false;
-    }
-
-    // single-pass fused kernel plan (opt-in)
-    {
-        const char* ef = getenv("PRMF_FUSED");
-        h->use_fused = ef && atoi(ef) == 1 && k <= 10 && n <= 512 * kFMaxPanels;     // tags: epoch starts at 2^24 > 0
-        if (h->use_fused) {
-            FusedParams& f = h->fp;
-            f.panels = (int)((n + 511) / 512);
-            f.panel_w = (int)round_up((n + f.panels - 1) / f.panels, 4);
-            f.groups = std::max(1, h->sm_count / f.panels);
-            f.groups = (int)std::min<int64_t>(f.groups, std::max<int64_t>(1, m_local / 64));
-            f.rows_per_group = round_up(std::max<int64_t>(1, (m_local + f.groups - 1) / f.groups), kFRS);
-            uint32_t pitch = (uint32_t)f.panel_w * 8u;
-            while (pitch % 128u != 32u) pitch += 16u;
-            f.pitch = pitch;
-            const size_t stage = (size_t)kFRS * pitch + (((size_t)kFRS * k * 8 + 127) & ~(size_t)127);
-            const size_t fixed = sizeof(double) * ((size_t)kFPaSlots * kFConsWarps * kFRS * kFKP + ((k * k + 1) & ~1)) + 512;
-            int S = (int)((220 * 1024 - fixed) / (stage + sizeof(double) * kFRS * kFKP + 3 * sizeof(uint64_t)));
-            S = std::min(S, 8);
-            f.stages = S;
-            h->fused_smem = (size_t)S * stage + fixed + (size_t)S * (sizeof(double) * kFRS * kFKP + 3 * sizeof(uint64_t));
-            if (S < kFLag + 2 || f.panels * f.groups > h->sm_count) h->use_fused = false;
-            f.ldx = h->ldx; f.m = m_local; f.n = (int)n; f.k = k;
+        auto plan_passes = [&]() {         // true when both rings fit
+            plan(m_local, n, &h->panels1, &h->panel_w1, &h->chunks1, &h->rows_per_chunk1, &h->tma_smem1);
+            plan(n, m_local, &h->panels, &h->panel_w, &h->chunks, &h->rows_per_chunk, &h->tma_smem2);
+            return std::max(h->tma_smem1, h->tma_smem2) <= 220 * 1024;
+        };
+        // the default ring fits at every k <= 128 (tests/test_xstream_exact.py); a PRMF_TMA_STAGES override is kept
+        // where its ring fits as well, and the handle runs the default elsewhere
+        const int default_stages = h->tma_fg >= 4 ? 6 : h->tma_fg == 2 ? 4 : 3;
+        const char* es = getenv("PRMF_TMA_STAGES");
+        const int want = es ? atoi(es) : 0;
+        h->tma_stages = want >= 2 && want <= 12 ? want : default_stages;
+        if (!plan_passes()) {
+            h->tma_stages = default_stages;
+            plan_passes();
         }
     }
 
     h->x_tf32 = x_dtype == PRMF_X_TF32;
-    if (h->x_tf32) {
-        h->use_fused = false;
-        setup_tf32(h);
-    }
+    if (h->x_tf32) setup_tf32(h);
     {
         const char* ee = getenv("PRMF_EPI");
-        h->use_epi = !(ee && atoi(ee) == 0) && h->use_tma && k <= 10 && h->tma_rs == 8 && m_local > 0 && !h->x_tf32 &&
-                     !h->use_fused && h->tpanels1 * h->tchunks1 <= h->sm_count && h->tpanels * h->tchunks <= h->sm_count;
+        h->use_epi = !(ee && atoi(ee) == 0) && k <= 10 && m_local > 0 && !h->x_tf32 &&
+                     h->panels1 * h->chunks1 <= h->sm_count && h->panels * h->chunks <= h->sm_count;
         if (h->use_epi) {
             // the last CTA of a panel reuses the ring for Gv/Gu, the slice sums and the panel's new rows
-            const size_t share1 = (size_t)(h->tpanel_w1 + h->tchunks1 - 1) / h->tchunks1 * k;
-            const size_t share2 = (size_t)(h->tpanel_w + h->tchunks - 1) / h->tchunks * k;
+            const size_t share1 = (size_t)(h->panel_w1 + h->chunks1 - 1) / h->chunks1 * k;
+            const size_t share2 = (size_t)(h->panel_w + h->chunks - 1) / h->chunks * k;
             const size_t need1 = sizeof(double) * (128 + 8 * (size_t)k * k + 3 * share1);
             const size_t need2 = sizeof(double) * (128 + 8 * (size_t)k * k + 3 * share2);
             h->tma_smem1 = std::max(h->tma_smem1, need1);
             h->tma_smem2 = std::max(h->tma_smem2, need2);
         }
     }
-    const int gu_parts_max = std::max({h->uu_grid, h->fp.groups, h->use_epi ? h->tpanels1 : 0});
-    const int gv_parts_max = std::max(h->vu_grid, h->use_epi ? h->tpanels : 0);
+    const int gu_parts_max = std::max(h->uu_grid, h->use_epi ? h->panels1 : 0);
+    const int gv_parts_max = std::max(h->vu_grid, h->use_epi ? h->panels : 0);
 
     int rc = 0;
     const int64_t nk = n * k;
@@ -1513,16 +1384,14 @@ int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_glo
         const size_t d = sizeof(double);
         size_t total = 0;
         total += 3 * pad((size_t)(m_local + pad_rows) * k, d);                                      // U, U2, Ub
-        if (h->use_fused)
-            total += pad((size_t)h->fp.groups * kFExSlots * h->fp.panels * kFRS * kFKP * 2, sizeof(unsigned long long));
-        total += pad((size_t)std::max({h->chunks1, h->tchunks1, h->tc_chunks1}) * std::max<int64_t>(1, m_local) * k, d);   // Apart
+        total += pad((size_t)a_chunks(h) * std::max<int64_t>(1, m_local) * k, d);                  // Apart
         total += 2 * pad((size_t)(n + pad_rows) * k, d) + pad((size_t)nk, d);                      // Vbuf[2], Vb
         total += pad(128, d) + 4 * pad(kk2, d) + pad((size_t)gu_parts_max * kk2, d) + pad((size_t)gv_parts_max * kk2, d);
-        total += pad(gv_parts_max, d) + pad((size_t)std::max({h->chunks, h->tchunks, h->fp.groups, h->tc_chunks2}) * nk, d);   // VB_part, Bpart
-        total += pad(2 * ((size_t)h->tpanels1 + h->tpanels) + 2, sizeof(unsigned long long));     // fused-tail counters
-        total += pad(2 * ((size_t)h->tpanels1 + h->tpanels) + 4, sizeof(unsigned long long)) + pad(1, sizeof(unsigned int));   // block kernel
-        total += pad((size_t)std::max(h->tpanels1 * h->tchunks1, h->tpanels * h->tchunks) * kk2, d) +
-                 pad((size_t)h->tpanels * h->tchunks, d);                                          // per-CTA partials
+        total += pad(gv_parts_max, d) + pad((size_t)b_chunks(h) * nk, d);                           // VB_part, Bpart
+        total += pad(2 * ((size_t)h->panels1 + h->panels) + 2, sizeof(unsigned long long));     // fused-tail counters
+        total += pad(2 * ((size_t)h->panels1 + h->panels) + 4, sizeof(unsigned long long)) + pad(1, sizeof(unsigned int));   // block kernel
+        total += pad((size_t)std::max(h->panels1 * h->chunks1, h->panels * h->chunks) * kk2, d) +
+                 pad((size_t)h->panels * h->chunks, d);                                          // per-CTA partials
         total += pad((size_t)nk + kk2 + 2, d) + pad(1, d) + pad((size_t)h->sm_count * 8, d) + pad(2, d);
         total += pad(1, sizeof(int)) + pad(1, sizeof(unsigned int)) + pad(k, sizeof(int32_t)) + pad(nk, sizeof(int32_t));
         total += pad((size_t)h->obj_capacity * kObjStride, d);
@@ -1550,21 +1419,18 @@ int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_glo
     TAKE(h->U, double, (m_local + pad_rows) * k);
     TAKE(h->Ub, double, (m_local + pad_rows) * k);
     TAKE(h->U2, double, (m_local + pad_rows) * k);
-    if (h->use_fused) {
-        TAKE(h->fEx, unsigned long long, (size_t)h->fp.groups * kFExSlots * h->fp.panels * kFRS * kFKP * 2);
-    }
-    TAKE(h->Apart, double, (size_t)std::max({h->chunks1, h->tchunks1, h->tc_chunks1}) * std::max<int64_t>(1, m_local) * k);
+    TAKE(h->Apart, double, (size_t)a_chunks(h) * std::max<int64_t>(1, m_local) * k);
     TAKE(h->Vbuf[0], double, (n + pad_rows) * k); TAKE(h->Vbuf[1], double, (n + pad_rows) * k); TAKE(h->Vb, double, nk);
     TAKE(h->Gv, double, kk2); TAKE(h->Gvb, double, kk2); TAKE(h->Gu_glob, double, kk2); TAKE(h->mi_part, double, 128); TAKE(h->Gv_red, double, kk2);
     TAKE(h->Gu_part, double, (size_t)gu_parts_max * kk2);
     TAKE(h->Gv_part, double, (size_t)gv_parts_max * kk2);
     TAKE(h->VB_part, double, gv_parts_max);
-    TAKE(h->epi_counters, unsigned long long, 2 * ((size_t)h->tpanels1 + h->tpanels) + 2);
-    TAKE(h->blk_ctr, unsigned long long, 2 * ((size_t)h->tpanels1 + h->tpanels) + 4);
+    TAKE(h->epi_counters, unsigned long long, 2 * ((size_t)h->panels1 + h->panels) + 2);
+    TAKE(h->blk_ctr, unsigned long long, 2 * ((size_t)h->panels1 + h->panels) + 4);
     TAKE(h->err_word, unsigned int, 1);
-    TAKE(h->epi_part2, double, (size_t)std::max(h->tpanels1 * h->tchunks1, h->tpanels * h->tchunks) * kk2);
-    TAKE(h->epi_vb2, double, (size_t)h->tpanels * h->tchunks);
-    TAKE(h->Bpart, double, (size_t)std::max({h->chunks, h->tchunks, h->fp.groups, h->tc_chunks2}) * nk);
+    TAKE(h->epi_part2, double, (size_t)std::max(h->panels1 * h->chunks1, h->panels * h->chunks) * kk2);
+    TAKE(h->epi_vb2, double, (size_t)h->panels * h->chunks);
+    TAKE(h->Bpart, double, (size_t)b_chunks(h) * nk);
     TAKE(h->red, double, (size_t)nk + kk2 + 2);
     TAKE(h->normX_sq, double, 1);
     TAKE(h->scal_part, double, (size_t)h->sm_count * 8);
@@ -1585,16 +1451,11 @@ int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_glo
     if (!rc) {
         if (h->Xt) cudaMemsetAsync(h->Xt, 0, sizeof(double) * n * h->ldxt, h->stream);
         cudaMemsetAsync(h->ticket, 0, sizeof(unsigned int), h->stream);
-        cudaMemsetAsync(h->epi_counters, 0, sizeof(unsigned long long) * (2 * ((size_t)h->tpanels1 + h->tpanels) + 2), h->stream);
-        cudaMemsetAsync(h->blk_ctr, 0, sizeof(unsigned long long) * (2 * ((size_t)h->tpanels1 + h->tpanels) + 4), h->stream);
+        cudaMemsetAsync(h->epi_counters, 0, sizeof(unsigned long long) * (2 * ((size_t)h->panels1 + h->panels) + 2), h->stream);
+        cudaMemsetAsync(h->blk_ctr, 0, sizeof(unsigned long long) * (2 * ((size_t)h->panels1 + h->panels) + 4), h->stream);
         cudaMemsetAsync(h->err_word, 0, sizeof(unsigned int), h->stream);
         cudaMemsetAsync(h->U, 0, sizeof(double) * (m_local + pad_rows) * k, h->stream);
         cudaMemsetAsync(h->U2, 0, sizeof(double) * (m_local + pad_rows) * k, h->stream);
-        if (h->use_fused) {
-            cudaMemsetAsync(h->fEx, 0, sizeof(unsigned long long) * h->fp.groups * kFExSlots * h->fp.panels * kFRS * kFKP * 2, h->stream);
-            h->fp.X = h->X; h->fp.Gv = h->Gv; h->fp.Bpart = h->Bpart; h->fp.Gu_part = h->Gu_part;
-            h->fp.Ex = h->fEx; h->fp.Flags = nullptr;
-        }
         cudaMemsetAsync(h->Vbuf[0], 0, sizeof(double) * (n + pad_rows) * k, h->stream);
         cudaMemsetAsync(h->Vbuf[1], 0, sizeof(double) * (n + pad_rows) * k, h->stream);
         cudaMemsetAsync(h->red, 0, sizeof(double) * (nk + kk2 + 2), h->stream);
@@ -1606,7 +1467,7 @@ int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_glo
         const char* ed = getenv("PRMF_DEFER_OBJ");
         if (!(ed && atoi(ed) == 0)) {
             const size_t H = (size_t)h->obj_capacity, kk2s = (size_t)kk2;
-            const size_t n_gu = H * kk2s, n_gvp = H * h->tpanels * kk2s, n_vbp = H * h->tpanels, n_vh = H * kVhCap;
+            const size_t n_gu = H * kk2s, n_gvp = H * h->panels * kk2s, n_vbp = H * h->panels, n_vh = H * kVhCap;
             h->hist_bytes = sizeof(double) * (n_gu + n_gvp + n_vbp + n_vh);
             if (g_pool.alloc((void**)&h->hist, h->hist_bytes, device) == cudaSuccess) {
                 h->hist_Gu = h->hist;
@@ -1624,7 +1485,7 @@ int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_glo
         const char* et = getenv("PRMF_SPIN_TIMEOUT_MS");
         if (et && atof(et) > 0) h->spin_timeout_ns = (unsigned long long)(atof(et) * 1e6);
         const size_t wb = ((size_t)kBlkRS * k * 8 + 127) & ~(size_t)127;
-        h->blk_stage_bytes = (uint32_t)((size_t)kBlkRS * std::max(h->tpanel_w1, h->tpanel_w) * 8 + wb);
+        h->blk_stage_bytes = (uint32_t)((size_t)kBlkRS * std::max(h->panel_w1, h->panel_w) * 8 + wb);
         h->blk_smem = (size_t)h->tma_stages * h->blk_stage_bytes + 2 * h->tma_stages * sizeof(uint64_t) +
                       sizeof(double) * (256 + 8 * (size_t)k * k + (size_t)kBlkRowsCap * k);
         h->use_block = h->use_epi && h->defer_ok && !(eb && atoi(eb) == 0) && h->blk_smem <= 227 * 1024;
@@ -2122,8 +1983,8 @@ int prmf_p2p_finalize(prmf_handle* h) {
     const char* ex = getenv("PRMF_XCHG");
     // [in-kernel pull exchange wanted | persistent step kernel possible | pass-2 chunks | chunks^2]: the push exchange of
     // the persistent kernel pairs CTA c of every rank, so all ranks must split the genes the same way
-    const double mine[4] = {(h->use_epi && ex && atoi(ex) == 1) ? 1.0 : 0.0, h->use_block ? 1.0 : 0.0, (double)h->tchunks,
-                            (double)h->tchunks * h->tchunks};
+    const double mine[4] = {(h->use_epi && ex && atoi(ex) == 1) ? 1.0 : 0.0, h->use_block ? 1.0 : 0.0, (double)h->chunks,
+                            (double)h->chunks * h->chunks};
     CU(cudaMemcpyAsync(h->scal_part, mine, sizeof mine, cudaMemcpyHostToDevice, h->stream));
     int rc = allreduce(h, h->scal_part, 4);
     if (rc) return rc;
@@ -2190,8 +2051,7 @@ int prmf_project_t(prmf_handle* h, double* B_out) {
     if (rc) return rc;
     const int64_t cnt = h->n * h->k;
     double* dst = h->Vbuf[h->vcur ^ 1];                // scratch: the second V buffer is free between steps
-    sum_chunks_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, h->stream>>>(
-        h->Bpart, h->x_tf32 ? h->tc_chunks2 : h->use_tma ? h->tchunks : h->chunks, cnt, dst);
+    sum_chunks_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, h->stream>>>(h->Bpart, b_chunks(h), cnt, dst);
     LAUNCH_CHECK("sum_chunks_kernel");
     CU(cudaMemcpyAsync(B_out, dst, sizeof(double) * cnt, cudaMemcpyDeviceToHost, h->stream));
     CU(cudaStreamSynchronize(h->stream));
@@ -2303,12 +2163,6 @@ int prmf_debug_inject_fault(prmf_handle* h, int kind) {
 }
 
 void* prmf_stream(const prmf_handle* h) { return h ? (void*)h->stream : nullptr; }
-
-#ifdef PRMF_FUSED_TIMING
-int prmf_debug_fused(unsigned long long* out32) {
-    return cudaMemcpyFromSymbol(out32, g_fused_dbg, sizeof(unsigned long long) * 32) == cudaSuccess ? 0 : -1;
-}
-#endif
 
 #ifdef PRMF_TAIL_TIMING
 int prmf_debug_timeline(unsigned long long* out256, int reset) {

@@ -211,40 +211,6 @@ def test_standalone_objective_matches_oracle():
     assert list(got) == ["recon", "manifold", "ignore", "fro", "gamma", "delta", "obj"]
 
 
-# ---- single-pass fused X kernel (opt-in, PRMF_FUSED=1): same results as the two-pass path ----------------
-@pytest.mark.parametrize("m,n,k,P", [
-    (64, 256, 6, 8),
-    (37, 131, 3, 5),
-    (5, 33, 1, 3),
-    (130, 1030, 7, 9),      # 3 gene panels
-    (200, 517, 10, 12),     # k = 10: two factors through the DFMA + butterfly path
-    (333, 2100, 9, 6),      # k = 9, 5 panels
-    (1000, 6750, 10, 20),   # the benchmark's gene count: 14 panels x 10 groups
-])
-def test_fused_kernel_matches_oracle(monkeypatch, m, n, k, P):
-    from prmf_b200 import nmf_manifold_vec_update
-    monkeypatch.setenv("PRMF_FUSED", "1")
-    X, nodelist, Gs, U, V, active = _instance(m, n, k, P, seed=m + n + k, weighted=True)
-    gamma, delta = 2.5, 0.3
-    Uo, Vo, parts_o, _, _, _ = oracle_block(X, U, V, Gs, nodelist, active, 3, gamma, delta)
-    import contextlib, io
-    with contextlib.redirect_stdout(io.StringIO()):
-        Ug, Vg, od = nmf_manifold_vec_update(X, U, V, Gs, active, n_steps=3, gamma=gamma, delta=delta,
-                                             nodelist=nodelist)
-    np.testing.assert_allclose(Ug, Uo, rtol=1e-10, atol=1e-13)
-    np.testing.assert_allclose(Vg, Vo, rtol=1e-10, atol=1e-13)
-    for key, col in (("recon", 0), ("manifold", 1), ("ignore", 2), ("fro", 3), ("obj", 4)):
-        np.testing.assert_allclose(od[key], parts_o[-1, col], rtol=1e-9, atol=1e-12)
-
-
-@pytest.mark.parametrize("case", ["test1_norm", "small_planted"])
-def test_fused_whole_loop_matches_reference_fixture(monkeypatch, case):
-    monkeypatch.setenv("PRMF_FUSED", "1")
-    g = load_golden(case)
-    U, V, od, trace, _ = run_product(g)
-    check_run_against_golden(g, U, V, od, trace)
-
-
 @pytest.mark.parametrize("k", [6, 12])          # fused-tail path (k <= 10) and the separate-kernel path
 def test_speculative_pass_is_bitwise_neutral(k):
     """prmf_block_end(prefetch=1) starts the next step's X.V pass (and U update) before the host has the score
@@ -282,13 +248,13 @@ def test_speculative_pass_is_bitwise_neutral(k):
 
 
 # ---- the launch-structure switches must not change results ----------------------------------------------
-@pytest.mark.parametrize("env", [{"PRMF_EPI": "0"}, {"PRMF_BLOCK": "1"}, {"PRMF_TMA": "0"}])
+@pytest.mark.parametrize("env", [{"PRMF_EPI": "0"}, {"PRMF_BLOCK": "1"}, {"PRMF_TMA_STAGES": "2"}])
 @pytest.mark.parametrize("m,n,k,P", [(200, 517, 10, 12), (1000, 6750, 10, 20), (37, 131, 3, 5)] +
-                         [(48, 97 + 10 * k, k, 6) for k in (1, 2, 4, 5, 6, 7, 8, 9)])    # every K of the three paths
+                         [(48, 97 + 10 * k, k, 6) for k in (1, 2, 4, 5, 6, 7, 8, 9)])    # every K of the fused tails
 def test_launch_structure_switches(monkeypatch, env, m, n, k, P):
     """PRMF_EPI=0: separate U / V-update launches instead of the fused tails (the path of ranks without rows);
     PRMF_BLOCK=1: the persistent step kernel (the default of sharded runs) on one GPU instead of two fused-tail launches
-    per inner step; PRMF_TMA=0: the pre-TMA X-stream kernel."""
+    per inner step; PRMF_TMA_STAGES=2: the fused-tail X-stream kernels with a ring that wraps every two stages."""
     from prmf_b200 import nmf_manifold_vec_update
     for key, val in env.items():
         monkeypatch.setenv(key, val)
