@@ -54,9 +54,14 @@ int prmf_destroy(prmf_handle* h);
  * PRMF_X_TF32 (opt-in; BASELINE config 5, "dense-enough contraction for the tensor-core path") keeps X and X^T
  * in HBM as fp32 rounded to tf32 and runs X.V (:420) and X^T.U (:424) on the tcgen05 tensor cores with fp32
  * accumulation in TMEM; U, V, the updates, the objective and the reductions over ranks stay fp64.  Not bit-parity
- * with the reference: the tests state its tolerance. */
+ * with the reference: the tests state its tolerance.
+ * PRMF_X_F32 (opt-in) keeps X and X^T in HBM as exact fp32 values (half the bytes of PRMF_X_F64) and streams them
+ * through the same fp64 DFMA kernels, widening each element exactly before its first use.  Given X32, an f32 handle
+ * returns bit for bit what a PRMF_X_F64 handle returns given X32 widened to fp64.  Single rank only: m_local must
+ * equal m_global, and prmf_comm_init / prmf_p2p_attach return PRMF_ERR_STATE. */
 #define PRMF_X_F64  0
 #define PRMF_X_TF32 1
+#define PRMF_X_F32  2
 int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_global, int64_t n, int k,
                    void* stream, int x_dtype);
 int prmf_x_dtype(const prmf_handle* h);
@@ -69,8 +74,9 @@ const char* prmf_last_error(const prmf_handle* h);
  * layout on the handle's stream).  X argument of nmf_pathway / nmf_manifold_vec_update (:556,:374). */
 int prmf_set_X(prmf_handle* h, const double* X_host, int64_t ld);
 int prmf_set_X_device(prmf_handle* h, const double* X_dev, int64_t ld);
-/* PRMF_X_TF32 handles only: fp32 source (host pointer, or device pointer when on_device != 0), `ld` floats
- * between rows; the fp64 entry points above also work in that mode (the values are rounded on the device). */
+/* PRMF_X_TF32 and PRMF_X_F32 handles only: fp32 source (host pointer, or device pointer when on_device != 0), `ld`
+ * floats between rows, stored exactly (PRMF_X_F32) or rounded to tf32.  The fp64 entry points above also work in
+ * those modes: the values are rounded on the device, to tf32 or to the nearest fp32 value. */
 int prmf_set_X_f32(prmf_handle* h, const float* X, int64_t ld, int on_device);
 
 /* Global ||X||_F^2 (all-reduced when a communicator is attached); `np.linalg.norm(X)` at :640. */
@@ -204,7 +210,7 @@ int prmf_project_t(prmf_handle* h, double* B_out);
  * capacity (min(#equations, #unknowns, 1024) columns), -3 the Gram matrix of the passive columns lost positive
  * definiteness.  iter_out[k] (may be NULL): the iterations of each problem as scipy counts them (one per outer
  * iteration, including the last one that finds the optimum, and one per step back).  A problem with status -2 or -3 leaves a message in prmf_last_error; the call still returns PRMF_OK.
- * Repeated calls return bitwise-identical results.  Needs X; fp64, single-rank handles only (PRMF_ERR_STATE otherwise).
+ * Repeated calls return bitwise-identical results.  Needs X; fp64 or f32, single-rank handles only (PRMF_ERR_STATE otherwise).
  * U and V of the handle are unset afterwards: calls that read them fail with PRMF_ERR_STATE until prmf_set_UV gives
  * them again. */
 int prmf_nnls_x(prmf_handle* h, int transpose, const double* B_host, int maxiter, double* x_out, double* rnorm_out,

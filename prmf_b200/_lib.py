@@ -10,7 +10,7 @@ OBJ_STRIDE = 8
 UNIQUE_ID_BYTES = 128
 IPC_HANDLE_BYTES = 64
 N_PHASES = 6
-X_DTYPES = {"f64": 0, "tf32": 1}          # PRMF_X_F64 / PRMF_X_TF32
+X_DTYPES = {"f64": 0, "tf32": 1, "f32": 2}          # PRMF_X_F64 / PRMF_X_TF32 / PRMF_X_F32
 PHASES = ("xv", "u_update", "xtu", "reduce", "v_update", "objective")
 
 # every symbol include/prmf_b200.h declares: name -> (restype, argtypes)

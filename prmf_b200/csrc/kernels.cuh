@@ -125,15 +125,24 @@ __device__ __forceinline__ void block_sum_multi(double (&v)[NV], double* scratch
 // ----------------------------------------------------------------------------------------------------
 // ||X||_F^2  (np.linalg.norm(X), :640) : per-block partials, summed in order by sum_partials_kernel
 // ----------------------------------------------------------------------------------------------------
-static __global__ void __launch_bounds__(256) sumsq_kernel(const double* __restrict__ X, int64_t ldx, int64_t m,
+// T = double (fp64 X, and U in prmf_objective) or float (fp32 X, PRMF_X_F32: squares of widened values, same order)
+__device__ __forceinline__ double2 ld_stream_pair(const double* p) { return ld_stream(p); }
+__device__ __forceinline__ double2 ld_stream_pair(const float* p) {
+    float2 r;
+    asm volatile("ld.global.nc.L1::no_allocate.v2.f32 {%0, %1}, [%2];" : "=f"(r.x), "=f"(r.y) : "l"(p));
+    return make_double2((double)r.x, (double)r.y);
+}
+
+template <typename T>
+static __global__ void __launch_bounds__(256) sumsq_kernel(const T* __restrict__ X, int64_t ldx, int64_t m,
                                                     int n2, double* __restrict__ part) {
     __shared__ double scratch[32];
     double acc = 0.0;
     for (int64_t row = blockIdx.x; row < m; row += gridDim.x) {
-        const double* xr = X + row * ldx;
+        const T* xr = X + row * ldx;
         double a = 0.0;
         for (int j = threadIdx.x * 2; j < n2; j += blockDim.x * 2) {
-            double2 x = ld_stream(xr + j);
+            double2 x = ld_stream_pair(xr + j);
             a = fma(x.x, x.x, a);
             a = fma(x.y, x.y, a);
         }
@@ -852,18 +861,32 @@ __device__ __forceinline__ void epi_exchange_v_update(const EpiParams& ep, unsig
 }
 
 
-template <int KT, int RS, int EPI>
-__global__ void __launch_bounds__(kTmaThreads, 1)
-skinny_tma_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_total, int64_t cols,
-                  const double* __restrict__ W, int panel_w, int64_t rows_per_chunk, int stages,
-                  double* __restrict__ OutPart, const EpiParams ep) {
+// ----------------------------------------------------------------------------------------------------
+// X-stream kernels (k <= 10).  The body is shared by the fp64 storage mode (T = double) and the fp32 storage mode
+// (T = float, skinny_tma_f32_kernel): an fp32 element is widened to fp64 exactly before its DFMA, so every column runs
+// the same fma chain in the same row order on the same values, and the fp32 kernel returns, bit for bit, what the
+// fp64 kernel returns on the widened matrix under the same launch plan.
+// ----------------------------------------------------------------------------------------------------
+// the two consecutive elements i = 2p, 2p + 1 of a shared-memory row, as fp64
+__device__ __forceinline__ double2 x_pair(const double* row, int p) { return reinterpret_cast<const double2*>(row)[p]; }
+__device__ __forceinline__ double2 x_pair(const float* row, int p) {
+    const float2 v = reinterpret_cast<const float2*>(row)[p];
+    return make_double2((double)v.x, (double)v.y);
+}
+
+template <typename T, int KT, int RS, int EPI>
+__device__ __forceinline__ void
+skinny_tma_body(const T* __restrict__ M, int64_t ldm, int64_t rows_total, int64_t cols,
+                const double* __restrict__ W, int panel_w, int64_t rows_per_chunk, int stages,
+                double* __restrict__ OutPart, const EpiParams& ep, unsigned tid) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
+    constexpr uint32_t XB = (uint32_t)sizeof(T);                          // bytes per stored element of X
     const int panel = blockIdx.x;
     const int64_t chunk = blockIdx.y;
     const int64_t c0 = (int64_t)panel * panel_w;                          // first column of the panel
     const int width = (int)min((int64_t)panel_w, ldm - c0);               // columns held (multiple of 4)
-    const uint32_t row_bytes = (uint32_t)width * 8u;
-    const uint32_t x_stage_bytes = (uint32_t)RS * (uint32_t)panel_w * 8u;
+    const uint32_t row_bytes = (uint32_t)width * XB;
+    const uint32_t x_stage_bytes = (uint32_t)RS * (uint32_t)panel_w * XB;
     const uint32_t w_bytes = (uint32_t)RS * KT * 8u;
     const uint32_t stage_bytes = x_stage_bytes + ((w_bytes + 127u) & ~127u);
     uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem_raw + (size_t)stages * stage_bytes);
@@ -871,10 +894,10 @@ skinny_tma_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_total,
     const int64_t rbeg = chunk * rows_per_chunk;
     const int64_t rend = min(rows_total, rbeg + rows_per_chunk);
     const int nstage_iters = rend > rbeg ? (int)((rend - rbeg + RS - 1) / RS) : 0;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int warp = tid >> 5, lane = tid & 31;
     KT_STAMP_MIN(ep.dbg_slot, 0);
 
-    if (threadIdx.x == 0) {
+    if (tid == 0) {
         for (int s2 = 0; s2 < stages; ++s2) {
             mbar_init(&full_bar[s2], 1);
             mbar_init(&empty_bar[s2], kTmaConsumerWarps);
@@ -901,7 +924,7 @@ skinny_tma_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_total,
             }
             __syncwarp();
             if (lane < rows)
-                bulk_g2s(sx + (size_t)lane * panel_w * 8, M + (r0 + lane) * ldm + c0, row_bytes, &full_bar[s2], pol_x);
+                bulk_g2s(sx + (size_t)lane * panel_w * XB, M + (r0 + lane) * ldm + c0, row_bytes, &full_bar[s2], pol_x);
             if (++s2 == stages) { s2 = 0; phase ^= 1u; }
         }
         return;
@@ -909,7 +932,7 @@ skinny_tma_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_total,
 
     // ===== consumer warps =====
     const int H = panel_w >> 2;                        // double2 columns per half panel
-    const int t = threadIdx.x;                         // 0..255
+    const int t = tid;                         // 0..255
     const bool active = t < H && (2 * t) < width;      // first pair inside the held columns
     const bool active2 = t < H && (2 * (t + H)) < width;
     double acc[4][KT];
@@ -927,9 +950,9 @@ skinny_tma_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_total,
         if (rows == RS) {
 #pragma unroll
             for (int r = 0; r < RS; ++r) {
-                const double2* xrow = reinterpret_cast<const double2*>(sx + (size_t)r * panel_w * 8);
-                const double2 xa = active ? xrow[t] : make_double2(0.0, 0.0);
-                const double2 xb = active2 ? xrow[t + H] : make_double2(0.0, 0.0);
+                const T* xrow = reinterpret_cast<const T*>(sx + (size_t)r * panel_w * XB);
+                const double2 xa = active ? x_pair(xrow, t) : make_double2(0.0, 0.0);
+                const double2 xb = active2 ? x_pair(xrow, t + H) : make_double2(0.0, 0.0);
 #pragma unroll
                 for (int c = 0; c < KT; ++c) {
                     const double u = sw[r * KT + c];
@@ -941,9 +964,9 @@ skinny_tma_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_total,
             }
         } else {
             for (int r = 0; r < rows; ++r) {
-                const double2* xrow = reinterpret_cast<const double2*>(sx + (size_t)r * panel_w * 8);
-                const double2 xa = active ? xrow[t] : make_double2(0.0, 0.0);
-                const double2 xb = active2 ? xrow[t + H] : make_double2(0.0, 0.0);
+                const T* xrow = reinterpret_cast<const T*>(sx + (size_t)r * panel_w * XB);
+                const double2 xa = active ? x_pair(xrow, t) : make_double2(0.0, 0.0);
+                const double2 xb = active2 ? x_pair(xrow, t + H) : make_double2(0.0, 0.0);
 #pragma unroll
                 for (int c = 0; c < KT; ++c) {
                     const double u = sw[r * KT + c];
@@ -980,6 +1003,25 @@ skinny_tma_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_total,
     KT_STAMP_MAX(ep.dbg_slot, 2);
 }
 
+// fp64 X (PRMF_X_F64)
+template <int KT, int RS, int EPI>
+__global__ void __launch_bounds__(kTmaThreads, 1)
+skinny_tma_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_total, int64_t cols,
+                  const double* __restrict__ W, int panel_w, int64_t rows_per_chunk, int stages,
+                  double* __restrict__ OutPart, const EpiParams ep) {
+    skinny_tma_body<double, KT, RS, EPI>(M, ldm, rows_total, cols, W, panel_w, rows_per_chunk, stages, OutPart, ep, threadIdx.x);
+}
+
+// fp32 X (PRMF_X_F32); single rank, so the fused tails are the U update (EPI 1) and the V update (EPI 2) only
+template <int KT, int RS, int EPI>
+__global__ void __launch_bounds__(kTmaThreads, 1)
+skinny_tma_f32_kernel(const float* __restrict__ M, int64_t ldm, int64_t rows_total, int64_t cols,
+                      const double* __restrict__ W, int panel_w, int64_t rows_per_chunk, int stages,
+                      double* __restrict__ OutPart, const EpiParams ep) {
+    static_assert(EPI <= 2, "the fp32 storage mode has no sharded tails");
+    skinny_tma_body<float, KT, RS, EPI>(M, ldm, rows_total, cols, W, panel_w, rows_per_chunk, stages, OutPart, ep, threadIdx.x);
+}
+
 // ----------------------------------------------------------------------------------------------------
 // General-k TMA X-stream kernel (k > 10: BASELINE configs 4 and 5).  Same pipeline as skinny_tma_kernel; the
 // 256 consumer threads are split into FG factor groups of 256/FG threads.  A thread owns 4 columns of a
@@ -989,19 +1031,20 @@ skinny_tma_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_total,
 // reads W indices up to f0 + (RS-1) k + KT - 1, which for f0 < k is <= RS k + KT - 2, inside the RS k + KT doubles
 // of the W slot; groups with f0 >= k read group 0's columns instead.
 // ----------------------------------------------------------------------------------------------------
-template <int KT, int FG, int RS>
-__global__ void __launch_bounds__(kTmaThreads, 1)
-skinny_tma_gen_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_total, int64_t cols,
-                      const double* __restrict__ W, int k, int panel_w, int64_t rows_per_chunk, int stages,
-                      double* __restrict__ OutPart) {
+template <typename T, int KT, int FG, int RS>
+__device__ __forceinline__ void
+skinny_tma_gen_body(const T* __restrict__ M, int64_t ldm, int64_t rows_total, int64_t cols,
+                    const double* __restrict__ W, int k, int panel_w, int64_t rows_per_chunk, int stages,
+                    double* __restrict__ OutPart, unsigned tid) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
+    constexpr uint32_t XB = (uint32_t)sizeof(T);
     constexpr int TG = 256 / FG;                                          // threads per factor group
     const int panel = blockIdx.x;
     const int64_t chunk = blockIdx.y;
     const int64_t c0 = (int64_t)panel * panel_w;
     const int width = (int)min((int64_t)panel_w, ldm - c0);
-    const uint32_t row_bytes = (uint32_t)width * 8u;
-    const uint32_t x_stage_bytes = (uint32_t)RS * (uint32_t)panel_w * 8u;
+    const uint32_t row_bytes = (uint32_t)width * XB;
+    const uint32_t x_stage_bytes = (uint32_t)RS * (uint32_t)panel_w * XB;
     const uint32_t w_bytes = (uint32_t)RS * (uint32_t)k * 8u;
     const uint32_t w_slot = (((uint32_t)RS * (uint32_t)k + KT) * 8u + 127u) & ~127u;   // + KT doubles of slack
     const uint32_t stage_bytes = x_stage_bytes + w_slot;
@@ -1010,9 +1053,9 @@ skinny_tma_gen_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_to
     const int64_t rbeg = chunk * rows_per_chunk;
     const int64_t rend = min(rows_total, rbeg + rows_per_chunk);
     const int nstage_iters = rend > rbeg ? (int)((rend - rbeg + RS - 1) / RS) : 0;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int warp = tid >> 5, lane = tid & 31;
 
-    if (threadIdx.x == 0) {
+    if (tid == 0) {
         for (int s2 = 0; s2 < stages; ++s2) {
             mbar_init(&full_bar[s2], 1);
             mbar_init(&empty_bar[s2], kTmaConsumerWarps);
@@ -1020,7 +1063,7 @@ skinny_tma_gen_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_to
         fence_mbar_init();
     }
     // the slack behind every W slot is read (and discarded) by the last factor group: keep it finite
-    for (int s2 = threadIdx.x; s2 < stages * KT; s2 += blockDim.x)
+    for (int s2 = tid; s2 < stages * KT; s2 += blockDim.x)
         reinterpret_cast<double*>(smem_raw + (size_t)(s2 / KT) * stage_bytes + x_stage_bytes + w_bytes)[s2 % KT] = 0.0;
     __syncthreads();
 
@@ -1041,14 +1084,14 @@ skinny_tma_gen_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_to
             }
             __syncwarp();
             if (lane < rows)
-                bulk_g2s(sx + (size_t)lane * panel_w * 8, M + (r0 + lane) * ldm + c0, row_bytes, &full_bar[s2], pol_x);
+                bulk_g2s(sx + (size_t)lane * panel_w * XB, M + (r0 + lane) * ldm + c0, row_bytes, &full_bar[s2], pol_x);
             if (++s2 == stages) { s2 = 0; phase ^= 1u; }
         }
         return;
     }
 
     const int H = panel_w >> 2;
-    const int fg = threadIdx.x / TG, t = threadIdx.x % TG;
+    const int fg = tid / TG, t = tid % TG;
     const int f0 = fg * KT;                                               // first factor of this thread
     // groups whose factors all lie at or beyond k (k = 33..36, 65..84, 97..112) read group 0's columns, since their
     // own can lie past the W slot; what they compute is never written.  A branch around their loop instead measured
@@ -1069,9 +1112,9 @@ skinny_tma_gen_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_to
         const unsigned char* sx = smem_raw + (size_t)s2 * stage_bytes;
         const double* sw = reinterpret_cast<const double*>(sx + x_stage_bytes) + fr;
         for (int r = 0; r < rows; ++r) {
-            const double2* xrow = reinterpret_cast<const double2*>(sx + (size_t)r * panel_w * 8);
-            const double2 xa = active ? xrow[t] : make_double2(0.0, 0.0);
-            const double2 xb = active2 ? xrow[t + H] : make_double2(0.0, 0.0);
+            const T* xrow = reinterpret_cast<const T*>(sx + (size_t)r * panel_w * XB);
+            const double2 xa = active ? x_pair(xrow, t) : make_double2(0.0, 0.0);
+            const double2 xb = active2 ? x_pair(xrow, t + H) : make_double2(0.0, 0.0);
             const double* wr = sw + r * k;
 #pragma unroll
             for (int c = 0; c < KT; ++c) {
@@ -1097,6 +1140,22 @@ skinny_tma_gen_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_to
                 if (f0 + c < k) out[c] = acc[g][c];
         }
     }
+}
+
+template <int KT, int FG, int RS>
+__global__ void __launch_bounds__(kTmaThreads, 1)
+skinny_tma_gen_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_total, int64_t cols,
+                      const double* __restrict__ W, int k, int panel_w, int64_t rows_per_chunk, int stages,
+                      double* __restrict__ OutPart) {
+    skinny_tma_gen_body<double, KT, FG, RS>(M, ldm, rows_total, cols, W, k, panel_w, rows_per_chunk, stages, OutPart, threadIdx.x);
+}
+
+template <int KT, int FG, int RS>
+__global__ void __launch_bounds__(kTmaThreads, 1)
+skinny_tma_gen_f32_kernel(const float* __restrict__ M, int64_t ldm, int64_t rows_total, int64_t cols,
+                          const double* __restrict__ W, int k, int panel_w, int64_t rows_per_chunk, int stages,
+                          double* __restrict__ OutPart) {
+    skinny_tma_gen_body<float, KT, FG, RS>(M, ldm, rows_total, cols, W, k, panel_w, rows_per_chunk, stages, OutPart, threadIdx.x);
 }
 
 // Xt[j][i] = X[i][j] : the factor of 2 in HBM capacity buys a coalesced, reduction-free pass 1.

@@ -28,11 +28,13 @@ constexpr int kNnlsMaxIter = -1;
 constexpr int kNnlsCapacity = -2;
 constexpr int kNnlsSingular = -3;
 
-// Per-problem state in one workspace (cap = passive capacity, nun = number of unknowns).
+// Per-problem state in one workspace (cap = passive capacity, nun = number of unknowns).  T: element type of the stored
+// X (double, or float for PRMF_X_F32 handles, whose values are widened exactly before any arithmetic).
+template <typename T>
 struct NnlsWork {
     int k = 0, cap = 0;
     int64_t neq = 0, nun = 0;
-    const double* Arows = nullptr;            // column j of A = Arows[j * lda .. + neq)
+    const T* Arows = nullptr;                 // column j of A = Arows[j * lda .. + neq)
     int64_t lda = 0;
     const double* Bt = nullptr;               // [k][neq]
     double* w = nullptr;                      // duals [nun][k] (sum of the X-stream partials)
@@ -57,7 +59,8 @@ __device__ __forceinline__ double nnls_warp_sum(double v) {
 
 // r[e][c] = b_c[e] - sum_q xP[q] a_{pidx[q]}[e] for the running problems (every problem when `all`), 0 otherwise.
 // grid (ceil(neq / 256), k); W has row pitch k.
-__global__ void __launch_bounds__(kNnlsThreads) nnls_resid_kernel(NnlsWork wk, double* __restrict__ W, int all) {
+template <typename T>
+__global__ void __launch_bounds__(kNnlsThreads) nnls_resid_kernel(NnlsWork<T> wk, double* __restrict__ W, int all) {
     const int c = blockIdx.y;
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= wk.neq) return;
@@ -67,7 +70,7 @@ __global__ void __launch_bounds__(kNnlsThreads) nnls_resid_kernel(NnlsWork wk, d
         const int p = wk.np[c];
         const int* pidx = wk.pidx + (int64_t)c * wk.cap;
         const double* xP = wk.xP + (int64_t)c * wk.cap;
-        for (int q = 0; q < p; ++q) r = fma(-xP[q], wk.Arows[(int64_t)pidx[q] * wk.lda + e], r);
+        for (int q = 0; q < p; ++q) r = fma(-xP[q], (double)wk.Arows[(int64_t)pidx[q] * wk.lda + e], r);
     }
     W[e * wk.k + c] = r;
 }
@@ -132,6 +135,14 @@ __device__ void nnls_solve(const double* __restrict__ L, int cap, const double* 
     }
 }
 
+// a . b over n entries, lanes strided by 32 (widened to fp64 first), summed over the warp
+template <typename A, typename B>
+__device__ __forceinline__ double nnls_dot(const A* a, const B* b, int64_t n, int lane) {
+    double s = 0.0;
+    for (int64_t e = lane; e < n; e += 32) s = fma((double)a[e], (double)b[e], s);
+    return nnls_warp_sum(s);
+}
+
 // (value, index) maximum with the first index winning ties
 __device__ __forceinline__ void nnls_argmax_merge(double& v, int& j, double v2, int j2) {
     if (j2 >= 0 && (j < 0 || v2 > v || (v2 == v && j2 < j))) { v = v2; j = j2; }
@@ -143,7 +154,8 @@ __device__ __forceinline__ void nnls_argmax_merge(double& v, int& j, double v2, 
 // passive coefficient that turns non-positive makes the step stop at the boundary and drops it.  Iterations are counted
 // as scipy counts them: one per outer iteration (including the one that finds the optimum) and one per step back.
 // The loop also ends when the passive set reaches the number of equations, as the Fortran original does.
-__global__ void __launch_bounds__(kNnlsThreads) nnls_step_kernel(NnlsWork wk) {
+template <typename T>
+__global__ void __launch_bounds__(kNnlsThreads) nnls_step_kernel(NnlsWork<T> wk) {
     __shared__ double g[kNnlsMaxPassive + 2];
     __shared__ double row[kNnlsMaxPassive];
     __shared__ double y[kNnlsMaxPassive];
@@ -197,12 +209,16 @@ __global__ void __launch_bounds__(kNnlsThreads) nnls_step_kernel(NnlsWork wk) {
         if (enter < 0) { st = kNnlsConverged; break; }
         if (p >= cap) { st = kNnlsCapacity; break; }
         // Gram column of the candidate: a_enter . a_i (i passive), a_enter . a_enter, a_enter . b -- a warp per dot
-        const double* aj = wk.Arows + (int64_t)enter * wk.lda;
+        const T* aj = wk.Arows + (int64_t)enter * wk.lda;
         for (int q = warp; q < p + 2; q += kNnlsThreads / 32) {
-            const double* other = q < p ? wk.Arows + (int64_t)pidx[q] * wk.lda : q == p ? aj : bc;
-            double a = 0.0;
-            for (int64_t e = lane; e < neq; e += 32) a = fma(aj[e], other[e], a);
-            a = nnls_warp_sum(a);
+            double a;
+            if constexpr (sizeof(T) == sizeof(double)) {
+                const double* other = q < p ? wk.Arows + (int64_t)pidx[q] * wk.lda : q == p ? aj : bc;
+                a = nnls_dot(aj, other, neq, lane);
+            } else {                                         // b is fp64, the columns of A are not
+                a = q <= p ? nnls_dot(aj, q < p ? wk.Arows + (int64_t)pidx[q] * wk.lda : aj, neq, lane)
+                           : nnls_dot(aj, bc, neq, lane);
+            }
             if (lane == 0) g[q] = a;
         }
         __syncthreads();

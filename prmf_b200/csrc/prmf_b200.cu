@@ -1,7 +1,7 @@
 // libprmf_b200.so -- C ABI (include/prmf_b200.h) over the sm_100a kernels in kernels.cuh, block.cuh and tf32.cuh.
 // Host orchestration of one PRMF inner step (reference prmf_runner.py:419-449).  Both passes over X are TMA X-stream
-// launches: skinny_tma_kernel<k,kTmaRS,EPI> at k <= 10, skinny_tma_gen_kernel<KT,FG,kTmaRS> at k > 10, or
-// tc_rowdot_kernel in tf32 mode.
+// launches: skinny_tma_kernel<k,kTmaRS,EPI> at k <= 10, skinny_tma_gen_kernel<KT,FG,kTmaRS> at k > 10 (their _f32_
+// twins when X is stored in fp32, PRMF_X_F32), or tc_rowdot_kernel in tf32 mode.
 //
 // k <= 10, fp64 (fused tails, launch_xv_epi / launch_xtu_epi):
 //   skinny_tma_kernel<k,8,1>   A partials = Xt^T.V, then U <- U*A/(U.Gv+U) and Gu in the last CTA of each panel   (:420-422)
@@ -219,9 +219,11 @@ struct prmf_handle {
     unsigned long long small_seq = 0;
     size_t xcount = 0;
 
-    // TF32 tensor-core storage mode (opt-in: prmf_create_ex with PRMF_X_TF32): X, X^T kept as fp32 rounded to tf32,
-    // both passes by tc_rowdot_kernel, everything else unchanged
-    bool x_tf32 = false;
+    // Storage of X and the engine of the two products are separate properties.  x32: X, X^T kept in fp32 (X32, Xt32)
+    // instead of fp64 (X, Xt), in the tf32 mode (rounded to tf32) and the f32 mode (PRMF_X_F32, exact fp32 values).
+    // x_tc: both passes on the tensor cores by tc_rowdot_kernel (tf32 mode); otherwise the DFMA X streams, which read
+    // fp32 tiles in the f32 mode.  Everything else is the same in every mode.
+    bool x32 = false, x_tc = false;
     float *X32 = nullptr, *Xt32 = nullptr, *Vt32 = nullptr, *Ut32 = nullptr;
     int64_t ldx32 = 0, ldxt32 = 0;
     int Kp = 0;
@@ -317,23 +319,29 @@ int set_smem(prmf_handle* h, F kernel, size_t bytes) {
 }
 
 // ---- templated launch dispatch ---------------------------------------------------------------------
-template <int KT>
-int launch_skinny_tma_t(prmf_handle* h, const double* M, int64_t ldm, int64_t rows, int64_t cols, const double* W,
+// the X-stream kernel (k <= 10) for the storage type of M
+template <int KT, int EPI>
+auto tma_kernel(const double*) { return skinny_tma_kernel<KT, kTmaRS, EPI>; }
+template <int KT, int EPI>
+auto tma_kernel(const float*) { return skinny_tma_f32_kernel<KT, kTmaRS, EPI>; }
+
+template <int KT, typename T>
+int launch_skinny_tma_t(prmf_handle* h, const T* M, int64_t ldm, int64_t rows, int64_t cols, const double* W,
                         int panels, int panel_w, int chunks, int64_t rows_per_chunk, size_t smem, double* out) {
     dim3 grid(panels, chunks);
     EpiParams none{};
     none.dbg_slot = -1;
     none.err = h->err_word; none.timeout_ns = h->spin_timeout_ns;
-    CU(cudaFuncSetAttribute(skinny_tma_kernel<KT, kTmaRS, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    skinny_tma_kernel<KT, kTmaRS, 0><<<grid, kTmaThreads, smem, h->stream>>>(M, ldm, rows, cols, W, panel_w,
-                                                                             rows_per_chunk, h->tma_stages, out, none);
+    const auto fn = tma_kernel<KT, 0>(M);
+    CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    fn<<<grid, kTmaThreads, smem, h->stream>>>(M, ldm, rows, cols, W, panel_w, rows_per_chunk, h->tma_stages, out, none);
     return PRMF_OK;
 }
 
 // X-stream kernel with a fused tail (EPI 1: U update, 2: V update, 3: pack for the exchange over ranks).  The CTAs
 // of a panel wait for each other, so the launch is cooperative (all CTAs co-resident or the launch fails).
-template <int KT>
-int launch_skinny_epi_t(prmf_handle* h, int epi, const double* M, int64_t ldm, int64_t rows, int64_t cols,
+template <int KT, typename T>
+int launch_skinny_epi_t(prmf_handle* h, int epi, const T* M, int64_t ldm, int64_t rows, int64_t cols,
                         const double* W, int panels, int panel_w, int chunks, int64_t rows_per_chunk, size_t smem,
                         double* out, const EpiParams& ep_in) {
     dim3 grid(panels, chunks);
@@ -343,12 +351,12 @@ int launch_skinny_epi_t(prmf_handle* h, int epi, const double* M, int64_t ldm, i
                     (void*)&rows_per_chunk, (void*)&stages, (void*)&out, (void*)&ep};
     const void* fn = nullptr;
     switch (epi) {
-        case 1: fn = (const void*)skinny_tma_kernel<KT, kTmaRS, 1>; break;
-        case 2: fn = (const void*)skinny_tma_kernel<KT, kTmaRS, 2>; break;
-        case 3: fn = (const void*)skinny_tma_kernel<KT, kTmaRS, 3>; break;
-        case 4: fn = (const void*)skinny_tma_kernel<KT, kTmaRS, 4>; break;
-        default: return fail(h, PRMF_ERR_STATE, "bad fused-tail id %d", epi);
+        case 1: fn = (const void*)tma_kernel<KT, 1>(M); break;
+        case 2: fn = (const void*)tma_kernel<KT, 2>(M); break;
+        case 3: if constexpr (sizeof(T) == sizeof(double)) fn = (const void*)skinny_tma_kernel<KT, kTmaRS, 3>; break;
+        case 4: if constexpr (sizeof(T) == sizeof(double)) fn = (const void*)skinny_tma_kernel<KT, kTmaRS, 4>; break;
     }
+    if (!fn) return fail(h, PRMF_ERR_STATE, "bad fused-tail id %d", epi);
     CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     // always cooperative: the CTAs of a panel wait for each other, so co-residency must be guaranteed by the driver
     CU(cudaLaunchCooperativeKernel(fn, grid, dim3(kTmaThreads), args, smem, h->stream));
@@ -356,16 +364,22 @@ int launch_skinny_epi_t(prmf_handle* h, int epi, const double* M, int64_t ldm, i
 }
 
 template <int KT, int FG>
-int launch_skinny_gen_t(prmf_handle* h, const double* M, int64_t ldm, int64_t rows, int64_t cols, const double* W,
+auto gen_kernel(const double*) { return skinny_tma_gen_kernel<KT, FG, kTmaRS>; }
+template <int KT, int FG>
+auto gen_kernel(const float*) { return skinny_tma_gen_f32_kernel<KT, FG, kTmaRS>; }
+
+template <int KT, int FG, typename T>
+int launch_skinny_gen_t(prmf_handle* h, const T* M, int64_t ldm, int64_t rows, int64_t cols, const double* W,
                         int panels, int panel_w, int chunks, int64_t rows_per_chunk, size_t smem, double* out) {
     dim3 grid(panels, chunks);
-    CU(cudaFuncSetAttribute(skinny_tma_gen_kernel<KT, FG, kTmaRS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    skinny_tma_gen_kernel<KT, FG, kTmaRS><<<grid, kTmaThreads, smem, h->stream>>>(M, ldm, rows, cols, W, h->k, panel_w,
-                                                                                  rows_per_chunk, h->tma_stages, out);
+    const auto fn = gen_kernel<KT, FG>(M);
+    CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    fn<<<grid, kTmaThreads, smem, h->stream>>>(M, ldm, rows, cols, W, h->k, panel_w, rows_per_chunk, h->tma_stages, out);
     return PRMF_OK;
 }
 
-int launch_skinny_gen(prmf_handle* h, const double* M, int64_t ldm, int64_t rows, int64_t cols, const double* W,
+template <typename T>
+int launch_skinny_gen(prmf_handle* h, const T* M, int64_t ldm, int64_t rows, int64_t cols, const double* W,
                       int panels, int panel_w, int chunks, int64_t rows_per_chunk, size_t smem, double* out) {
 #define GEN_CASE(KT_, FG_) \
     if (h->tma_kt == KT_ && h->tma_fg == FG_) \
@@ -391,8 +405,8 @@ int launch_skinny_gen(prmf_handle* h, const double* M, int64_t ldm, int64_t rows
     }
 
 // number of per-chunk partials the passes leave in Apart / Bpart
-int a_chunks(const prmf_handle* h) { return h->x_tf32 ? h->tc_chunks1 : h->chunks1; }
-int b_chunks(const prmf_handle* h) { return h->x_tf32 ? h->tc_chunks2 : h->chunks; }
+int a_chunks(const prmf_handle* h) { return h->x_tc ? h->tc_chunks1 : h->chunks1; }
+int b_chunks(const prmf_handle* h) { return h->x_tc ? h->tc_chunks2 : h->chunks; }
 
 // TF32 mode: one tensor-core kernel serves both passes
 int launch_tc(prmf_handle* h, const CUtensorMap& tmM, const CUtensorMap& tmW, const TcParams& prm, int tiles, int chunks,
@@ -415,9 +429,15 @@ int refresh_wt(prmf_handle* h, const double* W, int64_t rows, float* Wt, int64_t
 // pass 1: A partials = Xt^T . V   (M = Xt: n rows x m cols)
 int launch_xv(prmf_handle* h) {
     if (h->m == 0) return PRMF_OK;
-    if (h->x_tf32) return launch_tc(h, h->tm_X, h->tm_Vt, h->tc1, h->tc_tiles1, h->tc_chunks1, "tc_rowdot_kernel(pass 1)");
+    if (h->x_tc) return launch_tc(h, h->tm_X, h->tm_Vt, h->tc1, h->tc_tiles1, h->tc_chunks1, "tc_rowdot_kernel(pass 1)");
     int rc = 0;
-    if (h->k > 10) {
+    if (h->x32 && h->k > 10) {
+        rc = launch_skinny_gen(h, h->Xt32, h->ldxt32, h->n, h->m, h->Vbuf[h->vcur], h->panels1, h->panel_w1, h->chunks1,
+                               h->rows_per_chunk1, h->tma_smem1, h->Apart);
+    } else if (h->x32) {
+        KT_SWITCH_RC(h->k, rc, launch_skinny_tma_t, h, h->Xt32, h->ldxt32, h->n, h->m, h->Vbuf[h->vcur], h->panels1,
+                     h->panel_w1, h->chunks1, h->rows_per_chunk1, h->tma_smem1, h->Apart);
+    } else if (h->k > 10) {
         rc = launch_skinny_gen(h, h->Xt, h->ldxt, h->n, h->m, h->Vbuf[h->vcur], h->panels1, h->panel_w1, h->chunks1,
                                h->rows_per_chunk1, h->tma_smem1, h->Apart);
     } else {
@@ -435,13 +455,19 @@ int launch_xtu(prmf_handle* h) {
         CU(cudaMemsetAsync(h->Bpart, 0, sizeof(double) * b_chunks(h) * h->n * h->k, h->stream));
         return PRMF_OK;
     }
-    if (h->x_tf32) {
+    if (h->x_tc) {
         int rc = refresh_wt(h, h->U, h->m, h->Ut32, h->ldxt32);
         if (rc) return rc;
         return launch_tc(h, h->tm_Xt, h->tm_Ut, h->tc2, h->tc_tiles2, h->tc_chunks2, "tc_rowdot_kernel(pass 2)");
     }
     int rc = 0;
-    if (h->k > 10) {
+    if (h->x32 && h->k > 10) {
+        rc = launch_skinny_gen(h, h->X32, h->ldx32, h->m, h->n, h->U, h->panels, h->panel_w, h->chunks, h->rows_per_chunk,
+                               h->tma_smem2, h->Bpart);
+    } else if (h->x32) {
+        KT_SWITCH_RC(h->k, rc, launch_skinny_tma_t, h, h->X32, h->ldx32, h->m, h->n, h->U, h->panels, h->panel_w, h->chunks,
+                     h->rows_per_chunk, h->tma_smem2, h->Bpart);
+    } else if (h->k > 10) {
         rc = launch_skinny_gen(h, h->X, h->ldx, h->m, h->n, h->U, h->panels, h->panel_w, h->chunks, h->rows_per_chunk,
                                h->tma_smem2, h->Bpart);
     } else {
@@ -579,7 +605,7 @@ int launch_v_update_objective(prmf_handle* h, bool sharded, double tradeoff) {
             h->normX_sq, h->Gv, h->gd, tradeoff, h->obj, h->step_counter, h->obj_capacity);
         LAUNCH_CHECK("objective_kernel");
     }
-    if (h->x_tf32) return refresh_wt(h, h->Vbuf[h->vcur], h->n, h->Vt32, h->ldx32);
+    if (h->x_tc) return refresh_wt(h, h->Vbuf[h->vcur], h->n, h->Vt32, h->ldx32);
     return PRMF_OK;
 }
 
@@ -670,8 +696,13 @@ int launch_xv_epi(prmf_handle* h, const double* gv_src = nullptr, int gv_parts =
     ep.gv_parts = gv_src ? gv_parts : 1;
     ep.Gu_part = h->Gu_part;
     int rc = 0;
-    KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, 1, h->Xt, h->ldxt, h->n, h->m, h->Vbuf[h->vcur], h->panels1,
-                 h->panel_w1, h->chunks1, h->rows_per_chunk1, h->tma_smem1, h->Apart, ep);
+    if (h->x32) {
+        KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, 1, h->Xt32, h->ldxt32, h->n, h->m, h->Vbuf[h->vcur], h->panels1,
+                     h->panel_w1, h->chunks1, h->rows_per_chunk1, h->tma_smem1, h->Apart, ep);
+    } else {
+        KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, 1, h->Xt, h->ldxt, h->n, h->m, h->Vbuf[h->vcur], h->panels1,
+                     h->panel_w1, h->chunks1, h->rows_per_chunk1, h->tma_smem1, h->Apart, ep);
+    }
     if (rc) { h->failed = true; return rc; }     // the panel counters expect this launch: no further steps on this handle
     LAUNCH_CHECK("skinny_tma_kernel(pass 1 + U update)");
     std::swap(h->U, h->U2);
@@ -726,8 +757,13 @@ int launch_xtu_epi(prmf_handle* h, int mode, double* packed_dst, int hist_slot =
         ep.Gu_glob = h->Gu_glob;
     }
     int rc = 0;
-    KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, mode, h->X, h->ldx, h->m, h->n, h->U, h->panels, h->panel_w,
-                 h->chunks, h->rows_per_chunk, h->tma_smem2, h->Bpart, ep);
+    if (h->x32) {
+        KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, mode, h->X32, h->ldx32, h->m, h->n, h->U, h->panels, h->panel_w,
+                     h->chunks, h->rows_per_chunk, h->tma_smem2, h->Bpart, ep);
+    } else {
+        KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, mode, h->X, h->ldx, h->m, h->n, h->U, h->panels, h->panel_w,
+                     h->chunks, h->rows_per_chunk, h->tma_smem2, h->Bpart, ep);
+    }
     if (rc) { h->failed = true; return rc; }
     LAUNCH_CHECK(mode == 3 ? "skinny_tma_kernel(pass 2 + pack)" : mode == 4 ? "skinny_tma_kernel(pass 2 + exchange + V update)"
                                                                             : "skinny_tma_kernel(pass 2 + V update)");
@@ -1153,15 +1189,21 @@ int finish_setup_tf32(prmf_handle* h) {
     return PRMF_OK;
 }
 
-// TF32 mode: round a row block (host or device, fp64 or fp32) to tf32 into the fp32 layout.  Host blocks go
-// through a bounded device staging buffer, block after block on the handle's stream.
+// fp32 storage (tf32 and f32 modes): store a row block (host or device, fp64 or fp32) into the fp32 layout, rounded to
+// tf32 in the tf32 mode and to the nearest fp32 value in the f32 mode (exact for fp32 input).  Host blocks go through a
+// bounded device staging buffer, block after block on the handle's stream.
+template <typename T, bool TF32>
+void launch_store_rows(prmf_handle* h, const T* X, int64_t ld, int64_t rows, float* dst) {
+    to_tf32_rows_kernel<T, TF32><<<h->sm_count * 8, 256, 0, h->stream>>>(X, ld, rows, h->n, dst, h->ldx32);
+}
+
 template <typename T>
-int store_tf32(prmf_handle* h, const T* X, int64_t ld, bool on_host) {
+int store_x32(prmf_handle* h, const T* X, int64_t ld, bool on_host) {
     const int64_t m = h->m, n = h->n;
     if (m == 0) return PRMF_OK;
-    const int grid = h->sm_count * 8;
+    auto store = h->x_tc ? launch_store_rows<T, true> : launch_store_rows<T, false>;
     if (!on_host) {
-        to_tf32_rows_kernel<T><<<grid, 256, 0, h->stream>>>(X, ld, m, n, h->X32, h->ldx32);
+        store(h, X, ld, m, h->X32);
         LAUNCH_CHECK("to_tf32_rows_kernel");
         return PRMF_OK;
     }
@@ -1175,19 +1217,20 @@ int store_tf32(prmf_handle* h, const T* X, int64_t ld, bool on_host) {
         e = cudaMemcpy2DAsync(stage, n * sizeof(T), X + r0 * ld, ld * sizeof(T), n * sizeof(T), rows,
                               cudaMemcpyHostToDevice, h->stream);
         if (e != cudaSuccess) break;
-        to_tf32_rows_kernel<T><<<grid, 256, 0, h->stream>>>(stage, n, rows, n, h->X32 + r0 * h->ldx32, h->ldx32);
+        store(h, stage, n, rows, h->X32 + r0 * h->ldx32);
         h->launches++;
         e = cudaGetLastError();
     }
     if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
     cudaFree(stage);
-    if (e != cudaSuccess) return fail(h, PRMF_ERR_CUDA, "TF32 upload of X failed: %s", cudaGetErrorString(e));
+    if (e != cudaSuccess) return fail(h, PRMF_ERR_CUDA, "fp32 upload of X failed: %s", cudaGetErrorString(e));
     return PRMF_OK;
 }
 
 // The Lawson-Hanson loop of prmf_nnls_x over a workspace laid out by the caller (wk).  W: the operand of the X stream
 // that computes the duals (V for A = X^T, pass 1; U for A = X, pass 2); its zero pad rows are left as they are.
-int nnls_loop(prmf_handle* h, int transpose, NnlsWork& wk, double* rnorm_dev, std::vector<int32_t>& status) {
+template <typename T>
+int nnls_loop(prmf_handle* h, int transpose, NnlsWork<T>& wk, double* rnorm_dev, std::vector<int32_t>& status) {
     const int k = wk.k;
     double* W = transpose ? h->Vbuf[h->vcur] : h->U;
     const double* part = transpose ? h->Apart : h->Bpart;
@@ -1219,12 +1262,17 @@ int finish_X(prmf_handle* h) {
     cancel_ahead(h);
     // transposed copy for pass 1, then ||X||^2 partial of this rank, all-reduced once
     const int blocks = h->sm_count * 4;
-    if (h->m > 0 && h->x_tf32) {
+    if (h->m > 0 && h->x32) {
         dim3 tg((unsigned)((h->n + 31) / 32), (unsigned)((h->m + 31) / 32));
         transpose_f32_kernel<<<tg, 256, 0, h->stream>>>(h->X32, h->ldx32, h->m, h->n, h->Xt32, h->ldxt32);
         LAUNCH_CHECK("transpose_f32_kernel");
-        sumsq_f32_kernel<<<blocks, 256, 0, h->stream>>>(h->X32, h->ldx32, h->m, h->n, h->scal_part);
-        LAUNCH_CHECK("sumsq_f32_kernel");
+        if (h->x_tc) {
+            sumsq_f32_kernel<<<blocks, 256, 0, h->stream>>>(h->X32, h->ldx32, h->m, h->n, h->scal_part);
+            LAUNCH_CHECK("sumsq_f32_kernel");
+        } else {                    // f32 mode: the order of the fp64 mode, so ||X||^2 is that of the widened matrix
+            sumsq_kernel<<<blocks, 256, 0, h->stream>>>(h->X32, h->ldx32, h->m, h->n2, h->scal_part);
+            LAUNCH_CHECK("sumsq_kernel");
+        }
         sum_partials_kernel<<<1, 256, 0, h->stream>>>(h->scal_part, blocks, h->normX_sq);
         LAUNCH_CHECK("sum_partials_kernel");
     } else if (h->m > 0) {
@@ -1246,6 +1294,89 @@ int finish_X(prmf_handle* h) {
     return PRMF_OK;
 }
 
+// prmf_nnls_x after its checks, on the columns of A = Arows[j * lda ..] (rows of X or of its transposed copy)
+template <typename T>
+int nnls_x_run(prmf_handle* h, int transpose, const T* Arows, int64_t lda, const double* B_host, int maxiter,
+               double* x_out, double* rnorm_out, int32_t* status_out, int32_t* iter_out) {
+    NnlsWork<T> wk;
+    wk.k = h->k;
+    wk.neq = transpose ? h->n : h->m;
+    wk.nun = transpose ? h->m : h->n;
+    wk.Arows = Arows;
+    wk.lda = lda;
+    wk.cap = (int)std::min<int64_t>({wk.neq, wk.nun, (int64_t)kNnlsMaxPassive});
+    wk.maxiter = maxiter > 0 ? maxiter : (int)std::min<int64_t>(3 * wk.nun, INT32_MAX - 1);   // scipy: 3 * #unknowns
+    wk.tol = 10.0 * (double)std::max(wk.neq, wk.nun) * DBL_EPSILON;                          // 10 max(m, n) eps
+    const int k = wk.k;
+    const size_t cap = (size_t)wk.cap, kk = (size_t)k;
+    auto pad = [](size_t bytes) { return (bytes + 255) & ~(size_t)255; };
+    const size_t d = sizeof(double);
+    const size_t b_bt = pad(d * kk * wk.neq), b_w = pad(d * kk * wk.nun), b_g = pad(d * kk * cap * cap);
+    const size_t b_vec = pad(d * kk * cap), b_idx = pad(sizeof(int) * kk * cap), b_flag = pad(kk * wk.nun);
+    const size_t b_small = pad(sizeof(int) * kk), b_rn = pad(d * kk);
+    const size_t total = b_bt + b_w + 2 * b_g + 2 * b_vec + b_idx + b_flag + 3 * b_small + b_rn;
+    unsigned char* ws = nullptr;
+    cudaError_t ea = g_pool.alloc((void**)&ws, total, h->device);
+    if (ea != cudaSuccess) return fail(h, PRMF_ERR_NOMEM, "cudaMalloc of %zu bytes failed: %s", total, cudaGetErrorString(ea));
+    size_t off = 0;
+    auto take = [&](size_t bytes) { unsigned char* p = ws + off; off += bytes; return p; };
+    wk.Bt = (const double*)take(b_bt);
+    wk.w = (double*)take(b_w);
+    wk.G = (double*)take(b_g);
+    wk.L = (double*)take(b_g);
+    wk.atb = (double*)take(b_vec);
+    unsigned char* zero_from = ws + off;               // everything from here on starts at zero
+    wk.xP = (double*)take(b_vec);
+    wk.pidx = (int*)take(b_idx);
+    wk.flag = (int8_t*)take(b_flag);
+    wk.np = (int*)take(b_small);
+    wk.iter = (int*)take(b_small);
+    wk.status = (int*)take(b_small);
+    double* rnorm_dev = (double*)take(b_rn);
+
+    std::vector<double> Bt((size_t)k * wk.neq);
+    for (int64_t e = 0; e < wk.neq; ++e)
+        for (int c = 0; c < k; ++c) Bt[(size_t)c * wk.neq + e] = B_host[e * k + c];
+    std::vector<int32_t> status(k, kNnlsRunning), np_h(k), pidx_h(kk * cap);
+    std::vector<double> xP_h(kk * cap);
+    int rc = PRMF_OK;
+    cudaError_t e = cudaMemcpyAsync((void*)wk.Bt, Bt.data(), sizeof(double) * Bt.size(), cudaMemcpyHostToDevice, h->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(zero_from, 0, (size_t)(ws + total - zero_from), h->stream);
+    if (e != cudaSuccess) rc = fail(h, PRMF_ERR_CUDA, "prmf_nnls_x upload: %s", cudaGetErrorString(e));
+    if (!rc) rc = nnls_loop(h, transpose, wk, rnorm_dev, status);
+    if (!rc) {
+        e = cudaMemcpyAsync(np_h.data(), wk.np, sizeof(int32_t) * k, cudaMemcpyDeviceToHost, h->stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(pidx_h.data(), wk.pidx, sizeof(int32_t) * kk * cap, cudaMemcpyDeviceToHost, h->stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(xP_h.data(), wk.xP, sizeof(double) * kk * cap, cudaMemcpyDeviceToHost, h->stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(status_out, wk.status, sizeof(int32_t) * k, cudaMemcpyDeviceToHost, h->stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(rnorm_out, rnorm_dev, sizeof(double) * k, cudaMemcpyDeviceToHost, h->stream);
+        if (e == cudaSuccess && iter_out)
+            e = cudaMemcpyAsync(iter_out, wk.iter, sizeof(int32_t) * k, cudaMemcpyDeviceToHost, h->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+        if (e != cudaSuccess) rc = fail(h, PRMF_ERR_CUDA, "prmf_nnls_x read-back: %s", cudaGetErrorString(e));
+    } else {
+        cudaStreamSynchronize(h->stream);
+    }
+    g_pool.release(ws, total, h->device);
+    if (rc) return rc;
+    std::fill(x_out, x_out + wk.nun * k, 0.0);
+    for (int c = 0; c < k; ++c)
+        for (int q = 0; q < np_h[c]; ++q) x_out[(int64_t)pidx_h[c * cap + q] * k + c] = xP_h[c * cap + q];
+    h->err.clear();
+    for (int c = 0; c < k; ++c) {
+        if (status_out[c] == kNnlsCapacity) {
+            fail(h, PRMF_OK, "prmf_nnls_x: problem %d needs more than %d passive columns (the workspace capacity)", c,
+                 wk.cap);
+            break;
+        }
+        if (status_out[c] == kNnlsSingular) {
+            fail(h, PRMF_OK, "prmf_nnls_x: problem %d: the Gram matrix of its passive columns lost positive definiteness", c);
+            break;
+        }
+    }
+    return PRMF_OK;
+}
+
 }  // namespace
 
 // =====================================================================================================
@@ -1262,13 +1393,17 @@ int prmf_create(prmf_handle** out, int device, int64_t m_local, int64_t m_global
 int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_global, int64_t n, int k, void* stream,
                    int x_dtype) {
     prmf_handle* h = nullptr;
-    if (x_dtype != PRMF_X_F64 && x_dtype != PRMF_X_TF32) return fail(h, PRMF_ERR_ARG, "unknown x_dtype %d", x_dtype);
+    if (x_dtype != PRMF_X_F64 && x_dtype != PRMF_X_TF32 && x_dtype != PRMF_X_F32)
+        return fail(h, PRMF_ERR_ARG, "unknown x_dtype %d", x_dtype);
     if (!out) return fail(h, PRMF_ERR_ARG, "out is NULL");
     *out = nullptr;
     if (m_local < 0 || n <= 0 || k <= 0 || m_global < m_local)
         return fail(h, PRMF_ERR_ARG, "bad shape m_local=%lld m_global=%lld n=%lld k=%d", (long long)m_local,
                     (long long)m_global, (long long)n, k);
     if (k > 128) return fail(h, PRMF_ERR_ARG, "k=%d not supported (max 128)", k);
+    if (x_dtype == PRMF_X_F32 && m_local != m_global)
+        return fail(h, PRMF_ERR_ARG, "PRMF_X_F32 handles are single-rank (m_local=%lld, m_global=%lld)", (long long)m_local,
+                    (long long)m_global);
     if (n > (int64_t)1 << 30) return fail(h, PRMF_ERR_ARG, "n too large");
     int ndev = 0;
     cudaError_t e = cudaGetDeviceCount(&ndev);
@@ -1317,7 +1452,11 @@ int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_glo
         h->vu_rows = 32;
         h->vu_grid = (int)std::max<int64_t>(1, std::min<int64_t>(h->sm_count, (n + 31) / 32));
     }
-    // X-stream plan: one CTA per SM, column panels of at most 1024 / FG columns, row chunks of at least 4 stages
+    h->x32 = x_dtype != PRMF_X_F64;
+    h->x_tc = x_dtype == PRMF_X_TF32;
+    // X-stream plan: one CTA per SM, column panels of at most 1024 / FG columns, row chunks of at least 4 stages.  The
+    // panels and chunks do not depend on the storage type, which is what makes an fp32 handle bitwise equal to an fp64
+    // handle on the widened matrix; only the ring differs (an fp32 stage holds half the bytes of X).
     if (k > 10) {                          // general-k kernel: FG factor groups x KT factors per thread
         const int groups = (k + 15) / 16;
         h->tma_fg = groups <= 1 ? 1 : groups <= 2 ? 2 : groups <= 4 ? 4 : 8;
@@ -1334,7 +1473,7 @@ int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_glo
             // rows per chunk: even (the W rows of a chunk must start 16-byte aligned for the bulk copies), not a multiple
             // of the stage height -- a ragged last stage costs less than a last chunk that is nearly empty
             *rpc = round_up(std::max<int64_t>(1, (rows + *chunks - 1) / *chunks), 2);
-            const size_t xb = (size_t)kTmaRS * *panel_w * 8;
+            const size_t xb = (size_t)kTmaRS * *panel_w * (h->x32 ? 4 : 8);
             const size_t wb = (((size_t)kTmaRS * k + 16) * 8 + 127) & ~(size_t)127;
             *smem = h->tma_stages * (xb + wb) + 2 * h->tma_stages * sizeof(uint64_t);
         };
@@ -1343,9 +1482,10 @@ int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_glo
             plan(n, m_local, &h->panels, &h->panel_w, &h->chunks, &h->rows_per_chunk, &h->tma_smem2);
             return std::max(h->tma_smem1, h->tma_smem2) <= 220 * 1024;
         };
-        // the default ring fits at every k <= 128 (tests/test_xstream_exact.py); a PRMF_TMA_STAGES override is kept
-        // where its ring fits as well, and the handle runs the default elsewhere
-        const int default_stages = h->tma_fg >= 4 ? 6 : h->tma_fg == 2 ? 4 : 3;
+        // the default ring fits at every k <= 128 (tests/test_xstream_exact.py, tests/test_f32_storage.py); a
+        // PRMF_TMA_STAGES override is kept where its ring fits as well, and the handle runs the default elsewhere.  fp32
+        // tiles: twice the stages, the same bytes of X in flight.
+        const int default_stages = (h->tma_fg >= 4 ? 6 : h->tma_fg == 2 ? 4 : 3) * (h->x32 ? 2 : 1);
         const char* es = getenv("PRMF_TMA_STAGES");
         const int want = es ? atoi(es) : 0;
         h->tma_stages = want >= 2 && want <= 12 ? want : default_stages;
@@ -1355,11 +1495,14 @@ int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_glo
         }
     }
 
-    h->x_tf32 = x_dtype == PRMF_X_TF32;
-    if (h->x_tf32) setup_tf32(h);
+    if (h->x_tc) setup_tf32(h);
+    if (h->x32 && !h->x_tc) {
+        h->ldx32 = round_up(n, 32);
+        h->ldxt32 = round_up(std::max<int64_t>(1, m_local), 32);
+    }
     {
         const char* ee = getenv("PRMF_EPI");
-        h->use_epi = !(ee && atoi(ee) == 0) && k <= 10 && m_local > 0 && !h->x_tf32 &&
+        h->use_epi = !(ee && atoi(ee) == 0) && k <= 10 && m_local > 0 && !h->x_tc &&
                      h->panels1 * h->chunks1 <= h->sm_count && h->panels * h->chunks <= h->sm_count;
         if (h->use_epi) {
             // the last CTA of a panel reuses the ring for Gv/Gu, the slice sums and the panel's new rows
@@ -1406,12 +1549,15 @@ int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_glo
         cudaError_t eb_ = g_pool.alloc((void**)&ptr, bytes_, device);                                                \
         if (eb_ != cudaSuccess) { ptr = nullptr; rc = fail(h, PRMF_ERR_NOMEM, "cudaMalloc of %zu bytes failed: %s", bytes_, cudaGetErrorString(eb_)); } \
     }
-    if (h->x_tf32) {
+    if (h->x32) {
         ALLOC_BIG(h->X32, float, (size_t)std::max<int64_t>(1, m_local) * h->ldx32);
         ALLOC_BIG(h->Xt32, float, (size_t)n * h->ldxt32);
+    }
+    if (h->x_tc) {
         ALLOC(h->Vt32, (size_t)h->Kp * h->ldx32);
         ALLOC(h->Ut32, (size_t)h->Kp * h->ldxt32);
-    } else {
+    }
+    if (!h->x32) {
         ALLOC_BIG(h->X, double, (size_t)std::max<int64_t>(1, m_local) * h->ldx);
         ALLOC_BIG(h->Xt, double, (size_t)n * h->ldxt);
     }
@@ -1442,8 +1588,8 @@ int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_glo
     TAKE(h->obj, double, (size_t)h->obj_capacity * kObjStride);
 #undef TAKE
 #undef ALLOC
-    if (!rc && h->x_tf32) {
-        cudaMemsetAsync(h->Xt32, 0, sizeof(float) * n * h->ldxt32, h->stream);
+    if (!rc && h->x32) cudaMemsetAsync(h->Xt32, 0, sizeof(float) * n * h->ldxt32, h->stream);
+    if (!rc && h->x_tc) {
         cudaMemsetAsync(h->Vt32, 0, sizeof(float) * h->Kp * h->ldx32, h->stream);
         cudaMemsetAsync(h->Ut32, 0, sizeof(float) * h->Kp * h->ldxt32, h->stream);
         rc = finish_setup_tf32(h);
@@ -1488,7 +1634,8 @@ int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_glo
         h->blk_stage_bytes = (uint32_t)((size_t)kBlkRS * std::max(h->panel_w1, h->panel_w) * 8 + wb);
         h->blk_smem = (size_t)h->tma_stages * h->blk_stage_bytes + 2 * h->tma_stages * sizeof(uint64_t) +
                       sizeof(double) * (256 + 8 * (size_t)k * k + (size_t)kBlkRowsCap * k);
-        h->use_block = h->use_epi && h->defer_ok && !(eb && atoi(eb) == 0) && h->blk_smem <= 227 * 1024;
+        // (block_kernel streams fp64 X: not for fp32 storage, where PRMF_BLOCK=1 is ignored)
+        h->use_block = h->use_epi && h->defer_ok && !h->x32 && !(eb && atoi(eb) == 0) && h->blk_smem <= 227 * 1024;
         h->block_forced = eb && atoi(eb) == 1;
         h->err_host = pinned_word();
     }
@@ -1550,8 +1697,8 @@ int prmf_set_X(prmf_handle* h, const double* X_host, int64_t ld) {
     if (!h) return PRMF_ERR_ARG;
     if ((!X_host && h->m > 0) || ld < h->n) return fail(h, PRMF_ERR_ARG, "prmf_set_X: bad pointer or ld < n");
     CU(cudaSetDevice(h->device));
-    if (h->x_tf32) {
-        int rc = store_tf32<double>(h, X_host, ld, true);
+    if (h->x32) {
+        int rc = store_x32<double>(h, X_host, ld, true);
         return rc ? rc : finish_X(h);
     }
     if (h->m > 0) {
@@ -1566,8 +1713,8 @@ int prmf_set_X_device(prmf_handle* h, const double* X_dev, int64_t ld) {
     if (!h) return PRMF_ERR_ARG;
     if ((!X_dev && h->m > 0) || ld < h->n) return fail(h, PRMF_ERR_ARG, "prmf_set_X_device: bad pointer or ld < n");
     CU(cudaSetDevice(h->device));
-    if (h->x_tf32) {
-        int rc = store_tf32<double>(h, X_dev, ld, false);
+    if (h->x32) {
+        int rc = store_x32<double>(h, X_dev, ld, false);
         return rc ? rc : finish_X(h);
     }
     if (h->m > 0) {
@@ -1580,14 +1727,17 @@ int prmf_set_X_device(prmf_handle* h, const double* X_dev, int64_t ld) {
 
 int prmf_set_X_f32(prmf_handle* h, const float* X, int64_t ld, int on_device) {
     if (!h) return PRMF_ERR_ARG;
-    if (!h->x_tf32) return fail(h, PRMF_ERR_STATE, "prmf_set_X_f32 needs a handle created with PRMF_X_TF32");
+    if (!h->x32) return fail(h, PRMF_ERR_STATE, "prmf_set_X_f32 needs a handle created with PRMF_X_TF32 or PRMF_X_F32");
     if ((!X && h->m > 0) || ld < h->n) return fail(h, PRMF_ERR_ARG, "prmf_set_X_f32: bad pointer or ld < n");
     CU(cudaSetDevice(h->device));
-    int rc = store_tf32<float>(h, X, ld, on_device == 0);
+    int rc = store_x32<float>(h, X, ld, on_device == 0);
     return rc ? rc : finish_X(h);
 }
 
-int prmf_x_dtype(const prmf_handle* h) { return h && h->x_tf32 ? PRMF_X_TF32 : PRMF_X_F64; }
+int prmf_x_dtype(const prmf_handle* h) {
+    if (!h || !h->x32) return PRMF_X_F64;
+    return h->x_tc ? PRMF_X_TF32 : PRMF_X_F32;
+}
 
 int prmf_get_normX_sq(prmf_handle* h, double* out) {
     if (!h || !out) return PRMF_ERR_ARG;
@@ -1699,7 +1849,7 @@ int prmf_set_UV(prmf_handle* h, const double* U_local, const double* V) {
         CU(cudaMemcpyAsync(h->Vbuf[h->vcur], V, sizeof(double) * nk, cudaMemcpyHostToDevice, h->stream));
         int rc = recompute_Gv(h);
         if (rc) return rc;
-        if (h->x_tf32 && (rc = refresh_wt(h, h->Vbuf[h->vcur], h->n, h->Vt32, h->ldx32))) return rc;
+        if (h->x_tc && (rc = refresh_wt(h, h->Vbuf[h->vcur], h->n, h->Vt32, h->ldx32))) return rc;
     }
     CU(cudaStreamSynchronize(h->stream));
     if (U_local || h->m == 0) h->have_U = true;          // a handle without rows has no U to set
@@ -1817,7 +1967,7 @@ int prmf_restore_best(prmf_handle* h) {
     const int64_t nk = h->n * h->k;
     CU(cudaMemcpyAsync(h->Vbuf[h->vcur], h->Vb, sizeof(double) * nk, cudaMemcpyDeviceToDevice, h->stream));
     CU(cudaMemcpyAsync(h->Gv, h->Gvb, sizeof(double) * h->k * h->k, cudaMemcpyDeviceToDevice, h->stream));
-    if (h->x_tf32) {
+    if (h->x_tc) {
         int rc = refresh_wt(h, h->Vbuf[h->vcur], h->n, h->Vt32, h->ldx32);
         if (rc) return rc;
     }
@@ -1834,7 +1984,7 @@ int prmf_residual_sq(prmf_handle* h, double* out) {
     int rc = dalloc(h, &d, 1);
     if (rc) return rc;
     if (h->m > 0) {
-        if (h->x_tf32)
+        if (h->x32)
             residual_f32_kernel<<<blocks, 256, 0, h->stream>>>(h->X32, h->ldx32, h->m, (int)h->n, cur_U(h), h->Vbuf[h->vcur], h->k,
                                                                 h->scal_part);
         else
@@ -1911,6 +2061,7 @@ int prmf_comm_unique_id(uint8_t* id_out) {
 
 int prmf_comm_init(prmf_handle* h, int rank, int nranks, const uint8_t* id) {
     if (!h || !id) return PRMF_ERR_ARG;
+    if (h->x32 && !h->x_tc) return fail(h, PRMF_ERR_STATE, "PRMF_X_F32 handles are single-rank: no communicator");
     if (!g_nccl.loaded()) return fail(h, PRMF_ERR_NCCL, "call prmf_nccl_load first");
     if (nranks < 1 || rank < 0 || rank >= nranks) return fail(h, PRMF_ERR_ARG, "bad rank %d / %d", rank, nranks);
     CU(cudaSetDevice(h->device));
@@ -1951,6 +2102,7 @@ int prmf_p2p_export(prmf_handle* h, uint8_t* handle_out) {
 
 int prmf_p2p_attach(prmf_handle* h, int rank, int nranks, const uint8_t* handles) {
     if (!h || !handles) return PRMF_ERR_ARG;
+    if (h->x32 && !h->x_tc) return fail(h, PRMF_ERR_STATE, "PRMF_X_F32 handles are single-rank: no peer exchange");
     if (!h->p2p_buf) return fail(h, PRMF_ERR_STATE, "call prmf_p2p_export first");
     if (nranks < 2 || nranks > kMaxPeers || rank < 0 || rank >= nranks)
         return fail(h, PRMF_ERR_ARG, "prmf_p2p_attach: bad rank %d / %d (max %d ranks)", rank, nranks, kMaxPeers);
@@ -2061,7 +2213,7 @@ int prmf_project_t(prmf_handle* h, double* B_out) {
 int prmf_nnls_x(prmf_handle* h, int transpose, const double* B_host, int maxiter, double* x_out, double* rnorm_out,
                 int32_t* status_out, int32_t* iter_out) {
     if (!h || !B_host || !x_out || !rnorm_out || !status_out) return PRMF_ERR_ARG;
-    if (h->x_tf32) return fail(h, PRMF_ERR_STATE, "prmf_nnls_x needs an fp64 handle (X is stored as tf32)");
+    if (h->x_tc) return fail(h, PRMF_ERR_STATE, "prmf_nnls_x needs an fp64 or f32 handle (X is stored as tf32)");
     if (h->m != h->m_global) return fail(h, PRMF_ERR_STATE, "prmf_nnls_x needs a single-rank handle (m_local != m_global)");
     if (!h->have_X) return fail(h, PRMF_ERR_STATE, "prmf_nnls_x needs X");
     if (h->failed) return fail(h, PRMF_ERR_STATE, "the handle is in a failed state");
@@ -2069,84 +2221,11 @@ int prmf_nnls_x(prmf_handle* h, int transpose, const double* B_host, int maxiter
     CU(cudaSetDevice(h->device));
     cancel_ahead(h);
     h->have_U = h->have_V = false;                     // U and V serve as the residual operand from here on
-
-    NnlsWork wk;
-    wk.k = h->k;
-    wk.neq = transpose ? h->n : h->m;
-    wk.nun = transpose ? h->m : h->n;
-    wk.Arows = transpose ? h->X : h->Xt;
-    wk.lda = transpose ? h->ldx : h->ldxt;
-    wk.cap = (int)std::min<int64_t>({wk.neq, wk.nun, (int64_t)kNnlsMaxPassive});
-    wk.maxiter = maxiter > 0 ? maxiter : (int)std::min<int64_t>(3 * wk.nun, INT32_MAX - 1);   // scipy: 3 * #unknowns
-    wk.tol = 10.0 * (double)std::max(wk.neq, wk.nun) * DBL_EPSILON;                          // 10 max(m, n) eps
-    const int k = wk.k;
-    const size_t cap = (size_t)wk.cap, kk = (size_t)k;
-    auto pad = [](size_t bytes) { return (bytes + 255) & ~(size_t)255; };
-    const size_t d = sizeof(double);
-    const size_t b_bt = pad(d * kk * wk.neq), b_w = pad(d * kk * wk.nun), b_g = pad(d * kk * cap * cap);
-    const size_t b_vec = pad(d * kk * cap), b_idx = pad(sizeof(int) * kk * cap), b_flag = pad(kk * wk.nun);
-    const size_t b_small = pad(sizeof(int) * kk), b_rn = pad(d * kk);
-    const size_t total = b_bt + b_w + 2 * b_g + 2 * b_vec + b_idx + b_flag + 3 * b_small + b_rn;
-    unsigned char* ws = nullptr;
-    cudaError_t ea = g_pool.alloc((void**)&ws, total, h->device);
-    if (ea != cudaSuccess) return fail(h, PRMF_ERR_NOMEM, "cudaMalloc of %zu bytes failed: %s", total, cudaGetErrorString(ea));
-    size_t off = 0;
-    auto take = [&](size_t bytes) { unsigned char* p = ws + off; off += bytes; return p; };
-    wk.Bt = (const double*)take(b_bt);
-    wk.w = (double*)take(b_w);
-    wk.G = (double*)take(b_g);
-    wk.L = (double*)take(b_g);
-    wk.atb = (double*)take(b_vec);
-    unsigned char* zero_from = ws + off;               // everything from here on starts at zero
-    wk.xP = (double*)take(b_vec);
-    wk.pidx = (int*)take(b_idx);
-    wk.flag = (int8_t*)take(b_flag);
-    wk.np = (int*)take(b_small);
-    wk.iter = (int*)take(b_small);
-    wk.status = (int*)take(b_small);
-    double* rnorm_dev = (double*)take(b_rn);
-
-    std::vector<double> Bt((size_t)k * wk.neq);
-    for (int64_t e = 0; e < wk.neq; ++e)
-        for (int c = 0; c < k; ++c) Bt[(size_t)c * wk.neq + e] = B_host[e * k + c];
-    std::vector<int32_t> status(k, kNnlsRunning), np_h(k), pidx_h(kk * cap);
-    std::vector<double> xP_h(kk * cap);
-    int rc = PRMF_OK;
-    cudaError_t e = cudaMemcpyAsync((void*)wk.Bt, Bt.data(), sizeof(double) * Bt.size(), cudaMemcpyHostToDevice, h->stream);
-    if (e == cudaSuccess) e = cudaMemsetAsync(zero_from, 0, (size_t)(ws + total - zero_from), h->stream);
-    if (e != cudaSuccess) rc = fail(h, PRMF_ERR_CUDA, "prmf_nnls_x upload: %s", cudaGetErrorString(e));
-    if (!rc) rc = nnls_loop(h, transpose, wk, rnorm_dev, status);
-    if (!rc) {
-        e = cudaMemcpyAsync(np_h.data(), wk.np, sizeof(int32_t) * k, cudaMemcpyDeviceToHost, h->stream);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(pidx_h.data(), wk.pidx, sizeof(int32_t) * kk * cap, cudaMemcpyDeviceToHost, h->stream);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(xP_h.data(), wk.xP, sizeof(double) * kk * cap, cudaMemcpyDeviceToHost, h->stream);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(status_out, wk.status, sizeof(int32_t) * k, cudaMemcpyDeviceToHost, h->stream);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(rnorm_out, rnorm_dev, sizeof(double) * k, cudaMemcpyDeviceToHost, h->stream);
-        if (e == cudaSuccess && iter_out)
-            e = cudaMemcpyAsync(iter_out, wk.iter, sizeof(int32_t) * k, cudaMemcpyDeviceToHost, h->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-        if (e != cudaSuccess) rc = fail(h, PRMF_ERR_CUDA, "prmf_nnls_x read-back: %s", cudaGetErrorString(e));
-    } else {
-        cudaStreamSynchronize(h->stream);
-    }
-    g_pool.release(ws, total, h->device);
-    if (rc) return rc;
-    std::fill(x_out, x_out + wk.nun * k, 0.0);
-    for (int c = 0; c < k; ++c)
-        for (int q = 0; q < np_h[c]; ++q) x_out[(int64_t)pidx_h[c * cap + q] * k + c] = xP_h[c * cap + q];
-    h->err.clear();
-    for (int c = 0; c < k; ++c) {
-        if (status_out[c] == kNnlsCapacity) {
-            fail(h, PRMF_OK, "prmf_nnls_x: problem %d needs more than %d passive columns (the workspace capacity)", c,
-                 wk.cap);
-            break;
-        }
-        if (status_out[c] == kNnlsSingular) {
-            fail(h, PRMF_OK, "prmf_nnls_x: problem %d: the Gram matrix of its passive columns lost positive definiteness", c);
-            break;
-        }
-    }
-    return PRMF_OK;
+    if (h->x32)
+        return nnls_x_run<float>(h, transpose, transpose ? h->X32 : h->Xt32, transpose ? h->ldx32 : h->ldxt32, B_host,
+                                 maxiter, x_out, rnorm_out, status_out, iter_out);
+    return nnls_x_run<double>(h, transpose, transpose ? h->X : h->Xt, transpose ? h->ldx : h->ldxt, B_host, maxiter,
+                              x_out, rnorm_out, status_out, iter_out);
 }
 
 int prmf_release_pool(void) {

@@ -210,15 +210,17 @@ tc_rowdot_kernel(const __grid_constant__ CUtensorMap tmM, const __grid_constant_
 }
 
 // ---- storage conversions --------------------------------------------------------------------------------
-// dst[r][c] = tf32(src[r][c]) for c < n, 0 for n <= c < ld_dst (T = double or float source)
-template <typename T>
+// dst[r][c] = tf32(src[r][c]) (TF32) or the nearest fp32 value, as astype(np.float32) rounds (PRMF_X_F32), for c < n;
+// 0 for n <= c < ld_dst (T = double or float source)
+template <typename T, bool TF32>
 __global__ void __launch_bounds__(256)
 to_tf32_rows_kernel(const T* __restrict__ src, int64_t ld_src, int64_t rows, int64_t n, float* __restrict__ dst,
                     int64_t ld_dst) {
     const int64_t total = rows * ld_dst;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
         const int64_t r = i / ld_dst, c = i - r * ld_dst;
-        dst[i] = c < n ? to_tf32((float)src[r * ld_src + c]) : 0.0f;
+        if (TF32) dst[i] = c < n ? to_tf32((float)src[r * ld_src + c]) : 0.0f;
+        else dst[i] = c < n ? (float)src[r * ld_src + c] : 0.0f;
     }
 }
 

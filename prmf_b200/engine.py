@@ -26,8 +26,10 @@ class CudaEngine:
     """Owns the device-resident X row block, U, V, pathway tables and scratch of one rank."""
 
     def __init__(self, m_local, m_global, n, k, device=0, stream=None, x_dtype="f64"):
-        """x_dtype: "f64" (parity mode, X streamed in fp64) or "tf32" (opt-in: X stored as fp32 rounded to
-        tf32, X.V and X^T.U on the tcgen05 tensor cores; everything else stays fp64)."""
+        """x_dtype: "f64" (parity mode, X streamed in fp64), "f32" (opt-in, single rank: X stored as exact fp32
+        values and streamed through the fp64 kernels, bitwise what "f64" returns on X.astype(np.float64)) or "tf32"
+        (opt-in: X stored as fp32 rounded to tf32, X.V and X^T.U on the tcgen05 tensor cores; everything else stays
+        fp64)."""
         self.lib = _lib.load()
         self.m, self.m_global, self.n, self.k = int(m_local), int(m_global), int(n), int(k)
         self.P = 0
@@ -67,13 +69,15 @@ class CudaEngine:
 
     # -- data ----------------------------------------------------------------------------------------
     def set_X(self, X):
-        """X: this rank's row block; a C-contiguous float64 numpy array (host) or a CUDA torch tensor."""
+        """X: this rank's row block; a float64 numpy array (host) or a CUDA torch tensor.  "f32" and "tf32" engines
+        also take float32 input, and round float64 input to fp32 (to tf32 in the tf32 mode) on the device."""
+        x32 = self.x_dtype in ("tf32", "f32")
         if hasattr(X, "is_cuda") and X.is_cuda:
             import torch
-            f32_ok = self.x_dtype == "tf32" and X.dtype == torch.float32
+            f32_ok = x32 and X.dtype == torch.float32
             if (X.dtype != torch.float64 and not f32_ok) or X.dim() != 2 or X.stride(1) != 1:
                 raise ValueError("device X must be a 2-D float64 tensor with unit column stride"
-                                 " (float32 is accepted by a tf32 engine)")
+                                 " (float32 is accepted by f32 and tf32 engines)")
             if tuple(X.shape) != (self.m, self.n):
                 raise ValueError("X has shape %s, engine expects %s" % (tuple(X.shape), (self.m, self.n)))
             torch.cuda.current_stream(X.device).synchronize()
@@ -85,7 +89,7 @@ class CudaEngine:
         X = np.asarray(X)
         if X.shape != (self.m, self.n):
             raise ValueError("X has shape %s, engine expects %s" % (X.shape, (self.m, self.n)))
-        if self.x_dtype == "tf32" and X.dtype == np.float32 and X.strides[1] == 4 and X.strides[0] % 4 == 0:
+        if x32 and X.dtype == np.float32 and X.strides[1] == 4 and X.strides[0] % 4 == 0:
             self._ck(self.lib.prmf_set_X_f32(self.h, _ptr(X), X.strides[0] // 4 if self.m > 0 else self.n, 0))
             return
         if X.dtype != np.float64 or X.strides[1] != 8 or X.strides[0] % 8 != 0:

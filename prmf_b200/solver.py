@@ -340,11 +340,14 @@ def nmf_pathway(X, Gs, gamma=1.0, delta=1.0, tradeoff=None, k_latent=6, tol=1e-3
     the reference's.  Keyword-only extras: `ctx` (a `DistContext`; default: the initialised
     torch.distributed group, else single process), `X_is_local`/`m_global` (X is already this rank's row
     block), `trace` (dict collecting per-iteration diagnostics), `quiet` (suppress the per-step prints),
-    `x_dtype` ("f64": parity mode; "tf32": opt-in tensor-core X streams, see include/prmf_b200.h).
+    `x_dtype` ("f64": parity mode; "f32": X held as exact fp32 values, one rank only, bitwise the "f64" run on
+    X.astype(np.float64); "tf32": opt-in tensor-core X streams; see include/prmf_b200.h).
     With several ranks every rank must call this with the same seed and arguments; all return the same
     full U, V and obj_data.
     """
     ctx = ctx or DistContext.current()
+    if x_dtype == "f32" and ctx.world > 1:
+        raise ValueError('x_dtype="f32" runs on one rank only (this context has %d ranks)' % ctx.world)
     factory = engine_factory or default_engine_factory
     out = (lambda *a: None) if (quiet or ctx.rank != 0) else print
     if nodelist is None:
