@@ -168,7 +168,7 @@ int prmf_comm_init(prmf_handle* h, int rank, int nranks, const uint8_t* id);
  *     16-byte store each, no fence, no flag), polls the same entries of all ranks in its own memory, adds them in rank
  *     order and updates its rows of V.  No collective launch; bitwise identical on all ranks.
  *   - otherwise: the packed buffers of all ranks are pulled with P2P loads inside the V-update kernel (flag barrier in
- *     peer memory), or inside the pass-2 kernel with PRMF_XCHG=1.
+ *     peer memory).
  * Needs one process per rank on one node with peer access (or several ranks sharing one device: IPC works there too).
  * prmf_comm_init is OPTIONAL for the first variant: without a communicator the set-up reductions (||X||^2, the
  * agreement itself) are summed over the same peer buffers; configurations that need the other variants then fail with
@@ -179,8 +179,9 @@ int prmf_p2p_attach(prmf_handle* h, int rank, int nranks, const uint8_t* handles
 int prmf_p2p_finalize(prmf_handle* h);
 
 /* How the per-step sum over ranks is done: 0 one rank, 1 ncclAllReduce, 2 NVLink peer loads inside the V-update
- * kernel, 3 NVLink peer loads inside the pass-2 X-stream kernel, 4 NVLink peer stores (push) inside the persistent
- * step kernel (the default for k <= 10 when every rank can take it; agreed in prmf_p2p_finalize). */
+ * kernel, 4 NVLink peer stores (push) inside the persistent step kernel (the default for k <= 10 when every rank can
+ * take it; agreed in prmf_p2p_finalize).  3 (NVLink peer loads inside the pass-2 X-stream kernel) is retired and no
+ * longer returned. */
 int prmf_exchange_mode(const prmf_handle* h);
 
 /* ---- introspection used by bench.py and the tests ---------------------------------------------------*/

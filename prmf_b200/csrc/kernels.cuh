@@ -356,9 +356,6 @@ __device__ __forceinline__ unsigned long long ld_acquire_gpu_u64(const unsigned 
     asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
     return v;
 }
-__device__ __forceinline__ void st_release_sys_u64(unsigned long long* p, unsigned long long v) {
-    asm volatile("st.release.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
 __device__ __forceinline__ unsigned long long ld_acquire_sys_u64(const unsigned long long* p) {
     unsigned long long v;
     asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
@@ -449,11 +446,8 @@ __device__ __forceinline__ double sum_peers(const PeerExchange& px, int64_t idx)
 //          second U buffer, partials of U_new^T U_new
 //   EPI 2 (pass 2, panel = genes, one GPU): B = fixed-order sum of the chunk partials, V update (:425-444) into
 //          the second V buffer, partials of V_new^T V_new and sum(V_new * B) for the objective
-//   EPI 3 (pass 2, sharded, NCCL path): B sums and the Gu sum written to the packed buffer that is all-reduced
-//   EPI 4 (pass 2, sharded, NVLink peer path): every CTA publishes the B sums of its share in this rank's packed
-//          buffer, announces them with a flag in every peer's memory, waits for the same share of all peers, adds
-//          the ranks' buffers in rank order over P2P loads (bitwise identical on all ranks) and performs the V
-//          update of its share -- exchange and update overlap CTA by CTA, no separate launch, no collective call
+//   EPI 3 (pass 2, sharded): B sums and the Gu sum written to the packed buffer that the ranks sum, either with
+//          ncclAllReduce or with the P2P pull of the V-update kernel
 // The per-CTA Gram partials are folded per panel by the last CTA of the panel to finish (second counter), so
 // the next consumer adds only `panels` terms.  All CTAs of the grid must be co-resident (they wait for each
 // other): the grid never exceeds the SM count and the launch is cooperative.  Only the 8 consumer warps take
@@ -489,11 +483,6 @@ struct EpiParams {
     const int64_t* doff;          // per-factor offsets into that order (ActiveSet)
     // EPI 3
     double* red;                  // [n*k | k*k | 2]
-    // EPI 4 (sharded, NVLink peer exchange inside the kernel)
-    PeerExchange px;              // packed buffers of all ranks (this step's parity), rank, nranks, seq
-    unsigned long long* xflags[kMaxPeers];   // rank r's flag array [nranks][ctas + 1]: flags[q][c] = last step in which
-                                  // rank q published the segment of CTA c (c == ctas: its Gu)
-    double* Gu_glob;              // out: U^T U summed over ranks (k*k), for the objective kernel
     int dbg_slot;                 // developer timing builds only: timeline slot of this launch (-1: none)
     unsigned int* err;            // bounded waits: error word and deadline
     unsigned long long timeout_ns;
@@ -502,20 +491,17 @@ struct EpiParams {
 __device__ __forceinline__ void cons_bar() { asm volatile("bar.sync 1, 256;" ::: "memory"); }
 
 #ifdef PRMF_EPI_TIMING
-// Developer instrumentation (not part of the product build): per-CTA time stamps of the pass-2 fused tail.
-__device__ unsigned long long g_epi_dbg[160 * 8];
+// Developer instrumentation (not part of the product build): per-launch timeline of the X-stream kernels.
 __device__ __forceinline__ unsigned long long epi_gtime() {
     unsigned long long t;
     asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
     return t;
 }
-#define EPI_STAMP(i) do { if (threadIdx.x == 0) g_epi_dbg[(blockIdx.x * gridDim.y + blockIdx.y) * 8 + (i)] = epi_gtime(); } while (0)
 // per-launch timeline: [slot][0] first CTA start, [1] last CTA past its main loop, [2] last CTA end
 __device__ unsigned long long g_kt_dbg[64 * 4];
 #define KT_STAMP_MIN(slot, i) do { if (threadIdx.x == 0 && (slot) >= 0 && (slot) < 64) atomicMin(&g_kt_dbg[(slot) * 4 + (i)], epi_gtime()); } while (0)
 #define KT_STAMP_MAX(slot, i) do { if (threadIdx.x == 0 && (slot) >= 0 && (slot) < 64) atomicMax(&g_kt_dbg[(slot) * 4 + (i)], epi_gtime()); } while (0)
 #else
-#define EPI_STAMP(i) do { } while (0)
 #define KT_STAMP_MIN(slot, i) do { } while (0)
 #define KT_STAMP_MAX(slot, i) do { } while (0)
 #endif
@@ -753,114 +739,6 @@ __device__ __forceinline__ void epi_pack(const EpiParams& ep, int panel, int64_t
 }
 
 
-template <int K>
-__device__ __forceinline__ void epi_exchange_v_update(const EpiParams& ep, unsigned char* smem, int* s_flag, int panel,
-                                                      int64_t c0, int width, int64_t cols,
-                                                      const double* __restrict__ Bpart) {
-    const int t = threadIdx.x;
-    const int chunks = (int)gridDim.y;
-    int rb, rows;
-    epi_share(width, cols, c0, rb, rows);
-    const int n_el = rows * K;
-    double* sG = reinterpret_cast<double*>(smem);            // K*K (Gu summed over ranks)
-    double* sBuf = sG + 128;
-    double* sT = sBuf + 8 * K * K;                           // rows x K new rows
-    double* sB = sT + n_el;                                  // rows x K  X^T U (local, then summed over ranks)
-    double* sV = sB + n_el;                                  // rows x K old rows
-    double* sW = sG + 112;
-    const int64_t base = (c0 + rb) * K;
-    const PeerExchange& px = ep.px;
-    const int cta = panel * chunks + (int)blockIdx.y;
-    const int ncta = (int)(gridDim.x * gridDim.y);
-    const int fstride = ncta + 1;
-    const int64_t nk = cols * K;
-    double* mine = const_cast<double*>(px.red[px.rank]);
-    // this rank's Gu is complete since pass 1: CTA 0 publishes it straight away
-    if (cta == 0 && t < K * K) mine[nk + t] = sum_strided(ep.Gu_part_in + t, ep.gu_parts, K * K);
-    for (int e = t; e < n_el; e += 256) sV[e] = ep.Vold[base + e];
-    const double gamma = ep.gd[0], delta = ep.gd[1];
-    EPI_STAMP(0);
-    epi_panel_barrier(ep, panel);
-    EPI_STAMP(1);
-    epi_stage_sums(sB, Bpart + base, n_el, chunks, cols * K);                               // local X^T U  (:424)
-    cons_bar();
-    for (int e = t; e < n_el; e += 256) mine[base + e] = sB[e];
-    __threadfence_system();
-    cons_bar();
-    EPI_STAMP(2);
-    // announce the segment (and, from CTA 0, Gu) to every rank, then wait for the same from every rank
-    if (t < px.nranks) st_release_sys_u64(ep.xflags[t] + (size_t)px.rank * fstride + cta, px.seq);
-    if (cta == 0 && t >= 32 && t < 32 + px.nranks)
-        st_release_sys_u64(ep.xflags[t - 32] + (size_t)px.rank * fstride + ncta, px.seq);
-    if (t < px.nranks) {
-        blk_wait_ge<true>(ep.xflags[px.rank] + (size_t)t * fstride + cta, px.seq, ep.err, ep.timeout_ns);
-    } else if (t >= 32 && t < 32 + px.nranks) {
-        blk_wait_ge<true>(ep.xflags[px.rank] + (size_t)(t - 32) * fstride + ncta, px.seq, ep.err, ep.timeout_ns);
-    }
-    cons_bar();
-    EPI_STAMP(3);
-    if (t < K * K) {
-        const double g = sum_peers(px, nk + t);
-        sG[t] = g;
-        if (cta == 0) {
-            ep.Gu_glob[t] = g;
-            if (ep.hist_Gu != nullptr) ep.hist_Gu[t] = g;
-        }
-    }
-    for (int e = t; e < n_el; e += 256) sB[e] = sum_peers(px, base + e);                    // sum over ranks, rank order
-    cons_bar();
-    EPI_STAMP(4);
-    double vb = 0.0;
-    for (int e = t; e < n_el; e += 256) {
-        const int r = e / K, c = e - r * K;
-        const int64_t j = c0 + rb + r;
-        const double* vrow = sV + r * K;
-        const double b = sB[e];
-        double cden = 0.0;
-#pragma unroll
-        for (int l = 0; l < K; ++l) cden = fma(vrow[l], sG[l * K + c], cden);               // V.Gu   (:425)
-        const double v = vrow[c];
-        double num = b, den = cden;
-        const int32_t pr = ep.pos[j * K + c];
-        if (pr >= 0) {
-            const Pathways& pw = ep.pw;
-            const int64_t pbase = pw.path_ptr[ep.active[c]];
-            double wv = 0.0;
-            for (int64_t e2 = pw.row_ptr[pr]; e2 < pw.row_ptr[pr + 1]; ++e2)
-                wv = fma(pw.w[e2], ep.Vold[(int64_t)pw.support_idx[pbase + pw.col_local[e2]] * K + c], wv);
-            const double vp1 = v + 1.0;
-            const double man = gamma * wv;                                                  // :434
-            const double ign = delta * (1.0 / (vp1 * vp1));                                 // :438
-            num = b + (man + ign);                                                          // :440
-            den = cden + gamma * (pw.deg[pr] * v);                                          // :435,:441
-        }
-        if (den < kEps) den = kEps;                                                         // :442
-        double vn = v * (num / den);                                                        // :443
-        if (vn < kEps) vn = kEps;                                                           // :444
-        sT[e] = vn;
-        ep.Vnew[j * K + c] = vn;
-        if (pr >= 0 && ep.hist_vh != nullptr) ep.hist_vh[ep.doff[c] + (pr - ep.pw.path_ptr[ep.active[c]])] = vn;
-        vb = fma(vn, b, vb);
-    }
-    vb = warp_sum(vb);
-    if ((t & 31) == 0) sW[t >> 5] = vb;
-    cons_bar();
-    const int64_t me = (int64_t)panel * chunks + blockIdx.y;
-    if (t == 0) {
-        double s = 0.0;
-#pragma unroll
-        for (int w = 0; w < 8; ++w) s += sW[w];
-        ep.vb2[me] = s;
-    }
-    epi_gram<K>(sT, rows, sBuf, ep.part2 + me * K * K);
-    EPI_STAMP(5);
-    if (epi_panel_done(ep, panel, s_flag)) {
-        if (t < K * K) ep.Gv_part[(int64_t)panel * K * K + t] = sum_strided_cg(ep.part2 + (int64_t)panel * chunks * K * K + t, chunks, K * K);
-        if (t == 128) ep.VB_part[panel] = sum_strided_cg(ep.vb2 + (int64_t)panel * chunks, chunks, 1);
-    }
-}
-
-
 // ----------------------------------------------------------------------------------------------------
 // X-stream kernels (k <= 10).  The body is shared by the fp64 storage mode (T = double) and the fp32 storage mode
 // (T = float, skinny_tma_f32_kernel): an fp32 element is widened to fp64 exactly before its DFMA, so every column runs
@@ -998,7 +876,6 @@ skinny_tma_body(const T* __restrict__ M, int64_t ldm, int64_t rows_total, int64_
         if constexpr (EPI == 1) epi_u_update<KT>(ep, smem_raw, &s_last, panel, c0, width, cols, OutPart);
         if constexpr (EPI == 2) epi_v_update<KT>(ep, smem_raw, &s_last, panel, c0, width, cols, OutPart);
         if constexpr (EPI == 3) epi_pack<KT>(ep, panel, c0, width, cols, OutPart);
-        if constexpr (EPI == 4) epi_exchange_v_update<KT>(ep, smem_raw, &s_last, panel, c0, width, cols, OutPart);
     }
     KT_STAMP_MAX(ep.dbg_slot, 2);
 }

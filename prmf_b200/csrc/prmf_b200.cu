@@ -7,8 +7,8 @@
 //   skinny_tma_kernel<k,8,1>   A partials = Xt^T.V, then U <- U*A/(U.Gv+U) and Gu in the last CTA of each panel   (:420-422)
 //   skinny_tma_kernel<k,8,2>   B partials = X^T.U_new, then V_new, Gv/VB partials                                 (:424-444)
 //   objective_(parts|deferred)_kernel   recon/manifold/ignore/fro/obj, per step or once per block                 (:336-372)
-//   sharded: the pass-2 tail packs for ncclAllReduce (EPI 3) or exchanges over NVLink (EPI 4); or the whole block
-//   of steps runs as one persistent launch (block_kernel<K>, block.cuh)
+//   sharded: the pass-2 tail packs (EPI 3) for ncclAllReduce or for the V-update kernel's NVLink pull; or the whole
+//   block of steps runs as one persistent launch (block_kernel<K>, block.cuh)
 //
 // otherwise (k > 10, tf32 mode, PRMF_EPI=0, ranks without rows):
 //   X-stream pass 1 (launch_xv)   A partials = Xt^T.V                                      (:420)
@@ -235,16 +235,14 @@ struct prmf_handle {
     // multi-GPU
     NcclComm comm = nullptr;
     int rank = 0, nranks = 1;
-    // NVLink peer exchange (fused all-reduce): [red parity 0 | red parity 1 | flags]
+    // NVLink peer exchange: [red parity 0 | red parity 1 | flags | ...] (layout: prmf_p2p_export)
     double* p2p_buf = nullptr;
     size_t p2p_red_count = 0;
     bool p2p_ready = false;
     void* peer_base[kMaxPeers] = {nullptr};
     unsigned long long p2p_seq = 0;
     int p2p_parity = 0;
-    // exchange + V update inside the pass-2 kernel (fused-tail path on every rank; agreed in prmf_p2p_finalize)
-    bool use_xchg = false;
-    double* Gu_glob = nullptr;
+    double* Gu_glob = nullptr;                // large k: U^T U summed over the U-update CTAs (and over ranks when sharded)
 
     // Speculative pass 1: the first X.V pass (+ U update on the fused-tail path) of the NEXT inner step does not
     // depend on the active pathways, so prmf_block_end enqueues it before the host waits for the score tables;
@@ -354,7 +352,6 @@ int launch_skinny_epi_t(prmf_handle* h, int epi, const T* M, int64_t ldm, int64_
         case 1: fn = (const void*)tma_kernel<KT, 1>(M); break;
         case 2: fn = (const void*)tma_kernel<KT, 2>(M); break;
         case 3: if constexpr (sizeof(T) == sizeof(double)) fn = (const void*)skinny_tma_kernel<KT, kTmaRS, 3>; break;
-        case 4: if constexpr (sizeof(T) == sizeof(double)) fn = (const void*)skinny_tma_kernel<KT, kTmaRS, 4>; break;
     }
     if (!fn) return fail(h, PRMF_ERR_STATE, "bad fused-tail id %d", epi);
     CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -709,7 +706,7 @@ int launch_xv_epi(prmf_handle* h, const double* gv_src = nullptr, int gv_parts =
     return PRMF_OK;
 }
 
-// mode 2: V update (one GPU); 3: pack into `packed_dst` (NCCL path); 4: NVLink peer exchange + V update
+// mode 2: V update (one GPU); 3: pack into `packed_dst` for the sum over ranks (sharded)
 int launch_xtu_epi(prmf_handle* h, int mode, double* packed_dst, int hist_slot = -1) {
     EpiParams ep{};
     ep.err = h->err_word; ep.timeout_ns = h->spin_timeout_ns;
@@ -742,20 +739,6 @@ int launch_xtu_epi(prmf_handle* h, int mode, double* packed_dst, int hist_slot =
             ep.doff = h->as_off;
         }
     }
-    if (mode == 4) {
-        PeerExchange& px = ep.px;
-        px.nranks = h->nranks;
-        px.rank = h->rank;
-        px.seq = ++h->p2p_seq;
-        for (int r = 0; r < h->nranks; ++r) {
-            double* base = (double*)h->peer_base[r];
-            px.red[r] = base + (size_t)h->p2p_parity * h->p2p_red_count;
-            px.flags[r] = nullptr;
-            ep.xflags[r] = (unsigned long long*)(base + 2 * h->p2p_red_count + 64);
-        }
-        h->p2p_parity ^= 1;
-        ep.Gu_glob = h->Gu_glob;
-    }
     int rc = 0;
     if (h->x32) {
         KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, mode, h->X32, h->ldx32, h->m, h->n, h->U, h->panels, h->panel_w,
@@ -765,8 +748,7 @@ int launch_xtu_epi(prmf_handle* h, int mode, double* packed_dst, int hist_slot =
                      h->chunks, h->rows_per_chunk, h->tma_smem2, h->Bpart, ep);
     }
     if (rc) { h->failed = true; return rc; }
-    LAUNCH_CHECK(mode == 3 ? "skinny_tma_kernel(pass 2 + pack)" : mode == 4 ? "skinny_tma_kernel(pass 2 + exchange + V update)"
-                                                                            : "skinny_tma_kernel(pass 2 + V update)");
+    LAUNCH_CHECK(mode == 3 ? "skinny_tma_kernel(pass 2 + pack)" : "skinny_tma_kernel(pass 2 + V update)");
     if (mode != 3) h->vcur ^= 1;
     return PRMF_OK;
 }
@@ -978,8 +960,8 @@ int enqueue_steps(prmf_handle* h, int n_steps, double gamma, double delta, doubl
         if (!h->profiling) return;
         cudaEventRecord(h->ev_pool[h->ev_pairs.back().second + 1], h->stream);
     };
-    // deferred objective: one GPU, or sharded with the in-kernel exchange (every rank evaluates the same numbers)
-    const bool defer = h->defer_ok && h->use_epi && (!sharded(h) || h->use_xchg || h->blk_xchg) && tradeoff < 0.0 &&
+    // deferred objective: one GPU, or sharded with the persistent step kernel (every rank evaluates the same numbers)
+    const bool defer = h->defer_ok && h->use_epi && (!sharded(h) || h->blk_xchg) && tradeoff < 0.0 &&
                        !h->profiling && h->as.n_diag <= kVhCap;
     if (defer && block_path(h)) {
         // the whole block in ONE persistent launch (block.cuh) + the deferred objective
@@ -1005,7 +987,7 @@ int enqueue_steps(prmf_handle* h, int n_steps, double gamma, double delta, doubl
                 rc = s == 0 ? launch_xv_epi(h) : launch_xv_epi(h, h->hist_Gvp + (size_t)(s - 1) * h->panels * kk2s, h->panels);
                 if (rc) return rc;
             }
-            if ((rc = launch_xtu_epi(h, !sharded(h) ? 2 : 4, nullptr, s))) return rc;
+            if ((rc = launch_xtu_epi(h, 2, nullptr, s))) return rc;
             if (s == n_steps - 1) {
                 objective_deferred_kernel<<<n_steps, kTailThreads, obj_smem(h), h->stream>>>(
                     h->k, h->hist_Gu, h->hist_Gvp, h->hist_VBp, h->panels, h->hist_vh, kVhCap, h->normX_sq, h->as, h->Gv,
@@ -1021,11 +1003,6 @@ int enqueue_steps(prmf_handle* h, int n_steps, double gamma, double delta, doubl
                 tic(2); rc = launch_xtu_epi(h, 2, nullptr); toc();               // + V update
                 if (rc) return rc;
                 tic(5); rc = launch_objective(h, tradeoff, h->Gu_part, h->panels1); toc();
-                if (rc) return rc;
-            } else if (h->use_xchg) {
-                tic(2); rc = launch_xtu_epi(h, 4, nullptr); toc();               // + exchange + V update
-                if (rc) return rc;
-                tic(5); rc = launch_objective(h, tradeoff, h->Gu_glob, 1); toc();
                 if (rc) return rc;
             } else {
                 double* dst = h->p2p_ready ? h->p2p_buf + (size_t)h->p2p_parity * h->p2p_red_count : h->red;
@@ -2081,17 +2058,20 @@ int prmf_p2p_export(prmf_handle* h, uint8_t* handle_out) {
     static_assert(sizeof(cudaIpcMemHandle_t) == PRMF_IPC_HANDLE_BYTES, "IPC handle size");
     CU(cudaSetDevice(h->device));
     if (!h->p2p_buf) {
+        // [red parity 0 | red parity 1 | 64 peer-barrier flag words | push receive slots | small all-reduce slots], in
+        // doubles; it depends on n and k only, so every rank computes the same offsets into every rank's buffer
         h->p2p_red_count = (size_t)round_up(h->n * h->k + (int64_t)h->k * h->k + 2, 32);
-        const size_t old_total = 2 * h->p2p_red_count + 64 + (size_t)kMaxPeers * (h->sm_count + 2);   // + per-CTA flags
+        const size_t flags_end = 2 * h->p2p_red_count + 64;
+        const size_t xbuf_at = (flags_end + 1) & ~(size_t)1;                   // 16-byte aligned
         // push exchange of the persistent step kernel: receive slots [parity][source rank][n*k + k*k] + its flags
         h->xcount = h->p2p_red_count;
         const size_t xdoubles = 2 * 2 * (size_t)kMaxPeers * h->xcount;        // 16-byte {value, sequence} entries
         const size_t sdoubles = 2 * 2 * (size_t)kMaxPeers * kSmallAllreduceMax;   // set-up scalars without NCCL
-        const size_t total = ((old_total + 1) & ~(size_t)1) + xdoubles + sdoubles;
+        const size_t total = xbuf_at + xdoubles + sdoubles;
         int rc = dalloc(h, &h->p2p_buf, total);
         if (rc) return rc;
         CU(cudaMemset(h->p2p_buf, 0, total * sizeof(double)));
-        h->xbuf = h->p2p_buf + ((old_total + 1) & ~(size_t)1);                // 16-byte aligned
+        h->xbuf = h->p2p_buf + xbuf_at;
         h->xsmall = h->xbuf + xdoubles;
     }
     cudaIpcMemHandle_t hd;
@@ -2129,31 +2109,28 @@ int prmf_p2p_finalize(prmf_handle* h) {
     if (!h) return PRMF_ERR_ARG;
     if (!h->p2p_ready) return fail(h, PRMF_ERR_STATE, "prmf_p2p_finalize needs prmf_p2p_attach (and prmf_comm_init unless NCCL is not used)");
     CU(cudaSetDevice(h->device));
-    // the in-kernel exchange is used only if EVERY rank runs the fused-tail path (ranks that disagreed would wait
-    // on flags nobody writes)
-    // opt-in (PRMF_XCHG=1): measured at 2 GPUs it does not beat the exchange inside the V-update kernel yet
-    const char* ex = getenv("PRMF_XCHG");
-    // [in-kernel pull exchange wanted | persistent step kernel possible | pass-2 chunks | chunks^2]: the push exchange of
-    // the persistent kernel pairs CTA c of every rank, so all ranks must split the genes the same way
-    const double mine[4] = {(h->use_epi && ex && atoi(ex) == 1) ? 1.0 : 0.0, h->use_block ? 1.0 : 0.0, (double)h->chunks,
-                            (double)h->chunks * h->chunks};
+    // The persistent step kernel is used only if EVERY rank can take it (ranks that disagreed would wait on flags
+    // nobody writes), and its push exchange pairs CTA c of every rank, so all ranks must split the genes the same
+    // way: [persistent step kernel possible | pass-2 chunks | chunks^2], summed over ranks
+    const double mine[3] = {h->use_block ? 1.0 : 0.0, (double)h->chunks, (double)h->chunks * h->chunks};
     CU(cudaMemcpyAsync(h->scal_part, mine, sizeof mine, cudaMemcpyHostToDevice, h->stream));
-    int rc = allreduce(h, h->scal_part, 4);
+    int rc = allreduce(h, h->scal_part, 3);
     if (rc) return rc;
-    double sum[4] = {0, 0, 0, 0};
+    double sum[3] = {0, 0, 0};
     CU(cudaMemcpyAsync(sum, h->scal_part, sizeof sum, cudaMemcpyDeviceToHost, h->stream));
     CU(cudaStreamSynchronize(h->stream));
-    h->use_xchg = sum[0] > h->nranks - 0.5;
-    const bool same_chunks = std::fabs(h->nranks * sum[3] - sum[2] * sum[2]) < 0.5;
-    h->blk_xchg = !h->use_xchg && sum[1] > h->nranks - 0.5 && same_chunks;
+    const bool same_chunks = std::fabs(h->nranks * sum[2] - sum[1] * sum[1]) < 0.5;
+    h->blk_xchg = sum[0] > h->nranks - 0.5 && same_chunks;
     return PRMF_OK;
 }
 
+// 0 one GPU, 1 NCCL, 2 P2P pull in the V-update kernel, 4 push inside the persistent step kernel (3, the pull inside
+// the pass-2 kernel, was removed; the numbers are part of the ABI)
 int prmf_exchange_mode(const prmf_handle* h) {
     if (!h || !sharded(h)) return 0;
     if (!h->p2p_ready) return 1;
     if (h->blk_xchg && h->use_block) return 4;
-    return h->use_xchg ? 3 : 2;
+    return 2;
 }
 
 int64_t prmf_launch_count(const prmf_handle* h) { return h ? h->launches : 0; }
@@ -2254,15 +2231,6 @@ int prmf_debug_timeline(unsigned long long* out256, int reset) {
     return cudaMemcpyFromSymbol(out256, g_kt_dbg, sizeof(unsigned long long) * 256) == cudaSuccess ? 0 : -1;
 #else
     (void)out256; (void)reset;
-    return -1;
-#endif
-}
-
-int prmf_debug_epi_stamps(unsigned long long* out, int count) {
-#ifdef PRMF_EPI_TIMING
-    return cudaMemcpyFromSymbol(out, g_epi_dbg, sizeof(unsigned long long) * count) == cudaSuccess ? 0 : -1;
-#else
-    (void)out; (void)count;
     return -1;
 #endif
 }

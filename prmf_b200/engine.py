@@ -247,7 +247,8 @@ class CudaEngine:
 
     @property
     def exchange_mode(self):
-        """"none" | "nccl" | "p2p-v-update" | "p2p-pass2" | "p2p-push-block": how the per-step sum over ranks is done."""
+        """"none" | "nccl" | "p2p-v-update" | "p2p-push-block": how the per-step sum over ranks is done.  Index 3,
+        "p2p-pass2" (the pull inside the pass-2 kernel), is retired and no longer returned; the indices are the ABI's."""
         return ("none", "nccl", "p2p-v-update", "p2p-pass2", "p2p-push-block")[int(self.lib.prmf_exchange_mode(self.h))]
 
     # -- introspection -------------------------------------------------------------------------------

@@ -105,11 +105,10 @@ def test_two_ranks_on_one_gpu(case, tmp_path):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("k,env", [
-    (6, {"PRMF_XCHG": "1"}),      # exchange + V update inside the pass-2 kernel (opt-in)
     (6, {"PRMF_P2P": "0"}),       # ncclAllReduce of the packed buffer
     (24, {}),                     # large k: tiled U / V updates, NVLink peer loads inside the tiled V update
     (24, {"PRMF_P2P": "0"}),
-])
+], ids=["6-env1", "24-env2", "24-env3"])   # fixed ids: a case keeps its id when other cases are added or removed
 def test_two_gpus_match_one_gpu(k, env, tmp_path):
     """Sharded runs (all exchange flavours) against the same solve on one GPU: identical sampled pathways and
     maps, objective parts rel 1e-9, U / V rel 1e-6; all ranks bitwise equal."""
