@@ -392,13 +392,7 @@ block_kernel(const BlockParams p) {
                     const int c = e % K;
                     double wv = 0.0, dg = -1.0;                                                  // dg < 0: not in the support
                     const int32_t pr = prs[q];
-                    if (pr >= 0) {
-                        const Pathways& pw = p.pw;
-                        const int64_t pbase = pw.path_ptr[p.active[c]];
-                        for (int64_t e2 = pw.row_ptr[pr]; e2 < pw.row_ptr[pr + 1]; ++e2)
-                            wv = fma(pw.w[e2], __ldcg(Vold + (int64_t)pw.support_idx[pbase + pw.col_local[e2]] * K + c), wv);
-                        dg = pw.deg[pr];
-                    }
+                    if (pr >= 0) { wv = pathway_term<true>(p.pw, p.active, pr, c, Vold, K); dg = p.pw.deg[pr]; }
                     pO[e] = vo[q];
                     pWv[e] = wv;
                     pDg[e] = dg;
@@ -553,13 +547,11 @@ block_kernel(const BlockParams p) {
                         if (e < n_el) {
                             const int r = e / K, c = e - r * K;
                             const double* urow = sR + r * K;
-                            double den = 0.0;
+                            double ugv = 0.0;
     #pragma unroll
-                            for (int l = 0; l < K; ++l) den = fma(urow[l], sGv[l * K + c], den);
+                            for (int l = 0; l < K; ++l) ugv = fma(urow[l], sGv[l * K + c], ugv);
                             const double u = urow[c];
-                            den += u;
-                            const double f = (den != 0.0) ? a[q] / den : 1.0;                        // 0/0 := 1 (:422)
-                            un[q] = u * f;
+                            un[q] = u_update_value(u, a[q], ugv);
                             Unew[base + e] = un[q];
                         }
                     }
@@ -587,13 +579,11 @@ block_kernel(const BlockParams p) {
                     for (int e = t; e < n_el; e += 256) {
                         const int r = e / K, c = e - r * K;
                         const double* urow = sO + r * K;
-                        double den = 0.0;
+                        double ugv = 0.0;
 #pragma unroll
-                        for (int l = 0; l < K; ++l) den = fma(urow[l], sGv[l * K + c], den);
+                        for (int l = 0; l < K; ++l) ugv = fma(urow[l], sGv[l * K + c], ugv);
                         const double u = urow[c];
-                        den += u;
-                        const double f = (den != 0.0) ? sS[e] / den : 1.0;                       // 0/0 := 1 (:422)
-                        const double un = u * f;
+                        const double un = u_update_value(u, sS[e], ugv);
                         sT[e] = un;
                         Unew[base + e] = un;
                     }
@@ -671,7 +661,6 @@ block_kernel(const BlockParams p) {
 #pragma unroll
                     for (int l = 0; l < K; ++l) cden = fma(vrow[l], sGu[l * K + c], cden);      // V.Gu   (:425)
                     const double v = vrow[c];
-                    double num = bb, den = cden;
                     int32_t pr = -1;
                     double wv = 0.0, dg = 0.0;
                     if (pre2) {
@@ -680,6 +669,7 @@ block_kernel(const BlockParams p) {
                     } else {
                         pr = p.pos[j * K + c];
                         if (pr >= 0) {
+                            // pathway_term<true>, written out: called here, it makes ptxas spill block_kernel<4> and <8>
                             const Pathways& pw = p.pw;
                             const int64_t pbase = pw.path_ptr[p.active[c]];
                             for (int64_t e2 = pw.row_ptr[pr]; e2 < pw.row_ptr[pr + 1]; ++e2)
@@ -687,19 +677,10 @@ block_kernel(const BlockParams p) {
                             dg = pw.deg[pr];
                         }
                     }
-                    if (pr >= 0) {
-                        const double vp1 = v + 1.0;
-                        const double man = gamma * wv;                                           // :434
-                        const double ign = delta * (1.0 / (vp1 * vp1));                          // :438
-                        num = bb + (man + ign);                                                  // :440
-                        den = cden + gamma * (dg * v);                                           // :435,:441
-                    }
-                    if (den < kEps) den = kEps;                                                  // :442
-                    double vn = v * (num / den);                                                 // :443
-                    if (vn < kEps) vn = kEps;                                                    // :444
+                    const double vn = v_update_value(v, bb, cden, pr >= 0, wv, dg, gamma, delta);
                     aT[e] = vn;
                     Vnew[j * K + c] = vn;
-                    if (pr >= 0) p.hist_vh[(size_t)step * kVhCap + p.doff[c] + (pr - p.pw.path_ptr[p.active[c]])] = vn;
+                    if (pr >= 0) p.hist_vh[(size_t)step * kVhCap + active_slot(p.doff, c, pr, p.pw.path_ptr[p.active[c]])] = vn;
                     vb = fma(vn, bb, vb);
                 }
                 cons_bar();

@@ -243,8 +243,20 @@ __device__ __forceinline__ void gram_store(double* __restrict__ sBuf, int k, int
 }
 
 // ----------------------------------------------------------------------------------------------------
-// U update (:421-422) + per-block partials of U^T U (:425).  sum(U^2) (:359) is its trace.
-//   A = sum of the pass-1 partials ; den = U.Gv + U ; U <- U * (A / den  if den != 0 else 1)
+// Elementwise update rules (u_update_value here, pathway_term / v_update_value / active_slot after ActiveSet): one
+// definition for every kernel that updates U or V.  Keep each expression's shape: nvcc contracts device code into
+// FMAs, so a re-associated form changes bits.
+// ----------------------------------------------------------------------------------------------------
+
+// New U element from u, a = (X.V)[r][c] and ugv = (U.Gv)[r][c] (:421-422): 0/0 := 1, no clamp.  `a` is read only
+// when den != 0.
+__device__ __forceinline__ double u_update_value(double u, const double& a, double ugv) {
+    const double den = ugv + u;
+    return u * ((den != 0.0) ? a / den : 1.0);
+}
+
+// ----------------------------------------------------------------------------------------------------
+// U update (u_update_value) + per-block partials of U^T U (:425).  sum(U^2) (:359) is its trace.
 // Blocks of 1024 threads loop over row tiles; the tile of new U rows is staged in shared memory.
 // ----------------------------------------------------------------------------------------------------
 template <int NI>
@@ -268,13 +280,11 @@ u_update_kernel(double* __restrict__ U, const double* __restrict__ Apart, int ac
         for (int e = threadIdx.x; e < rows * k; e += blockDim.x) {
             const int r = e / k, c = e - r * k;
             const double* urow = U + (r0 + r) * k;
-            double den = 0.0;
-            for (int l = 0; l < k; ++l) den = fma(urow[l], sGv[l * k + c], den);
+            double ugv = 0.0;
+            for (int l = 0; l < k; ++l) ugv = fma(urow[l], sGv[l * k + c], ugv);
             const double u = urow[c];
-            den += u;
             const double a = sum_strided(Apart + (r0 + r) * k + c, achunks, m * k);      // X.V   (:420)
-            const double f = (den != 0.0) ? a / den : 1.0;                                  // 0/0 := 1 (:422)
-            sU[e] = u * f;
+            sU[e] = u_update_value(u, a, ugv);
         }
         __syncthreads();
         for (int e = threadIdx.x; e < rows * k; e += blockDim.x) U[r0 * k + e] = sU[e];
@@ -314,6 +324,44 @@ struct ActiveSet {
     const int32_t* off_factor;
     const double* off_coef;      // isd_r * (-w_rc * isd_c)   (0 for a self loop: it is part of diag(L))
 };
+
+// (W v)[j][c] of the V update (:434) over packed support row pr (gene j in factor c's active pathway).  kCg: read V_old
+// (leading dimension ld) through L2 only, as needed where other CTAs of the same launch wrote it.
+template <bool kCg>
+__device__ __forceinline__ double pathway_term(const Pathways& pw, const int32_t* active, int32_t pr, int c,
+                                               const double* Vold, int ld) {
+    const int64_t base = pw.path_ptr[active[c]];
+    double wv = 0.0;
+    for (int64_t e2 = pw.row_ptr[pr]; e2 < pw.row_ptr[pr + 1]; ++e2) {
+        const double* src = Vold + (int64_t)pw.support_idx[base + pw.col_local[e2]] * ld + c;
+        wv = fma(pw.w[e2], kCg ? __ldcg(src) : *src, wv);
+    }
+    return wv;
+}
+
+// New V element from v, b = (X^T.U)[j][c] and vgu = (V.Gu)[j][c] (:425-444).  On the support (wv = pathway_term,
+// deg = column sum of W) it adds the raw W / D terms, not the objective's normalised Laplacian; clamps at float32 eps.
+__device__ __forceinline__ double v_update_value(double v, double b, double vgu, bool in_support, double wv, double deg,
+                                                 double gamma, double delta) {
+    double num = b, den = vgu;
+    if (in_support) {
+        const double vp1 = v + 1.0;
+        const double man = gamma * wv;                          // :434
+        const double ign = delta * (1.0 / (vp1 * vp1));         // :438
+        num = b + (man + ign);                                  // :440
+        den = vgu + gamma * (deg * v);                          // :435, :441
+    }
+    if (den < kEps) den = kEps;
+    double vn = v * (num / den);                                // :443
+    if (vn < kEps) vn = kEps;
+    return vn;
+}
+
+// Index of (support row `row`, factor c) in the ActiveSet's diagonal order, which is also the order of the per-step
+// V_new values of the deferred objective (hist_vh).  path_begin = path_ptr[active[c]].
+__device__ __forceinline__ int64_t active_slot(const int64_t* doff, int c, int64_t row, int64_t path_begin) {
+    return doff[c] + (row - path_begin);
+}
 
 // ----------------------------------------------------------------------------------------------------
 // The X-stream kernel, used for BOTH passes:   Out[chunk][j][0:KT] = sum_{i in chunk} M[i][j] * W[i][0:KT]   (KT == k)
@@ -628,13 +676,11 @@ __device__ __forceinline__ void epi_u_update(const EpiParams& ep, unsigned char*
     for (int e = t; e < n_el; e += 256) {
         const int r = e / K, c = e - r * K;
         const double* urow = sU + r * K;
-        double den = 0.0;
+        double ugv = 0.0;
 #pragma unroll
-        for (int l = 0; l < K; ++l) den = fma(urow[l], sG[l * K + c], den);
+        for (int l = 0; l < K; ++l) ugv = fma(urow[l], sG[l * K + c], ugv);
         const double u = urow[c];
-        den += u;
-        const double f = (den != 0.0) ? sA[e] / den : 1.0;                                  // 0/0 := 1 (:422)
-        const double un = u * f;
+        const double un = u_update_value(u, sA[e], ugv);
         sT[e] = un;
         ep.Unew[base + e] = un;
     }
@@ -681,26 +727,13 @@ __device__ __forceinline__ void epi_v_update(const EpiParams& ep, unsigned char*
 #pragma unroll
         for (int l = 0; l < K; ++l) cden = fma(vrow[l], sG[l * K + c], cden);               // V.Gu   (:425)
         const double v = vrow[c];
-        double num = b, den = cden;
         const int32_t pr = ep.pos[j * K + c];
-        if (pr >= 0) {
-            const Pathways& pw = ep.pw;
-            const int64_t base = pw.path_ptr[ep.active[c]];
-            double wv = 0.0;
-            for (int64_t e2 = pw.row_ptr[pr]; e2 < pw.row_ptr[pr + 1]; ++e2)
-                wv = fma(pw.w[e2], ep.Vold[(int64_t)pw.support_idx[base + pw.col_local[e2]] * K + c], wv);
-            const double vp1 = v + 1.0;
-            const double man = gamma * wv;                                                  // :434
-            const double ign = delta * (1.0 / (vp1 * vp1));                                 // :438
-            num = b + (man + ign);                                                          // :440
-            den = cden + gamma * (pw.deg[pr] * v);                                          // :435,:441
-        }
-        if (den < kEps) den = kEps;                                                         // :442
-        double vn = v * (num / den);                                                        // :443
-        if (vn < kEps) vn = kEps;                                                           // :444
+        double wv = 0.0, dg = 0.0;
+        if (pr >= 0) { wv = pathway_term<false>(ep.pw, ep.active, pr, c, ep.Vold, K); dg = ep.pw.deg[pr]; }
+        const double vn = v_update_value(v, b, cden, pr >= 0, wv, dg, gamma, delta);
         sT[e] = vn;
         ep.Vnew[j * K + c] = vn;
-        if (pr >= 0 && ep.hist_vh != nullptr) ep.hist_vh[ep.doff[c] + (pr - ep.pw.path_ptr[ep.active[c]])] = vn;
+        if (pr >= 0 && ep.hist_vh != nullptr) ep.hist_vh[active_slot(ep.doff, c, pr, ep.pw.path_ptr[ep.active[c]])] = vn;
         vb = fma(vn, b, vb);
     }
     // sum(V_new * B) of this share: warp sums, then the 8 warp sums in order
@@ -1097,7 +1130,7 @@ static __global__ void build_active_kernel(Pathways pw, const int32_t* __restric
         const int32_t g = pw.support_idx[r];
         pos[(int64_t)g * k + c] = (int32_t)r;
         const double ir = pw.isd[r];
-        const int64_t di = doff[c] + (r - beg);
+        const int64_t di = active_slot(doff, c, r, beg);
         diag_gene[di] = g;
         diag_factor[di] = c;
         diag_coef[di] = ir * (pw.ldiag[r] * ir);
@@ -1107,7 +1140,7 @@ static __global__ void build_active_kernel(Pathways pw, const int32_t* __restric
             off_r[oi] = g;
             off_c[oi] = pw.support_idx[rc];
             off_lr[oi] = (int32_t)di;
-            off_lc[oi] = (int32_t)(doff[c] + (rc - beg));
+            off_lc[oi] = (int32_t)active_slot(doff, c, rc, beg);
             off_factor[oi] = c;
             off_coef[oi] = (rc == r) ? 0.0 : ir * (-pw.w[e2] * pw.isd[rc]);
         }
@@ -1348,22 +1381,10 @@ v_update_objective_kernel(const double* __restrict__ Vold, double* __restrict__ 
             double cden = 0.0;
             for (int l = 0; l < k; ++l) cden = fma(vrow[l], sGu[l * k + c], cden);       // V.Gu   (:425)
             const double v = vrow[c];
-            double num = b, den = cden;
             const int32_t pr = pos[(int64_t)j * k + c];
-            if (pr >= 0) {
-                const int64_t base = pw.path_ptr[active[c]];
-                double wv = 0.0;
-                for (int64_t e2 = pw.row_ptr[pr]; e2 < pw.row_ptr[pr + 1]; ++e2)
-                    wv = fma(pw.w[e2], Vold[(int64_t)pw.support_idx[base + pw.col_local[e2]] * k + c], wv);
-                const double vp1 = v + 1.0;
-                const double man = gamma * wv;                                          // :434
-                const double ign = delta * (1.0 / (vp1 * vp1));                         // :438
-                num = b + (man + ign);                                                  // :440
-                den = cden + gamma * (pw.deg[pr] * v);                                  // :435,:441
-            }
-            if (den < kEps) den = kEps;                                                 // :442
-            double vn = v * (num / den);                                                // :443
-            if (vn < kEps) vn = kEps;                                                   // :444
+            double wv = 0.0, dg = 0.0;
+            if (pr >= 0) { wv = pathway_term<false>(pw, active, pr, c, Vold, k); dg = pw.deg[pr]; }
+            const double vn = v_update_value(v, b, cden, pr >= 0, wv, dg, gamma, delta);
             sV[e] = vn;
             Vnew[(int64_t)j0 * k + e] = vn;
             vb = fma(vn, b, vb);
@@ -1480,9 +1501,7 @@ u_update_tiled_kernel(double* __restrict__ U, const double* __restrict__ Apart, 
                 const int c = tiled_col<CPT>(tx, j);
                 double v = 0.0;
                 if (row < m && c < k) {
-                    const double u0 = sU[r * LD + c];
-                    const double d = den[i][j] + u0;
-                    v = u0 * ((d != 0.0) ? sA[r * k + c] / d : 1.0);                              // 0/0 := 1 (:422)
+                    v = u_update_value(sU[r * LD + c], sA[r * k + c], den[i][j]);
                     U[row * k + c] = v;
                 }
                 un[i][j] = v;
@@ -1604,22 +1623,10 @@ v_update_tiled_kernel(const double* __restrict__ Vold, double* __restrict__ Vnew
                 if (jg < n && c < k) {
                     const double v = sV[r * LD + c];
                     const double b = sB[r * k + c];
-                    double num = b, dd = den[i][j];
                     const int32_t pr = pos[(int64_t)jg * k + c];
-                    if (pr >= 0) {
-                        const int64_t base = pw.path_ptr[active[c]];
-                        double wv = 0.0;
-                        for (int64_t e2 = pw.row_ptr[pr]; e2 < pw.row_ptr[pr + 1]; ++e2)
-                            wv = fma(pw.w[e2], Vold[(int64_t)pw.support_idx[base + pw.col_local[e2]] * k + c], wv);
-                        const double vp1 = v + 1.0;
-                        const double man = gamma * wv;                                      // :434
-                        const double ign = delta * (1.0 / (vp1 * vp1));                     // :438
-                        num = b + (man + ign);                                              // :440
-                        dd = den[i][j] + gamma * (pw.deg[pr] * v);                          // :435,:441
-                    }
-                    if (dd < kEps) dd = kEps;                                               // :442
-                    vn = v * (num / dd);                                                    // :443
-                    if (vn < kEps) vn = kEps;                                               // :444
+                    double wv = 0.0, dg = 0.0;
+                    if (pr >= 0) { wv = pathway_term<false>(pw, active, pr, c, Vold, k); dg = pw.deg[pr]; }
+                    vn = v_update_value(v, b, den[i][j], pr >= 0, wv, dg, gamma, delta);
                     Vnew[(int64_t)jg * k + c] = vn;
                     vb = fma(vn, b, vb);
                 }
