@@ -66,6 +66,26 @@ int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_glo
                    void* stream, int x_dtype);
 int prmf_x_dtype(const prmf_handle* h);
 
+/* Launch plan of the two X streams, as prmf_create_ex computes it for a handle on a device with `sm_count` SMs: pass 1
+ * (X.V) streams X^T (n rows, m_local columns), pass 2 (X^T.U) streams X (m_local rows, n columns).  The DFMA kernels run
+ * one CTA per (column panel, row chunk), each through a TMA ring of `stages` stages of 8 rows; `stages_override`
+ * (PRMF_TMA_STAGES, 0 for none) is kept when it lies in 2..12 and the rings of both passes fit 220 KB.  The tf32 fields
+ * are set for PRMF_X_TF32 only: tiles of 128 rows x chunks of columns on the tensor cores.  Plain host arithmetic: no
+ * device needed.  Returns PRMF_ERR_ARG on a bad shape, x_dtype or SM count. */
+typedef struct prmf_xstream_pass {
+    int64_t panels, panel_w, chunks, rows_per_chunk;
+    int64_t ring_smem;   /* bytes of the TMA ring */
+    int64_t tail_smem;   /* bytes a launch of this pass requests on a handle with fused U / V tails (k <= 10) */
+} prmf_xstream_pass;
+typedef struct prmf_xstream_plan {
+    int64_t fg, kt;      /* factor groups and factors per thread of the general-k kernel (k > 10; else 1, 0) */
+    int64_t stages;
+    prmf_xstream_pass pass1, pass2;
+    int64_t tc_tiles1, tc_chunks1, tc_cols_per_chunk1, tc_tiles2, tc_chunks2, tc_cols_per_chunk2, tc_stages, tc_smem;
+} prmf_xstream_plan;
+int prmf_plan_xstream(int64_t m_local, int64_t n, int k, int x_dtype, int sm_count, int stages_override,
+                      prmf_xstream_plan* out);
+
 /* Last error text of `h` (or of the last failed prmf_create when h is NULL). */
 const char* prmf_last_error(const prmf_handle* h);
 

@@ -1,7 +1,7 @@
 """ctypes binding of libprmf_b200.so (include/prmf_b200.h).  No torch types cross this boundary."""
 import ctypes
 import os
-from ctypes import POINTER, c_char_p, c_double, c_int, c_int32, c_int64, c_uint8, c_void_p
+from ctypes import POINTER, Structure, c_char_p, c_double, c_int, c_int32, c_int64, c_uint8, c_void_p
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libprmf_b200.so")
@@ -13,6 +13,18 @@ N_PHASES = 6
 X_DTYPES = {"f64": 0, "tf32": 1, "f32": 2}          # PRMF_X_F64 / PRMF_X_TF32 / PRMF_X_F32
 PHASES = ("xv", "u_update", "xtu", "reduce", "v_update", "objective")
 
+
+class XstreamPass(Structure):
+    _fields_ = [(name, c_int64) for name in ("panels", "panel_w", "chunks", "rows_per_chunk", "ring_smem", "tail_smem")]
+
+
+class XstreamPlan(Structure):
+    """prmf_xstream_plan: the launch plan of the two X-stream passes (prmf_plan_xstream)."""
+    _fields_ = [("fg", c_int64), ("kt", c_int64), ("stages", c_int64), ("pass1", XstreamPass), ("pass2", XstreamPass)] + \
+               [(name, c_int64) for name in ("tc_tiles1", "tc_chunks1", "tc_cols_per_chunk1", "tc_tiles2", "tc_chunks2",
+                                             "tc_cols_per_chunk2", "tc_stages", "tc_smem")]
+
+
 # every symbol include/prmf_b200.h declares: name -> (restype, argtypes)
 _P = c_void_p
 SYMBOLS = {
@@ -20,6 +32,7 @@ SYMBOLS = {
     "prmf_create": (c_int, [POINTER(_P), c_int, c_int64, c_int64, c_int64, c_int, _P]),
     "prmf_create_ex": (c_int, [POINTER(_P), c_int, c_int64, c_int64, c_int64, c_int, _P, c_int]),
     "prmf_x_dtype": (c_int, [_P]),
+    "prmf_plan_xstream": (c_int, [c_int64, c_int64, c_int, c_int, c_int, c_int, POINTER(XstreamPlan)]),
     "prmf_destroy": (c_int, [_P]),
     "prmf_last_error": (c_char_p, [_P]),
     "prmf_set_X": (c_int, [_P, _P, c_int64]),

@@ -174,14 +174,7 @@ struct prmf_handle {
     int uu_grid = 0, uu_rows = 0, vu_grid = 0, vu_rows = 0;
     int nq = 1, ni = 1;
     unsigned int* ticket = nullptr;
-    // fp64 X-stream kernels (TMA ring of tma_stages stages of kTmaRS rows)
-    int tma_fg = 1, tma_kt = 0;               // factor groups / factors per thread of the general-k kernel
-    int tma_stages = 3;
-    int panels1 = 0, panel_w1 = 0, chunks1 = 0;      // pass 1: panels over samples, chunks over genes
-    int64_t rows_per_chunk1 = 0;
-    int panels = 0, panel_w = 0, chunks = 0;         // pass 2: panels over genes, chunks over samples
-    int64_t rows_per_chunk = 0;
-    size_t tma_smem1 = 0, tma_smem2 = 0;
+    prmf_xstream_plan plan{};                 // both X-stream passes (prmf_plan_xstream)
 
     // large k (> 16): register-tiled U update, Gram partials folded by gram_reduce_kernel, objective as its own launch
     bool big_k = false;
@@ -192,7 +185,7 @@ struct prmf_handle {
 
     // fused tails (k <= 10, TMA path): the U / V updates run in the last CTA of each panel of the X-stream kernels
     bool use_epi = false;
-    unsigned long long* epi_counters = nullptr;   // arrive | done, each [panels1 + panels], monotone over launches
+    unsigned long long* epi_counters = nullptr;   // arrive | done, each [pass-1 + pass-2 panels], monotone over launches
     unsigned long long epi_seq1 = 0, epi_seq2 = 0;
     // deferred objective: per-step history [obj_capacity] of what the objective needs (one cudaMalloc)
     double* hist = nullptr;
@@ -229,8 +222,6 @@ struct prmf_handle {
     int Kp = 0;
     CUtensorMap tm_X{}, tm_Xt{}, tm_Vt{}, tm_Ut{};
     TcParams tc1{}, tc2{};                    // pass 1: M = X (m x n), W = V^T; pass 2: M = X^T (n x m), W = U^T
-    int tc_tiles1 = 0, tc_chunks1 = 0, tc_tiles2 = 0, tc_chunks2 = 0;
-    size_t tc_smem = 0;
 
     // multi-GPU
     NcclComm comm = nullptr;
@@ -323,16 +314,21 @@ auto tma_kernel(const double*) { return skinny_tma_kernel<KT, kTmaRS, EPI>; }
 template <int KT, int EPI>
 auto tma_kernel(const float*) { return skinny_tma_f32_kernel<KT, kTmaRS, EPI>; }
 
+// every launch of a pass on a fused-tail handle requests the tail's shared memory
+size_t pass_smem(const prmf_handle* h, const prmf_xstream_pass& p) { return h->use_epi ? p.tail_smem : p.ring_smem; }
+
 template <int KT, typename T>
 int launch_skinny_tma_t(prmf_handle* h, const T* M, int64_t ldm, int64_t rows, int64_t cols, const double* W,
-                        int panels, int panel_w, int chunks, int64_t rows_per_chunk, size_t smem, double* out) {
-    dim3 grid(panels, chunks);
+                        const prmf_xstream_pass& p, double* out) {
+    dim3 grid(p.panels, p.chunks);
     EpiParams none{};
     none.dbg_slot = -1;
     none.err = h->err_word; none.timeout_ns = h->spin_timeout_ns;
     const auto fn = tma_kernel<KT, 0>(M);
+    const size_t smem = pass_smem(h, p);
     CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    fn<<<grid, kTmaThreads, smem, h->stream>>>(M, ldm, rows, cols, W, panel_w, rows_per_chunk, h->tma_stages, out, none);
+    fn<<<grid, kTmaThreads, smem, h->stream>>>(M, ldm, rows, cols, W, p.panel_w, p.rows_per_chunk, h->plan.stages, out,
+                                               none);
     return PRMF_OK;
 }
 
@@ -340,13 +336,13 @@ int launch_skinny_tma_t(prmf_handle* h, const T* M, int64_t ldm, int64_t rows, i
 // of a panel wait for each other, so the launch is cooperative (all CTAs co-resident or the launch fails).
 template <int KT, typename T>
 int launch_skinny_epi_t(prmf_handle* h, int epi, const T* M, int64_t ldm, int64_t rows, int64_t cols,
-                        const double* W, int panels, int panel_w, int chunks, int64_t rows_per_chunk, size_t smem,
-                        double* out, const EpiParams& ep_in) {
-    dim3 grid(panels, chunks);
+                        const double* W, const prmf_xstream_pass& p, double* out, const EpiParams& ep_in) {
+    dim3 grid(p.panels, p.chunks);
     EpiParams ep = ep_in;
-    int stages = h->tma_stages;
+    int panel_w = (int)p.panel_w, stages = (int)h->plan.stages;     // the kernel's parameter types
+    const size_t smem = pass_smem(h, p);
     void* args[] = {(void*)&M, (void*)&ldm, (void*)&rows, (void*)&cols, (void*)&W, (void*)&panel_w,
-                    (void*)&rows_per_chunk, (void*)&stages, (void*)&out, (void*)&ep};
+                    (void*)&p.rows_per_chunk, (void*)&stages, (void*)&out, (void*)&ep};
     const void* fn = nullptr;
     switch (epi) {
         case 1: fn = (const void*)tma_kernel<KT, 1>(M); break;
@@ -367,24 +363,25 @@ auto gen_kernel(const float*) { return skinny_tma_gen_f32_kernel<KT, FG, kTmaRS>
 
 template <int KT, int FG, typename T>
 int launch_skinny_gen_t(prmf_handle* h, const T* M, int64_t ldm, int64_t rows, int64_t cols, const double* W,
-                        int panels, int panel_w, int chunks, int64_t rows_per_chunk, size_t smem, double* out) {
-    dim3 grid(panels, chunks);
+                        const prmf_xstream_pass& p, double* out) {
+    dim3 grid(p.panels, p.chunks);
     const auto fn = gen_kernel<KT, FG>(M);
+    const size_t smem = pass_smem(h, p);
     CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    fn<<<grid, kTmaThreads, smem, h->stream>>>(M, ldm, rows, cols, W, h->k, panel_w, rows_per_chunk, h->tma_stages, out);
+    fn<<<grid, kTmaThreads, smem, h->stream>>>(M, ldm, rows, cols, W, h->k, p.panel_w, p.rows_per_chunk, h->plan.stages,
+                                               out);
     return PRMF_OK;
 }
 
 template <typename T>
 int launch_skinny_gen(prmf_handle* h, const T* M, int64_t ldm, int64_t rows, int64_t cols, const double* W,
-                      int panels, int panel_w, int chunks, int64_t rows_per_chunk, size_t smem, double* out) {
+                      const prmf_xstream_pass& p, double* out) {
 #define GEN_CASE(KT_, FG_) \
-    if (h->tma_kt == KT_ && h->tma_fg == FG_) \
-        return launch_skinny_gen_t<KT_, FG_>(h, M, ldm, rows, cols, W, panels, panel_w, chunks, rows_per_chunk, smem, out);
+    if (h->plan.kt == KT_ && h->plan.fg == FG_) return launch_skinny_gen_t<KT_, FG_>(h, M, ldm, rows, cols, W, p, out);
     GEN_CASE(12, 1) GEN_CASE(16, 1) GEN_CASE(8, 2) GEN_CASE(12, 2) GEN_CASE(16, 2) GEN_CASE(8, 4) GEN_CASE(12, 4)
     GEN_CASE(16, 4) GEN_CASE(8, 8) GEN_CASE(12, 8) GEN_CASE(16, 8)
 #undef GEN_CASE
-    return fail(h, PRMF_ERR_STATE, "no general-k kernel for KT=%d FG=%d", h->tma_kt, h->tma_fg);
+    return fail(h, PRMF_ERR_STATE, "no general-k kernel for KT=%d FG=%d", (int)h->plan.kt, (int)h->plan.fg);
 }
 
 #define KT_SWITCH_RC(kt, rc, FN, ...)          \
@@ -402,14 +399,14 @@ int launch_skinny_gen(prmf_handle* h, const T* M, int64_t ldm, int64_t rows, int
     }
 
 // number of per-chunk partials the passes leave in Apart / Bpart
-int a_chunks(const prmf_handle* h) { return h->x_tc ? h->tc_chunks1 : h->chunks1; }
-int b_chunks(const prmf_handle* h) { return h->x_tc ? h->tc_chunks2 : h->chunks; }
+int a_chunks(const prmf_handle* h) { return (int)(h->x_tc ? h->plan.tc_chunks1 : h->plan.pass1.chunks); }
+int b_chunks(const prmf_handle* h) { return (int)(h->x_tc ? h->plan.tc_chunks2 : h->plan.pass2.chunks); }
 
 // TF32 mode: one tensor-core kernel serves both passes
-int launch_tc(prmf_handle* h, const CUtensorMap& tmM, const CUtensorMap& tmW, const TcParams& prm, int tiles, int chunks,
-              const char* name) {
+int launch_tc(prmf_handle* h, const CUtensorMap& tmM, const CUtensorMap& tmW, const TcParams& prm, int64_t tiles,
+              int64_t chunks, const char* name) {
     dim3 grid(tiles, chunks);
-    tc_rowdot_kernel<<<grid, kTcThreads, h->tc_smem, h->stream>>>(tmM, tmW, prm);
+    tc_rowdot_kernel<<<grid, kTcThreads, h->plan.tc_smem, h->stream>>>(tmM, tmW, prm);
     LAUNCH_CHECK(name);
     return PRMF_OK;
 }
@@ -426,20 +423,19 @@ int refresh_wt(prmf_handle* h, const double* W, int64_t rows, float* Wt, int64_t
 // pass 1: A partials = Xt^T . V   (M = Xt: n rows x m cols)
 int launch_xv(prmf_handle* h) {
     if (h->m == 0) return PRMF_OK;
-    if (h->x_tc) return launch_tc(h, h->tm_X, h->tm_Vt, h->tc1, h->tc_tiles1, h->tc_chunks1, "tc_rowdot_kernel(pass 1)");
+    if (h->x_tc)
+        return launch_tc(h, h->tm_X, h->tm_Vt, h->tc1, h->plan.tc_tiles1, h->plan.tc_chunks1, "tc_rowdot_kernel(pass 1)");
+    const prmf_xstream_pass& p = h->plan.pass1;
+    const double* V = h->Vbuf[h->vcur];
     int rc = 0;
     if (h->x32 && h->k > 10) {
-        rc = launch_skinny_gen(h, h->Xt32, h->ldxt32, h->n, h->m, h->Vbuf[h->vcur], h->panels1, h->panel_w1, h->chunks1,
-                               h->rows_per_chunk1, h->tma_smem1, h->Apart);
+        rc = launch_skinny_gen(h, h->Xt32, h->ldxt32, h->n, h->m, V, p, h->Apart);
     } else if (h->x32) {
-        KT_SWITCH_RC(h->k, rc, launch_skinny_tma_t, h, h->Xt32, h->ldxt32, h->n, h->m, h->Vbuf[h->vcur], h->panels1,
-                     h->panel_w1, h->chunks1, h->rows_per_chunk1, h->tma_smem1, h->Apart);
+        KT_SWITCH_RC(h->k, rc, launch_skinny_tma_t, h, h->Xt32, h->ldxt32, h->n, h->m, V, p, h->Apart);
     } else if (h->k > 10) {
-        rc = launch_skinny_gen(h, h->Xt, h->ldxt, h->n, h->m, h->Vbuf[h->vcur], h->panels1, h->panel_w1, h->chunks1,
-                               h->rows_per_chunk1, h->tma_smem1, h->Apart);
+        rc = launch_skinny_gen(h, h->Xt, h->ldxt, h->n, h->m, V, p, h->Apart);
     } else {
-        KT_SWITCH_RC(h->k, rc, launch_skinny_tma_t, h, h->Xt, h->ldxt, h->n, h->m, h->Vbuf[h->vcur], h->panels1,
-                     h->panel_w1, h->chunks1, h->rows_per_chunk1, h->tma_smem1, h->Apart);
+        KT_SWITCH_RC(h->k, rc, launch_skinny_tma_t, h, h->Xt, h->ldxt, h->n, h->m, V, p, h->Apart);
     }
     if (rc) return rc;
     LAUNCH_CHECK("skinny_tma_kernel(pass 1)");
@@ -455,21 +451,18 @@ int launch_xtu(prmf_handle* h) {
     if (h->x_tc) {
         int rc = refresh_wt(h, h->U, h->m, h->Ut32, h->ldxt32);
         if (rc) return rc;
-        return launch_tc(h, h->tm_Xt, h->tm_Ut, h->tc2, h->tc_tiles2, h->tc_chunks2, "tc_rowdot_kernel(pass 2)");
+        return launch_tc(h, h->tm_Xt, h->tm_Ut, h->tc2, h->plan.tc_tiles2, h->plan.tc_chunks2, "tc_rowdot_kernel(pass 2)");
     }
+    const prmf_xstream_pass& p = h->plan.pass2;
     int rc = 0;
     if (h->x32 && h->k > 10) {
-        rc = launch_skinny_gen(h, h->X32, h->ldx32, h->m, h->n, h->U, h->panels, h->panel_w, h->chunks, h->rows_per_chunk,
-                               h->tma_smem2, h->Bpart);
+        rc = launch_skinny_gen(h, h->X32, h->ldx32, h->m, h->n, h->U, p, h->Bpart);
     } else if (h->x32) {
-        KT_SWITCH_RC(h->k, rc, launch_skinny_tma_t, h, h->X32, h->ldx32, h->m, h->n, h->U, h->panels, h->panel_w, h->chunks,
-                     h->rows_per_chunk, h->tma_smem2, h->Bpart);
+        KT_SWITCH_RC(h->k, rc, launch_skinny_tma_t, h, h->X32, h->ldx32, h->m, h->n, h->U, p, h->Bpart);
     } else if (h->k > 10) {
-        rc = launch_skinny_gen(h, h->X, h->ldx, h->m, h->n, h->U, h->panels, h->panel_w, h->chunks, h->rows_per_chunk,
-                               h->tma_smem2, h->Bpart);
+        rc = launch_skinny_gen(h, h->X, h->ldx, h->m, h->n, h->U, p, h->Bpart);
     } else {
-        KT_SWITCH_RC(h->k, rc, launch_skinny_tma_t, h, h->X, h->ldx, h->m, h->n, h->U, h->panels, h->panel_w, h->chunks,
-                     h->rows_per_chunk, h->tma_smem2, h->Bpart);
+        KT_SWITCH_RC(h->k, rc, launch_skinny_tma_t, h, h->X, h->ldx, h->m, h->n, h->U, p, h->Bpart);
     }
     if (rc) return rc;
     LAUNCH_CHECK("skinny_tma_kernel(pass 2)");
@@ -680,9 +673,8 @@ int ensure_pos(prmf_handle* h) {
 int launch_xv_epi(prmf_handle* h, const double* gv_src = nullptr, int gv_parts = 1) {
     EpiParams ep{};
     ep.err = h->err_word; ep.timeout_ns = h->spin_timeout_ns;
-    const size_t np = (size_t)h->panels1 + h->panels;
     ep.arrive = h->epi_counters;
-    ep.done = h->epi_counters + np;
+    ep.done = h->epi_counters + h->plan.pass1.panels + h->plan.pass2.panels;
     ep.seq = ++h->epi_seq1;
     ep.dbg_slot = (int)((2 * (h->epi_seq1 - 1)) % 64);
     ep.part2 = h->epi_part2;
@@ -694,11 +686,11 @@ int launch_xv_epi(prmf_handle* h, const double* gv_src = nullptr, int gv_parts =
     ep.Gu_part = h->Gu_part;
     int rc = 0;
     if (h->x32) {
-        KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, 1, h->Xt32, h->ldxt32, h->n, h->m, h->Vbuf[h->vcur], h->panels1,
-                     h->panel_w1, h->chunks1, h->rows_per_chunk1, h->tma_smem1, h->Apart, ep);
+        KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, 1, h->Xt32, h->ldxt32, h->n, h->m, h->Vbuf[h->vcur],
+                     h->plan.pass1, h->Apart, ep);
     } else {
-        KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, 1, h->Xt, h->ldxt, h->n, h->m, h->Vbuf[h->vcur], h->panels1,
-                     h->panel_w1, h->chunks1, h->rows_per_chunk1, h->tma_smem1, h->Apart, ep);
+        KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, 1, h->Xt, h->ldxt, h->n, h->m, h->Vbuf[h->vcur], h->plan.pass1,
+                     h->Apart, ep);
     }
     if (rc) { h->failed = true; return rc; }     // the panel counters expect this launch: no further steps on this handle
     LAUNCH_CHECK("skinny_tma_kernel(pass 1 + U update)");
@@ -710,15 +702,15 @@ int launch_xv_epi(prmf_handle* h, const double* gv_src = nullptr, int gv_parts =
 int launch_xtu_epi(prmf_handle* h, int mode, double* packed_dst, int hist_slot = -1) {
     EpiParams ep{};
     ep.err = h->err_word; ep.timeout_ns = h->spin_timeout_ns;
-    const size_t np = (size_t)h->panels1 + h->panels;
-    ep.arrive = h->epi_counters + h->panels1;
-    ep.done = h->epi_counters + np + h->panels1;
+    const int64_t panels1 = h->plan.pass1.panels, panels2 = h->plan.pass2.panels;
+    ep.arrive = h->epi_counters + panels1;
+    ep.done = h->epi_counters + panels1 + panels2 + panels1;
     ep.seq = ++h->epi_seq2;
     ep.dbg_slot = (int)((2 * (h->epi_seq2 - 1) + 1) % 64);
     ep.part2 = h->epi_part2;
     ep.vb2 = h->epi_vb2;
     ep.Gu_part_in = h->Gu_part;
-    ep.gu_parts = h->panels1;
+    ep.gu_parts = (int)panels1;
     if (mode == 3) {
         ep.red = packed_dst;
     } else {
@@ -732,8 +724,8 @@ int launch_xtu_epi(prmf_handle* h, int mode, double* packed_dst, int hist_slot =
         ep.VB_part = h->VB_part;
         if (hist_slot >= 0) {                       // deferred objective: this step's slots
             const size_t kk2 = (size_t)h->k * h->k;
-            ep.Gv_part = h->hist_Gvp + (size_t)hist_slot * h->panels * kk2;
-            ep.VB_part = h->hist_VBp + (size_t)hist_slot * h->panels;
+            ep.Gv_part = h->hist_Gvp + (size_t)hist_slot * panels2 * kk2;
+            ep.VB_part = h->hist_VBp + (size_t)hist_slot * panels2;
             ep.hist_Gu = h->hist_Gu + (size_t)hist_slot * kk2;
             ep.hist_vh = h->hist_vh + (size_t)hist_slot * kVhCap;
             ep.doff = h->as_off;
@@ -741,11 +733,10 @@ int launch_xtu_epi(prmf_handle* h, int mode, double* packed_dst, int hist_slot =
     }
     int rc = 0;
     if (h->x32) {
-        KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, mode, h->X32, h->ldx32, h->m, h->n, h->U, h->panels, h->panel_w,
-                     h->chunks, h->rows_per_chunk, h->tma_smem2, h->Bpart, ep);
+        KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, mode, h->X32, h->ldx32, h->m, h->n, h->U, h->plan.pass2, h->Bpart,
+                     ep);
     } else {
-        KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, mode, h->X, h->ldx, h->m, h->n, h->U, h->panels, h->panel_w,
-                     h->chunks, h->rows_per_chunk, h->tma_smem2, h->Bpart, ep);
+        KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, mode, h->X, h->ldx, h->m, h->n, h->U, h->plan.pass2, h->Bpart, ep);
     }
     if (rc) { h->failed = true; return rc; }
     LAUNCH_CHECK(mode == 3 ? "skinny_tma_kernel(pass 2 + pack)" : "skinny_tma_kernel(pass 2 + V update)");
@@ -756,8 +747,8 @@ int launch_xtu_epi(prmf_handle* h, int mode, double* packed_dst, int hist_slot =
 // fused-tail path (k <= 10): objective of the step from the per-panel partials the pass-2 kernel left
 int launch_objective(prmf_handle* h, double tradeoff, const double* Gu_parts, int gu_parts) {
     objective_parts_kernel<<<1, kTailThreads, obj_smem(h), h->stream>>>(
-        h->Vbuf[h->vcur], h->k, Gu_parts, gu_parts, h->Gv_part, h->VB_part, h->panels, h->normX_sq, h->as, h->Gv, h->gd,
-        tradeoff, h->obj, h->step_counter, h->obj_capacity);
+        h->Vbuf[h->vcur], h->k, Gu_parts, gu_parts, h->Gv_part, h->VB_part, h->plan.pass2.panels, h->normX_sq, h->as,
+        h->Gv, h->gd, tradeoff, h->obj, h->step_counter, h->obj_capacity);
     LAUNCH_CHECK("objective_parts_kernel");
     return PRMF_OK;
 }
@@ -813,9 +804,10 @@ int launch_block(prmf_handle* h, int h0, int nh) {
     if (nh <= 0) return PRMF_OK;
     BlockParams prm{};
     prm.X = h->X; prm.Xt = h->Xt; prm.ldx = h->ldx; prm.ldxt = h->ldxt; prm.m = h->m; prm.n = h->n;
-    prm.panels1 = h->panels1; prm.panel_w1 = h->panel_w1; prm.chunks1 = h->chunks1; prm.rpc1 = h->rows_per_chunk1;
-    prm.panels2 = h->panels; prm.panel_w2 = h->panel_w; prm.chunks2 = h->chunks; prm.rpc2 = h->rows_per_chunk;
-    prm.stages = h->tma_stages;
+    const prmf_xstream_pass &p1 = h->plan.pass1, &p2 = h->plan.pass2;
+    prm.panels1 = p1.panels; prm.panel_w1 = p1.panel_w; prm.chunks1 = p1.chunks; prm.rpc1 = p1.rows_per_chunk;
+    prm.panels2 = p2.panels; prm.panel_w2 = p2.panel_w; prm.chunks2 = p2.chunks; prm.rpc2 = p2.rows_per_chunk;
+    prm.stages = h->plan.stages;
     prm.ring_stage_bytes = h->blk_stage_bytes;
     prm.U[0] = h->U; prm.U[1] = h->U2;
     prm.V[0] = h->Vbuf[h->vcur]; prm.V[1] = h->Vbuf[h->vcur ^ 1];
@@ -823,10 +815,10 @@ int launch_block(prmf_handle* h, int h0, int nh) {
     prm.part2 = h->epi_part2; prm.vb2 = h->epi_vb2;
     prm.Gv0 = h->Gv;
     unsigned long long* c = h->blk_ctr;
-    prm.arrive1 = c; c += h->panels1;
-    prm.done1 = c; c += h->panels1;
-    prm.arrive2 = c; c += h->panels;
-    prm.done2 = c; c += h->panels;
+    prm.arrive1 = c; c += p1.panels;
+    prm.done1 = c; c += p1.panels;
+    prm.arrive2 = c; c += p2.panels;
+    prm.done2 = c; c += p2.panels;
     prm.udone = c; prm.vdone = c + 1; prm.ufold = c + 2; prm.vfold = c + 3;
     prm.base1 = h->blk_n1; prm.base2 = h->blk_n2;
     prm.h0 = h0; prm.nh = nh;
@@ -844,7 +836,7 @@ int launch_block(prmf_handle* h, int h0, int nh) {
     }
     int n_p1 = 0, n_p2 = 0;
     for (int i = 0; i < nh; ++i) (((h0 + i) & 1) == 0 ? n_p1 : n_p2)++;
-    const int grid = std::max(h->panels1 * h->chunks1, h->panels * h->chunks);
+    const int grid = (int)std::max(p1.panels * p1.chunks, p2.panels * p2.chunks);
     cudaError_t e_ = prmf_launch_block_kernel(h->k, prm, grid, h->blk_smem, h->stream);
     if (e_ == cudaSuccess) e_ = cudaGetLastError();
     if (e_ != cudaSuccess) {                      // the counters below only move for a launch that is really queued
@@ -969,7 +961,7 @@ int enqueue_steps(prmf_handle* h, int n_steps, double gamma, double delta, doubl
         h->ahead = 0;
         if ((rc = launch_block(h, h0, 2 * n_steps - h0))) return rc;
         objective_deferred_kernel<<<n_steps, kTailThreads, obj_smem(h), h->stream>>>(
-            h->k, h->hist_Gu, h->hist_Gvp, h->hist_VBp, h->panels, h->hist_vh, kVhCap, h->normX_sq, h->as, h->Gv,
+            h->k, h->hist_Gu, h->hist_Gvp, h->hist_VBp, h->plan.pass2.panels, h->hist_vh, kVhCap, h->normX_sq, h->as, h->Gv,
             h->gd, h->obj, h->obj_capacity);
         LAUNCH_CHECK("objective_deferred_kernel");
         return PRMF_OK;
@@ -984,13 +976,14 @@ int enqueue_steps(prmf_handle* h, int n_steps, double gamma, double delta, doubl
             // one GPU, fixed gamma / delta: the objective of every step is evaluated by ONE launch after the block
             if (!skip_pass1) {
                 const size_t kk2s = (size_t)h->k * h->k;
-                rc = s == 0 ? launch_xv_epi(h) : launch_xv_epi(h, h->hist_Gvp + (size_t)(s - 1) * h->panels * kk2s, h->panels);
+                const int64_t panels2 = h->plan.pass2.panels;
+                rc = s == 0 ? launch_xv_epi(h) : launch_xv_epi(h, h->hist_Gvp + (size_t)(s - 1) * panels2 * kk2s, (int)panels2);
                 if (rc) return rc;
             }
             if ((rc = launch_xtu_epi(h, 2, nullptr, s))) return rc;
             if (s == n_steps - 1) {
                 objective_deferred_kernel<<<n_steps, kTailThreads, obj_smem(h), h->stream>>>(
-                    h->k, h->hist_Gu, h->hist_Gvp, h->hist_VBp, h->panels, h->hist_vh, kVhCap, h->normX_sq, h->as, h->Gv,
+                    h->k, h->hist_Gu, h->hist_Gvp, h->hist_VBp, h->plan.pass2.panels, h->hist_vh, kVhCap, h->normX_sq, h->as, h->Gv,
                     h->gd, h->obj, h->obj_capacity);
                 LAUNCH_CHECK("objective_deferred_kernel");
             }
@@ -1002,7 +995,7 @@ int enqueue_steps(prmf_handle* h, int n_steps, double gamma, double delta, doubl
             if (!sharded(h)) {
                 tic(2); rc = launch_xtu_epi(h, 2, nullptr); toc();               // + V update
                 if (rc) return rc;
-                tic(5); rc = launch_objective(h, tradeoff, h->Gu_part, h->panels1); toc();
+                tic(5); rc = launch_objective(h, tradeoff, h->Gu_part, h->plan.pass1.panels); toc();
                 if (rc) return rc;
             } else {
                 double* dst = h->p2p_ready ? h->p2p_buf + (size_t)h->p2p_parity * h->p2p_red_count : h->red;
@@ -1114,9 +1107,9 @@ int make_tensor_map(prmf_handle* h, CUtensorMap* map, const float* base, int64_t
 
 // Tiles of 128 rows x column chunks: pick the smallest chunk count whose wave quantisation over the
 // 2 x SM-count resident CTAs is within 3 % of the best one.
-void plan_tc(const prmf_handle* h, int64_t R, int64_t C, int* tiles, int* chunks, int64_t* cols_per_chunk) {
-    *tiles = (int)std::max<int64_t>(1, (R + kTcTileRows - 1) / kTcTileRows);
-    const double slots = 2.0 * h->sm_count;
+void plan_tc(int sm_count, int64_t R, int64_t C, int64_t* tiles, int64_t* chunks, int64_t* cols_per_chunk) {
+    *tiles = std::max<int64_t>(1, (R + kTcTileRows - 1) / kTcTileRows);
+    const double slots = 2.0 * sm_count;
     const int max_chunks = (int)std::max<int64_t>(1, std::min<int64_t>(64, C / 512));
     double best = 0.0;
     std::vector<double> eff(max_chunks + 1, 0.0);
@@ -1129,32 +1122,23 @@ void plan_tc(const prmf_handle* h, int64_t R, int64_t C, int* tiles, int* chunks
     for (int c = 1; c <= max_chunks; ++c)
         if (eff[c] >= best - 0.03) { pick = c; break; }
     *cols_per_chunk = round_up(std::max<int64_t>(1, (C + pick - 1) / pick), kTcBlockK);
-    *chunks = (int)std::max<int64_t>(1, (C + *cols_per_chunk - 1) / *cols_per_chunk);
+    *chunks = std::max<int64_t>(1, (C + *cols_per_chunk - 1) / *cols_per_chunk);
 }
 
-int setup_tf32(prmf_handle* h) {
-    const int k = h->k;
-    h->Kp = (int)round_up(k, 16);
-    h->ldx32 = round_up(h->n, 32);
-    h->ldxt32 = round_up(std::max<int64_t>(1, h->m), 32);
-    int64_t cpc1 = 0, cpc2 = 0;
-    plan_tc(h, h->m, h->n, &h->tc_tiles1, &h->tc_chunks1, &cpc1);
-    plan_tc(h, h->n, h->m, &h->tc_tiles2, &h->tc_chunks2, &cpc2);
-    const size_t stage = (size_t)kTcTileRows * kTcBlockK * 4 + (size_t)h->Kp * kTcBlockK * 4;
-    int stages = (int)((108 * 1024) / stage);                      // two CTAs per SM
-    stages = std::max(2, std::min(8, stages));
-    h->tc_smem = (size_t)stages * stage + (2 * stages + 1) * sizeof(uint64_t) + 16 + 1024;
+void setup_tf32(prmf_handle* h) {
+    const prmf_xstream_plan& p = h->plan;
+    h->Kp = (int)round_up(h->k, 16);
     uint32_t tcols = 32;
     while ((int)tcols < h->Kp) tcols <<= 1;
-    h->tc1 = TcParams{h->m, h->n, k, h->Kp, cpc1, stages, tcols, nullptr};
-    h->tc2 = TcParams{h->n, h->m, k, h->Kp, cpc2, stages, tcols, nullptr};
-    return PRMF_OK;
+    const int stages = (int)p.tc_stages;
+    h->tc1 = TcParams{h->m, h->n, h->k, h->Kp, p.tc_cols_per_chunk1, stages, tcols, nullptr};
+    h->tc2 = TcParams{h->n, h->m, h->k, h->Kp, p.tc_cols_per_chunk2, stages, tcols, nullptr};
 }
 
 int finish_setup_tf32(prmf_handle* h) {
     h->tc1.Out = h->Apart;
     h->tc2.Out = h->Bpart;
-    CU(cudaFuncSetAttribute(tc_rowdot_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->tc_smem));
+    CU(cudaFuncSetAttribute(tc_rowdot_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->plan.tc_smem));
     CU(cudaFuncSetAttribute(tc_rowdot_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
     int rc = 0;
     if (h->m > 0) {
@@ -1363,6 +1347,65 @@ int prmf_abi_version(void) { return 1; }
 
 const char* prmf_last_error(const prmf_handle* h) { return h ? h->err.c_str() : g_create_error.c_str(); }
 
+int prmf_plan_xstream(int64_t m_local, int64_t n, int k, int x_dtype, int sm_count, int stages_override,
+                      prmf_xstream_plan* out) {
+    if (!out || m_local < 0 || n <= 0 || k <= 0 || k > 128 || sm_count <= 0 ||
+        (x_dtype != PRMF_X_F64 && x_dtype != PRMF_X_TF32 && x_dtype != PRMF_X_F32))
+        return PRMF_ERR_ARG;
+    prmf_xstream_plan p{};
+    // DFMA kernels: one CTA per SM, column panels of at most 1024 / FG columns, row chunks of at least 4 stages.  The
+    // panels and chunks do not depend on the storage type, which is what makes an fp32 handle bitwise equal to an fp64
+    // handle on the widened matrix; only the ring differs (an fp32 stage holds half the bytes of X).
+    const bool x32 = x_dtype != PRMF_X_F64;
+    p.fg = 1;
+    if (k > 10) {                          // general-k kernel: FG factor groups x KT factors per thread
+        const int groups = (k + 15) / 16;
+        p.fg = groups <= 1 ? 1 : groups <= 2 ? 2 : groups <= 4 ? 4 : 8;
+        const int64_t per = (k + p.fg - 1) / p.fg;
+        p.kt = per <= 8 ? 8 : per <= 12 ? 12 : 16;
+    }
+    const int64_t max_panel = 1024 / p.fg;
+    auto plan = [&](int64_t cols, int64_t rows, prmf_xstream_pass& q) {
+        q.panels = std::max<int64_t>(1, (cols + max_panel - 1) / max_panel);
+        q.panel_w = round_up((std::max<int64_t>(1, cols) + q.panels - 1) / q.panels, 4);
+        q.chunks = std::max<int64_t>(1, sm_count / q.panels);
+        q.chunks = std::min<int64_t>(q.chunks, std::max<int64_t>(1, rows / (4 * kTmaRS)));
+        // rows per chunk: even (the W rows of a chunk must start 16-byte aligned for the bulk copies), not a multiple
+        // of the stage height -- a ragged last stage costs less than a last chunk that is nearly empty
+        q.rows_per_chunk = round_up(std::max<int64_t>(1, (rows + q.chunks - 1) / q.chunks), 2);
+        const int64_t xb = kTmaRS * q.panel_w * (x32 ? 4 : 8);
+        const int64_t wb = ((kTmaRS * (int64_t)k + 16) * 8 + 127) & ~(int64_t)127;
+        q.ring_smem = p.stages * (xb + wb) + 2 * p.stages * (int64_t)sizeof(uint64_t);
+        // the last CTA of a panel reuses the ring for Gv/Gu, the slice sums and the panel's new rows
+        const int64_t share = (q.panel_w + q.chunks - 1) / q.chunks * k;
+        const int64_t tail = (int64_t)sizeof(double) * (128 + 8 * (int64_t)k * k + 3 * share);
+        q.tail_smem = k <= 10 ? std::max(q.ring_smem, tail) : q.ring_smem;
+    };
+    auto plan_passes = [&]() {             // true when both rings fit
+        plan(m_local, n, p.pass1);
+        plan(n, m_local, p.pass2);
+        return std::max(p.pass1.ring_smem, p.pass2.ring_smem) <= 220 * 1024;
+    };
+    // the default ring fits at every k <= 128 (tests/test_xstream_exact.py, tests/test_f32_storage.py); an override is
+    // kept where its ring fits as well, and the default runs elsewhere.  fp32 tiles: twice the stages, the same bytes of
+    // X in flight.
+    const int64_t default_stages = (p.fg >= 4 ? 6 : p.fg == 2 ? 4 : 3) * (x32 ? 2 : 1);
+    p.stages = stages_override >= 2 && stages_override <= 12 ? stages_override : default_stages;
+    if (!plan_passes()) {
+        p.stages = default_stages;
+        plan_passes();
+    }
+    if (x_dtype == PRMF_X_TF32) {
+        plan_tc(sm_count, m_local, n, &p.tc_tiles1, &p.tc_chunks1, &p.tc_cols_per_chunk1);
+        plan_tc(sm_count, n, m_local, &p.tc_tiles2, &p.tc_chunks2, &p.tc_cols_per_chunk2);
+        const int64_t stage = (int64_t)kTcTileRows * kTcBlockK * 4 + round_up(k, 16) * kTcBlockK * 4;
+        p.tc_stages = std::max<int64_t>(2, std::min<int64_t>(8, (108 * 1024) / stage));      // two CTAs per SM
+        p.tc_smem = p.tc_stages * stage + (2 * p.tc_stages + 1) * (int64_t)sizeof(uint64_t) + 16 + 1024;
+    }
+    *out = p;
+    return PRMF_OK;
+}
+
 int prmf_create(prmf_handle** out, int device, int64_t m_local, int64_t m_global, int64_t n, int k, void* stream) {
     return prmf_create_ex(out, device, m_local, m_global, n, k, stream, PRMF_X_F64);
 }
@@ -1431,68 +1474,23 @@ int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_glo
     }
     h->x32 = x_dtype != PRMF_X_F64;
     h->x_tc = x_dtype == PRMF_X_TF32;
-    // X-stream plan: one CTA per SM, column panels of at most 1024 / FG columns, row chunks of at least 4 stages.  The
-    // panels and chunks do not depend on the storage type, which is what makes an fp32 handle bitwise equal to an fp64
-    // handle on the widened matrix; only the ring differs (an fp32 stage holds half the bytes of X).
-    if (k > 10) {                          // general-k kernel: FG factor groups x KT factors per thread
-        const int groups = (k + 15) / 16;
-        h->tma_fg = groups <= 1 ? 1 : groups <= 2 ? 2 : groups <= 4 ? 4 : 8;
-        const int per = (k + h->tma_fg - 1) / h->tma_fg;
-        h->tma_kt = per <= 8 ? 8 : per <= 12 ? 12 : 16;
-    }
     {
-        const int64_t max_panel = 1024 / h->tma_fg;
-        auto plan = [&](int64_t cols, int64_t rows, int* panels, int* panel_w, int* chunks, int64_t* rpc, size_t* smem) {
-            *panels = (int)std::max<int64_t>(1, (cols + max_panel - 1) / max_panel);
-            *panel_w = (int)round_up((std::max<int64_t>(1, cols) + *panels - 1) / *panels, 4);
-            *chunks = std::max(1, h->sm_count / *panels);
-            *chunks = (int)std::min<int64_t>(*chunks, std::max<int64_t>(1, rows / (4 * kTmaRS)));
-            // rows per chunk: even (the W rows of a chunk must start 16-byte aligned for the bulk copies), not a multiple
-            // of the stage height -- a ragged last stage costs less than a last chunk that is nearly empty
-            *rpc = round_up(std::max<int64_t>(1, (rows + *chunks - 1) / *chunks), 2);
-            const size_t xb = (size_t)kTmaRS * *panel_w * (h->x32 ? 4 : 8);
-            const size_t wb = (((size_t)kTmaRS * k + 16) * 8 + 127) & ~(size_t)127;
-            *smem = h->tma_stages * (xb + wb) + 2 * h->tma_stages * sizeof(uint64_t);
-        };
-        auto plan_passes = [&]() {         // true when both rings fit
-            plan(m_local, n, &h->panels1, &h->panel_w1, &h->chunks1, &h->rows_per_chunk1, &h->tma_smem1);
-            plan(n, m_local, &h->panels, &h->panel_w, &h->chunks, &h->rows_per_chunk, &h->tma_smem2);
-            return std::max(h->tma_smem1, h->tma_smem2) <= 220 * 1024;
-        };
-        // the default ring fits at every k <= 128 (tests/test_xstream_exact.py, tests/test_f32_storage.py); a
-        // PRMF_TMA_STAGES override is kept where its ring fits as well, and the handle runs the default elsewhere.  fp32
-        // tiles: twice the stages, the same bytes of X in flight.
-        const int default_stages = (h->tma_fg >= 4 ? 6 : h->tma_fg == 2 ? 4 : 3) * (h->x32 ? 2 : 1);
         const char* es = getenv("PRMF_TMA_STAGES");
-        const int want = es ? atoi(es) : 0;
-        h->tma_stages = want >= 2 && want <= 12 ? want : default_stages;
-        if (!plan_passes()) {
-            h->tma_stages = default_stages;
-            plan_passes();
-        }
+        prmf_plan_xstream(m_local, n, k, x_dtype, h->sm_count, es ? atoi(es) : 0, &h->plan);   // arguments checked above
     }
-
-    if (h->x_tc) setup_tf32(h);
-    if (h->x32 && !h->x_tc) {
+    const prmf_xstream_pass &p1 = h->plan.pass1, &p2 = h->plan.pass2;
+    if (h->x32) {
         h->ldx32 = round_up(n, 32);
         h->ldxt32 = round_up(std::max<int64_t>(1, m_local), 32);
     }
+    if (h->x_tc) setup_tf32(h);
     {
         const char* ee = getenv("PRMF_EPI");
         h->use_epi = !(ee && atoi(ee) == 0) && k <= 10 && m_local > 0 && !h->x_tc &&
-                     h->panels1 * h->chunks1 <= h->sm_count && h->panels * h->chunks <= h->sm_count;
-        if (h->use_epi) {
-            // the last CTA of a panel reuses the ring for Gv/Gu, the slice sums and the panel's new rows
-            const size_t share1 = (size_t)(h->panel_w1 + h->chunks1 - 1) / h->chunks1 * k;
-            const size_t share2 = (size_t)(h->panel_w + h->chunks - 1) / h->chunks * k;
-            const size_t need1 = sizeof(double) * (128 + 8 * (size_t)k * k + 3 * share1);
-            const size_t need2 = sizeof(double) * (128 + 8 * (size_t)k * k + 3 * share2);
-            h->tma_smem1 = std::max(h->tma_smem1, need1);
-            h->tma_smem2 = std::max(h->tma_smem2, need2);
-        }
+                     p1.panels * p1.chunks <= h->sm_count && p2.panels * p2.chunks <= h->sm_count;
     }
-    const int gu_parts_max = std::max(h->uu_grid, h->use_epi ? h->panels1 : 0);
-    const int gv_parts_max = std::max(h->vu_grid, h->use_epi ? h->panels : 0);
+    const int gu_parts_max = (int)std::max<int64_t>(h->uu_grid, h->use_epi ? p1.panels : 0);
+    const int gv_parts_max = (int)std::max<int64_t>(h->vu_grid, h->use_epi ? p2.panels : 0);
 
     int rc = 0;
     const int64_t nk = n * k;
@@ -1508,10 +1506,10 @@ int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_glo
         total += 2 * pad((size_t)(n + pad_rows) * k, d) + pad((size_t)nk, d);                      // Vbuf[2], Vb
         total += pad(128, d) + 4 * pad(kk2, d) + pad((size_t)gu_parts_max * kk2, d) + pad((size_t)gv_parts_max * kk2, d);
         total += pad(gv_parts_max, d) + pad((size_t)b_chunks(h) * nk, d);                           // VB_part, Bpart
-        total += pad(2 * ((size_t)h->panels1 + h->panels) + 2, sizeof(unsigned long long));     // fused-tail counters
-        total += pad(2 * ((size_t)h->panels1 + h->panels) + 4, sizeof(unsigned long long)) + pad(1, sizeof(unsigned int));   // block kernel
-        total += pad((size_t)std::max(h->panels1 * h->chunks1, h->panels * h->chunks) * kk2, d) +
-                 pad((size_t)h->panels * h->chunks, d);                                          // per-CTA partials
+        total += pad(2 * ((size_t)p1.panels + p2.panels) + 2, sizeof(unsigned long long));     // fused-tail counters
+        total += pad(2 * ((size_t)p1.panels + p2.panels) + 4, sizeof(unsigned long long)) + pad(1, sizeof(unsigned int));   // block kernel
+        total += pad((size_t)std::max(p1.panels * p1.chunks, p2.panels * p2.chunks) * kk2, d) +
+                 pad((size_t)p2.panels * p2.chunks, d);                                          // per-CTA partials
         total += pad((size_t)nk + kk2 + 2, d) + pad(1, d) + pad((size_t)h->sm_count * 8, d) + pad(2, d);
         total += pad(1, sizeof(int)) + pad(1, sizeof(unsigned int)) + pad(k, sizeof(int32_t)) + pad(nk, sizeof(int32_t));
         total += pad((size_t)h->obj_capacity * kObjStride, d);
@@ -1548,11 +1546,11 @@ int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_glo
     TAKE(h->Gu_part, double, (size_t)gu_parts_max * kk2);
     TAKE(h->Gv_part, double, (size_t)gv_parts_max * kk2);
     TAKE(h->VB_part, double, gv_parts_max);
-    TAKE(h->epi_counters, unsigned long long, 2 * ((size_t)h->panels1 + h->panels) + 2);
-    TAKE(h->blk_ctr, unsigned long long, 2 * ((size_t)h->panels1 + h->panels) + 4);
+    TAKE(h->epi_counters, unsigned long long, 2 * ((size_t)p1.panels + p2.panels) + 2);
+    TAKE(h->blk_ctr, unsigned long long, 2 * ((size_t)p1.panels + p2.panels) + 4);
     TAKE(h->err_word, unsigned int, 1);
-    TAKE(h->epi_part2, double, (size_t)std::max(h->panels1 * h->chunks1, h->panels * h->chunks) * kk2);
-    TAKE(h->epi_vb2, double, (size_t)h->panels * h->chunks);
+    TAKE(h->epi_part2, double, (size_t)std::max(p1.panels * p1.chunks, p2.panels * p2.chunks) * kk2);
+    TAKE(h->epi_vb2, double, (size_t)p2.panels * p2.chunks);
     TAKE(h->Bpart, double, (size_t)b_chunks(h) * nk);
     TAKE(h->red, double, (size_t)nk + kk2 + 2);
     TAKE(h->normX_sq, double, 1);
@@ -1574,8 +1572,8 @@ int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_glo
     if (!rc) {
         if (h->Xt) cudaMemsetAsync(h->Xt, 0, sizeof(double) * n * h->ldxt, h->stream);
         cudaMemsetAsync(h->ticket, 0, sizeof(unsigned int), h->stream);
-        cudaMemsetAsync(h->epi_counters, 0, sizeof(unsigned long long) * (2 * ((size_t)h->panels1 + h->panels) + 2), h->stream);
-        cudaMemsetAsync(h->blk_ctr, 0, sizeof(unsigned long long) * (2 * ((size_t)h->panels1 + h->panels) + 4), h->stream);
+        cudaMemsetAsync(h->epi_counters, 0, sizeof(unsigned long long) * (2 * ((size_t)p1.panels + p2.panels) + 2), h->stream);
+        cudaMemsetAsync(h->blk_ctr, 0, sizeof(unsigned long long) * (2 * ((size_t)p1.panels + p2.panels) + 4), h->stream);
         cudaMemsetAsync(h->err_word, 0, sizeof(unsigned int), h->stream);
         cudaMemsetAsync(h->U, 0, sizeof(double) * (m_local + pad_rows) * k, h->stream);
         cudaMemsetAsync(h->U2, 0, sizeof(double) * (m_local + pad_rows) * k, h->stream);
@@ -1590,7 +1588,7 @@ int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_glo
         const char* ed = getenv("PRMF_DEFER_OBJ");
         if (!(ed && atoi(ed) == 0)) {
             const size_t H = (size_t)h->obj_capacity, kk2s = (size_t)kk2;
-            const size_t n_gu = H * kk2s, n_gvp = H * h->panels * kk2s, n_vbp = H * h->panels, n_vh = H * kVhCap;
+            const size_t n_gu = H * kk2s, n_gvp = H * p2.panels * kk2s, n_vbp = H * p2.panels, n_vh = H * kVhCap;
             h->hist_bytes = sizeof(double) * (n_gu + n_gvp + n_vbp + n_vh);
             if (g_pool.alloc((void**)&h->hist, h->hist_bytes, device) == cudaSuccess) {
                 h->hist_Gu = h->hist;
@@ -1608,8 +1606,8 @@ int prmf_create_ex(prmf_handle** out, int device, int64_t m_local, int64_t m_glo
         const char* et = getenv("PRMF_SPIN_TIMEOUT_MS");
         if (et && atof(et) > 0) h->spin_timeout_ns = (unsigned long long)(atof(et) * 1e6);
         const size_t wb = ((size_t)kBlkRS * k * 8 + 127) & ~(size_t)127;
-        h->blk_stage_bytes = (uint32_t)((size_t)kBlkRS * std::max(h->panel_w1, h->panel_w) * 8 + wb);
-        h->blk_smem = (size_t)h->tma_stages * h->blk_stage_bytes + 2 * h->tma_stages * sizeof(uint64_t) +
+        h->blk_stage_bytes = (uint32_t)((size_t)kBlkRS * std::max(p1.panel_w, p2.panel_w) * 8 + wb);
+        h->blk_smem = (size_t)h->plan.stages * h->blk_stage_bytes + 2 * h->plan.stages * sizeof(uint64_t) +
                       sizeof(double) * (256 + 8 * (size_t)k * k + (size_t)kBlkRowsCap * k);
         // (block_kernel streams fp64 X: not for fp32 storage, where PRMF_BLOCK=1 is ignored)
         h->use_block = h->use_epi && h->defer_ok && !h->x32 && !(eb && atoi(eb) == 0) && h->blk_smem <= 227 * 1024;
@@ -2112,7 +2110,8 @@ int prmf_p2p_finalize(prmf_handle* h) {
     // The persistent step kernel is used only if EVERY rank can take it (ranks that disagreed would wait on flags
     // nobody writes), and its push exchange pairs CTA c of every rank, so all ranks must split the genes the same
     // way: [persistent step kernel possible | pass-2 chunks | chunks^2], summed over ranks
-    const double mine[3] = {h->use_block ? 1.0 : 0.0, (double)h->chunks, (double)h->chunks * h->chunks};
+    const double chunks = (double)h->plan.pass2.chunks;
+    const double mine[3] = {h->use_block ? 1.0 : 0.0, chunks, chunks * chunks};
     CU(cudaMemcpyAsync(h->scal_part, mine, sizeof mine, cudaMemcpyHostToDevice, h->stream));
     int rc = allreduce(h, h->scal_part, 3);
     if (rc) return rc;

@@ -62,6 +62,17 @@ def check_run_against_golden(g, U, V, od, trace, rtol_obj=1e-9, rtol_uv=1e-7):
         np.testing.assert_allclose(od[key], meta["final"][key], rtol=1e-8)
 
 
+def xstream_plan(m, n, k, x_dtype="f64", stages=0, sm_count=148):
+    """The launch plan libprmf_b200 gives the two X-stream passes of an m x n handle with k factors on a device with
+    `sm_count` SMs (prmf_plan_xstream, no GPU needed).  `stages`: the PRMF_TMA_STAGES override, 0 for none."""
+    import ctypes
+    from prmf_b200 import _lib
+    plan = _lib.XstreamPlan()
+    rc = _lib.load().prmf_plan_xstream(m, n, k, _lib.X_DTYPES[x_dtype], sm_count, stages, ctypes.byref(plan))
+    assert rc == 0, "prmf_plan_xstream returned %d" % rc
+    return plan
+
+
 def tf32_round(a):
     """Host model of `cvt.rna.tf32.f32` applied to float(a): round to nearest (ties away from zero) to a
     10-bit mantissa.  Returns float64 values that are exactly representable in tf32."""

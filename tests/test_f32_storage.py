@@ -14,34 +14,23 @@ import numpy as np
 import pytest
 
 from conftest import load_golden
-from helpers import run_product
+from helpers import run_product, xstream_plan
 from test_sass import _longest_dfma_region, _sass_by_function
 from test_xstream_exact import (K_GEN, K_SKINNY, RING_LIMIT, RS, SHAPES, _instance, _run_products, b200,  # noqa: F401
-                                default_stages, gen_fg_kt, host_wb)
+                                fg_kt)
 
 K_EQ = list(range(1, 11)) + [11, 17, 25, 64, 128]
 EQ_SHAPES = [(1, 1), (37, 131), (300, 257), (1025, 1000), (3, 4100), (993, 520), (2049, 33)]
 
 
 # ---- CPU: the ring plan ---------------------------------------------------------------------------------------
-def f32_default_stages(fg):
-    """Ring stages of an f32 handle without PRMF_TMA_STAGES (prmf_create_ex): twice the fp64 count."""
-    return 2 * default_stages(fg)
-
-
-def ring_bytes(panel_w, k, stages, elem):
-    """Shared memory of a ring of `stages` stages (X rows of `elem` bytes + the W slot + 2 mbarriers per stage)."""
-    return stages * (RS * panel_w * elem + host_wb(k)) + 2 * stages * 8
-
-
 def test_f32_default_ring_fits_and_keeps_the_fp64_bytes_in_flight():
     for k in range(1, 129):
-        fg = gen_fg_kt(k)[0] if k > 10 else 1
-        panel_w = 1024 // fg                                             # the widest panel
-        s32, s64 = f32_default_stages(fg), default_stages(fg)
-        assert s32 <= 12, k                                              # inside the PRMF_TMA_STAGES range
-        assert ring_bytes(panel_w, k, s32, 4) <= RING_LIMIT, k
-        assert s32 * RS * panel_w * 4 >= s64 * RS * panel_w * 8, k       # bytes of X in flight
+        p32, p64 = xstream_plan(1024, 1024, k, x_dtype="f32"), xstream_plan(1024, 1024, k)   # the widest panels
+        panel_w = p32.pass2.panel_w
+        assert p32.stages <= 12, k                                       # inside the PRMF_TMA_STAGES range
+        assert max(p32.pass1.ring_smem, p32.pass2.ring_smem) <= RING_LIMIT, k
+        assert p32.stages * RS * panel_w * 4 >= p64.stages * RS * panel_w * 8, k       # bytes of X in flight
 
 
 # ---- CPU: the shipped SASS ------------------------------------------------------------------------------------
@@ -58,7 +47,7 @@ def test_f32_stream_kernels_sass():
             loop = ops[a:b + 1]
             assert sum(op.startswith("DFMA") for op in loop) >= 8 * 4 * k, pattern
             assert not any(op.startswith(("LDL", "STL")) for op in loop), pattern
-    gen = {(kt, fg) for fg, kt in (gen_fg_kt(k) for k in range(11, 129))}
+    gen = {(kt, fg) for fg, kt in (fg_kt(k) for k in range(11, 129))}
     for kt, fg in gen:
         pattern = "skinny_tma_gen_f32_kernelILi%dELi%dELi8E" % (kt, fg)
         names = [n for n in funcs if pattern in n]

@@ -5,13 +5,15 @@ X, U and V hold small nonzero integers (uniform on 1..7).  Every product and par
 one dropped or repeated term moves an entry by at least 1.  The same holds in tf32 mode: integers below 2^11 are exact
 in tf32, and the fp32 accumulation of a chunk stays exact while its partial sums stay below 2^24.
 
-The first half restates the launch planner of `prmf_create_ex` on the host and checks, without a GPU, that the shape
-table below reaches the edges where a stream kernel can go wrong (empty chunks, ragged stages, narrow last panels,
-idle factor groups) and that no kernel reads W outside its shared-memory slot.  The GPU tests then run every kernel
-instantiation over that table and compare bitwise.
+The first half asks the library's launch planner (`prmf_plan_xstream`, the one `prmf_create_ex` runs) for the plan of
+every handle in the shape table below and checks, without a GPU, that the table reaches the edges where a stream kernel
+can go wrong (empty chunks, ragged stages, narrow last panels, idle factor groups) and that no kernel reads W outside its
+shared-memory slot.  The GPU tests then run every kernel instantiation over that table and compare bitwise.
 """
 import numpy as np
 import pytest
+
+from helpers import xstream_plan
 
 B200_SMS = 148          # the table proves its regimes for this SM count only
 RS = 8                  # stage height (rows) of the TMA kernels, kTmaRS in kernels.cuh
@@ -34,35 +36,11 @@ SWITCH_CASES = [
 SWITCH_IDS = ["stages2", "stages12", "stages12_fallback_skinny", "stages12_fallback_gen"]
 
 
-# ---- host restatement of the planner (prmf_b200/csrc/prmf_b200.cu) --------------------------------------------
-def round_up(a, b):
-    return (a + b - 1) // b * b
-
-
-def gen_fg_kt(k):
-    """(FG, KT) of the general-k kernel, prmf_b200.cu:1321-1326."""
-    groups = (k + 15) // 16
-    fg = 1 if groups <= 1 else 2 if groups <= 2 else 4 if groups <= 4 else 8
-    per = (k + fg - 1) // fg
-    return fg, 8 if per <= 8 else 12 if per <= 12 else 16
-
-
-def default_stages(fg):
-    """Ring stages of a handle without PRMF_TMA_STAGES, prmf_b200.cu:1348."""
-    return 6 if fg >= 4 else 4 if fg == 2 else 3
-
-
-def tma_config(m, n, k, env=None):
-    """(fg, kt, stages) as prmf_create_ex sets them for an m x n handle, prmf_b200.cu:1320-1356: a PRMF_TMA_STAGES
-    override (2..12) holds when the rings of both passes fit RING_LIMIT; otherwise the handle keeps the default."""
-    env = env or {}
-    fg, kt = gen_fg_kt(k) if k > 10 else (1, 0)
-    e3 = env.get("PRMF_TMA_STAGES")
-    if e3 is not None and 2 <= int(e3) <= 12:
-        want = int(e3)
-        if max(tma_plan(m, n, k, fg, want)["smem"], tma_plan(n, m, k, fg, want)["smem"]) <= RING_LIMIT:
-            return fg, kt, want
-    return fg, kt, default_stages(fg)
+# ---- the plan, and what the general-k kernel reads ---------------------------------------------------------------
+def fg_kt(k):
+    """(FG, KT) of the general-k kernel a handle with k > 10 factors runs."""
+    plan = xstream_plan(1, 1, k)
+    return plan.fg, plan.kt
 
 
 def w_slot_bytes(k, kt):
@@ -70,35 +48,18 @@ def w_slot_bytes(k, kt):
     return ((RS * k + kt) * 8 + 127) & ~127
 
 
-def host_wb(k):
-    """Bytes the host reserves per stage for W, the `wb` of the plan lambda, prmf_b200.cu:1338."""
-    return ((RS * k + 16) * 8 + 127) & ~127
-
-
-def tma_plan(cols, rows, k, fg, stages, sm_count=B200_SMS):
-    """The `plan` lambda of prmf_create_ex, prmf_b200.cu:1328-1340."""
-    max_panel = 1024 // fg
-    panels = max(1, -(-cols // max_panel))
-    panel_w = round_up(-(-max(1, cols) // panels), 4)
-    chunks = max(1, sm_count // panels)
-    chunks = min(chunks, max(1, rows // (4 * RS)))
-    rpc = round_up(max(1, -(-rows // chunks)), 2)
-    smem = stages * (RS * panel_w * 8 + host_wb(k)) + 2 * stages * 8
-    return dict(panels=panels, panel_w=panel_w, chunks=chunks, rpc=rpc, smem=smem, max_panel=max_panel)
-
-
 def kernel_of(k):
-    """Name of the X-stream kernel an fp64 handle with k factors runs (prmf_b200.cu:416-454)."""
+    """Name of the X-stream kernel an fp64 handle with k factors runs."""
     if k > 10:
-        return "skinny_tma_gen_kernel<%d,%d>" % gen_fg_kt(k)[::-1]
+        return "skinny_tma_gen_kernel<%d,%d>" % fg_kt(k)[::-1]
     return "skinny_tma_kernel<%d,%d,0>" % (k, RS)
 
 
-def pass_regimes(cols, rows, p):
+def pass_regimes(cols, rows, p, fg):
     """The edges one pass meets: the row chunks and column panels of its launch, as the kernels see them."""
     out = set()
-    out.add("one panel" if p["panels"] == 1 else "several panels")
-    if cols - (p["panels"] - 1) * p["panel_w"] < p["panel_w"]:     # the rest of its width is zero pad columns
+    out.add("one panel" if p.panels == 1 else "several panels")
+    if cols - (p.panels - 1) * p.panel_w < p.panel_w:             # the rest of its width is zero pad columns
         out.add("narrow last panel")
     if cols % 4:
         out.add("cols % 4 != 0")
@@ -108,24 +69,23 @@ def pass_regimes(cols, rows, p):
         out.add("rows == 1")
     if rows < RS:
         out.add("rows < RS")
-    if p["chunks"] == 1:
+    if p.chunks == 1:
         out.add("one chunk")
-    for c in range(p["chunks"]):
-        beg, end = c * p["rpc"], min(rows, (c + 1) * p["rpc"])
+    for c in range(p.chunks):
+        beg, end = c * p.rows_per_chunk, min(rows, (c + 1) * p.rows_per_chunk)
         if end <= beg:
             out.add("empty chunk")
         elif (end - beg) % RS:
             out.add("ragged last stage")
-    if p["panels"] > 1:
-        out.add("panel limit %d" % p["max_panel"])
+    if p.panels > 1:
+        out.add("several panels at FG %d" % fg)
     return out
 
 
-def regimes(m, n, k, env=None):
+def regimes(m, n, k):
     """{"pass 1": set, "pass 2": set} for an fp64 TMA handle."""
-    fg, kt, stages = tma_config(m, n, k, env)
-    return {"pass 1": pass_regimes(m, n, tma_plan(m, n, k, fg, stages)),
-            "pass 2": pass_regimes(n, m, tma_plan(n, m, k, fg, stages))}
+    plan = xstream_plan(m, n, k)
+    return {"pass 1": pass_regimes(m, n, plan.pass1, plan.fg), "pass 2": pass_regimes(n, m, plan.pass2, plan.fg)}
 
 
 def max_w_index(k, fg, kt, clamped=True):
@@ -134,17 +94,6 @@ def max_w_index(k, fg, kt, clamped=True):
     (kernels.cuh, `fr`).  `clamped=False` models a loop in which every group reads its own columns."""
     first = [g * kt if (g * kt < k or not clamped) else 0 for g in range(fg)]
     return max(first) + (RS - 1) * k + kt - 1
-
-
-def plan_tc(R, C, sm_count=B200_SMS):
-    """Column chunks of the tf32 tensor-core passes, prmf_b200.cu:1104-1120."""
-    tiles = max(1, -(-R // 128))
-    max_chunks = max(1, min(64, C // 512))
-    eff = [0.0] + [tiles * c / (np.ceil(tiles * c / (2.0 * sm_count)) * 2.0 * sm_count) for c in range(1, max_chunks + 1)]
-    best = max(eff)
-    pick = next(c for c in range(1, max_chunks + 1) if eff[c] >= best - 0.03)
-    cpc = round_up(max(1, -(-C // pick)), 32)
-    return max(1, -(-C // cpc))
 
 
 # ---- CPU checks of the table ----------------------------------------------------------------------------------
@@ -158,7 +107,7 @@ def test_shape_table_covers_the_launch_plan_edges():
         for m, n in SHAPES:
             for k in K_SKINNY + K_GEN:
                 seen |= regimes(m, n, k)[pas]
-        missing = [r for r in REQUIRED + ["panel limit %d" % (1024 // fg) for fg in (1, 2, 4, 8)] if r not in seen]
+        missing = [r for r in REQUIRED + ["several panels at FG %d" % fg for fg in (1, 2, 4, 8)] if r not in seen]
         assert not missing, "%s never meets %s" % (pas, missing)
 
 
@@ -171,7 +120,7 @@ def test_every_instantiation_meets_an_empty_chunk_a_ragged_stage_and_a_narrow_pa
             for pas in d:
                 d[pas] |= r[pas]
     want = {"skinny_tma_kernel<%d,8,0>" % k for k in K_SKINNY} | \
-           {"skinny_tma_gen_kernel<%d,%d>" % (kt, fg) for fg, kt in {gen_fg_kt(k) for k in range(11, 129)}}
+           {"skinny_tma_gen_kernel<%d,%d>" % (kt, fg) for fg, kt in {fg_kt(k) for k in range(11, 129)}}
     assert set(by_kernel) == want
     for name, d in sorted(by_kernel.items()):
         for pas, seen in d.items():
@@ -182,90 +131,88 @@ def test_every_instantiation_meets_an_empty_chunk_a_ragged_stage_and_a_narrow_pa
 def test_general_k_choices_reach_idle_and_ragged_factor_groups():
     """K_GEN holds a ragged last group (k = 25: 16 + 9), wholly idle groups (k = 66, 98: the worst W over-reads
     of the unclamped loop) and the FG = 4 idle group (k = 33)."""
-    assert gen_fg_kt(25) == (2, 16) and 25 % 16
-    assert gen_fg_kt(33) == (4, 12) and 3 * 12 >= 33
-    assert gen_fg_kt(66) == (8, 12) and sum(g * 12 >= 66 for g in range(8)) == 2
-    assert gen_fg_kt(98) == (8, 16) and 7 * 16 >= 98
+    assert fg_kt(25) == (2, 16) and 25 % 16
+    assert fg_kt(33) == (4, 12) and 3 * 12 >= 33
+    assert fg_kt(66) == (8, 12) and sum(g * 12 >= 66 for g in range(8)) == 2
+    assert fg_kt(98) == (8, 16) and 7 * 16 >= 98
     # every (FG, KT) that k = 11..128 can select; the KT = 8 instantiations are compiled but unreachable
-    assert {gen_fg_kt(k) for k in range(11, 129)} == {(1, 12), (1, 16), (2, 12), (2, 16), (4, 12), (4, 16), (8, 12),
-                                                     (8, 16)}
+    assert {fg_kt(k) for k in range(11, 129)} == {(1, 12), (1, 16), (2, 12), (2, 16), (4, 12), (4, 16), (8, 12), (8, 16)}
 
 
 @pytest.mark.parametrize("k", range(11, 129))
 def test_general_k_kernel_reads_w_inside_its_slot(k):
-    """The largest W index read lies inside the W slot for every stage count that fits, and the kernel's stage
-    layout (x rows + w_slot, then 2 mbarriers per stage) lies inside the shared memory the host requests."""
-    fg, kt = gen_fg_kt(k)
+    """The largest W index read lies inside the W slot, and the kernel's stage layout (x rows + w_slot, then 2
+    mbarriers per stage) lies inside the ring the host sizes, for every PRMF_TMA_STAGES a handle can be given, at the
+    narrowest panel (n = 1: 4 columns) and the widest (n = 1024: 1024 / FG columns)."""
+    fg, kt = fg_kt(k)
     slot = w_slot_bytes(k, kt) // 8
-    assert w_slot_bytes(k, kt) <= host_wb(k)
     assert max_w_index(k, fg, kt) <= RS * k + kt - 2 < slot
     for stages in range(2, 13):
-        for panel_w in (4, 1024 // fg):
-            smem = stages * (RS * panel_w * 8 + host_wb(k)) + 2 * stages * 8
-            if smem > RING_LIMIT:
-                continue
-            kernel_end = stages * (RS * panel_w * 8 + w_slot_bytes(k, kt)) + 2 * stages * 8
-            assert kernel_end <= smem
+        for n in (1, 1024):
+            plan = xstream_plan(1, n, k, stages=stages)
+            p = plan.pass2
+            kernel_end = plan.stages * (RS * p.panel_w * 8 + w_slot_bytes(k, kt)) + 2 * plan.stages * 8
+            assert kernel_end <= p.ring_smem
 
 
 def test_w_slot_check_flags_the_unclamped_loop():
     """If every group read its own columns, the last row of the last stage would read past the W slot at k = 66 and 98
     and, at the default 6 stages, 16 bytes past the end of the shared memory the host requests."""
     for k in (66, 98):
-        fg, kt = gen_fg_kt(k)
-        stages = tma_config(1000, 6750, k)[2]
+        fg, kt = fg_kt(k)
+        plan = xstream_plan(1000, 6750, k)
+        p = plan.pass2                                           # 6750 genes: panels of the widest width, 128 columns
         last = max_w_index(k, fg, kt, clamped=False)
         assert last >= w_slot_bytes(k, kt) // 8
-        x_stage = RS * (1024 // fg) * 8
-        smem = stages * (x_stage + host_wb(k)) + 2 * stages * 8
-        end_of_read = (stages - 1) * (x_stage + w_slot_bytes(k, kt)) + x_stage + (last + 1) * 8
-        assert end_of_read - smem == 16
-    bad = [k for k in range(11, 129) if max_w_index(k, *gen_fg_kt(k), clamped=False) >= w_slot_bytes(k, gen_fg_kt(k)[1]) // 8]
+        x_stage = RS * p.panel_w * 8
+        end_of_read = (plan.stages - 1) * (x_stage + w_slot_bytes(k, kt)) + x_stage + (last + 1) * 8
+        assert end_of_read - p.ring_smem == 16
+    bad = [k for k in range(11, 129) if max_w_index(k, *fg_kt(k), clamped=False) >= w_slot_bytes(k, fg_kt(k)[1]) // 8]
     assert {66, 98} <= set(bad) <= set(range(65, 79)) | set(range(97, 111))
 
 
 def test_default_ring_fits_at_the_widest_panel():
     """An oversized PRMF_TMA_STAGES gives way to the default stage count, so the default ring must fit at every k."""
     for k in range(1, 129):
-        fg = gen_fg_kt(k)[0] if k > 10 else 1
-        assert tma_plan(1024 // fg, 1, k, fg, default_stages(fg))["smem"] <= RING_LIMIT, k
+        plan = xstream_plan(1024, 1024, k)                      # 1024 columns: panels of 1024 / FG columns
+        assert max(plan.pass1.ring_smem, plan.pass2.ring_smem) <= RING_LIMIT, k
 
 
 def test_switch_cases_reach_the_intended_kernels():
     for m, n in SHAPES:
         for k in K_SKINNY + K_GEN:
-            assert tma_config(m, n, k, {"PRMF_TMA_STAGES": "2"})[2] == 2, (m, n, k)
-        assert tma_config(m, n, 97, {"PRMF_TMA_STAGES": "12"})[2] == 12, (m, n)
+            assert xstream_plan(m, n, k, stages=2).stages == 2, (m, n, k)
+        assert xstream_plan(m, n, 97, stages=12).stages == 12, (m, n)
     assert kernel_of(97) == "skinny_tma_gen_kernel<16,8>" and kernel_of(10) == "skinny_tma_kernel<10,8,0>"
     # at k = 10 and 25 a 12-stage ring fits narrow panels only: wider handles keep the default 3 / 4 stages
     for k, default in ((10, 3), (25, 4)):
-        stages = {(m, n): tma_config(m, n, k, {"PRMF_TMA_STAGES": "12"})[2] for m, n in SHAPES}
+        stages = {(m, n): xstream_plan(m, n, k, stages=12).stages for m, n in SHAPES}
         assert set(stages.values()) == {default, 12} and stages[(1000, 6750)] == default, k
     # PRMF_TMA_STAGES=2 wraps the mbarrier phase every two stages: some chunk of the table runs more than 2 stages
-    fg, kt, stages = tma_config(1000, 6750, 66, {"PRMF_TMA_STAGES": "2"})
-    p = tma_plan(6750, 1000, 66, fg, stages)
-    assert stages == 2 and p["rpc"] > 4 * RS
+    plan = xstream_plan(1000, 6750, 66, stages=2)
+    assert plan.stages == 2 and plan.pass2.rows_per_chunk > 4 * RS
 
 
 def test_tf32_table_covers_the_tensor_core_edges():
     seen = set()
     for m, n in TF32_SHAPES:
-        for R, C in ((m, n), (n, m)):
+        plan = xstream_plan(m, n, 16, x_dtype="tf32")
+        for R, C, chunks in ((m, n, plan.tc_chunks1), (n, m, plan.tc_chunks2)):
             if R % 128:
                 seen.add("rows % 128 != 0")
             if C % 32:
                 seen.add("cols % 32 != 0")
             if C < 32:
                 seen.add("cols < 32")
-            if C >= 1024 and plan_tc(R, C) > 1:
+            if C >= 1024 and chunks > 1:
                 seen.add("several column chunks")
     assert seen == {"rows % 128 != 0", "cols % 32 != 0", "cols < 32", "several column chunks"}
-    kp = {round_up(k, 16) for k in K_TF32}
+    kp = {-(-k // 16) * 16 for k in K_TF32}
     assert min(kp) == 16 and max(kp) == 128
     tcols = set()
-    for k in K_TF32:
+    for k in kp:
         t = 32
-        while t < round_up(k, 16):
+        while t < k:
             t *= 2
         tcols.add(t)
     assert tcols == {32, 64, 128}
