@@ -1,7 +1,8 @@
 // libprmf_b200.so -- C ABI (include/prmf_b200.h) over the sm_100a kernels in kernels.cuh, block.cuh and tf32.cuh.
 // Host orchestration of one PRMF inner step (reference prmf_runner.py:419-449).  Both passes over X are TMA X-stream
 // launches: skinny_tma_kernel<k,kTmaRS,EPI> at k <= 10, skinny_tma_gen_kernel<KT,FG,kTmaRS> at k > 10 (their _f32_
-// twins when X is stored in fp32, PRMF_X_F32), or tc_rowdot_kernel in tf32 mode.
+// twins when X is stored in fp32, PRMF_X_F32), or tc_rowdot_kernel in tf32 mode.  step_path chooses which of the
+// sequences below a block of steps runs (StepPath).
 //
 // k <= 10, fp64 (fused tails, launch_xv_epi / launch_xtu_epi):
 //   skinny_tma_kernel<k,8,1>   A partials = Xt^T.V, then U <- U*A/(U.Gv+U) and Gu in the last CTA of each panel   (:420-422)
@@ -307,96 +308,94 @@ int set_smem(prmf_handle* h, F kernel, size_t bytes) {
     return PRMF_OK;
 }
 
-// ---- templated launch dispatch ---------------------------------------------------------------------
-// the X-stream kernel (k <= 10) for the storage type of M
-template <int KT, int EPI>
-auto tma_kernel(const double*) { return skinny_tma_kernel<KT, kTmaRS, EPI>; }
-template <int KT, int EPI>
-auto tma_kernel(const float*) { return skinny_tma_f32_kernel<KT, kTmaRS, EPI>; }
+// ---- X-stream launches -----------------------------------------------------------------------------
+// One pass over X: out[chunk][j][0:k] = sum over the rows i of the chunk of M[i][j] * W[i][0:k]
+struct XStream {
+    const void* M;                            // fp32 when f32, else fp64
+    bool f32;
+    int64_t ldm, rows, cols;
+    const double* W;
+    double* out;                              // per-chunk partials
+    const prmf_xstream_pass& p;
+};
+
+// pass 1: A partials = Xt^T . V   (M = Xt: n rows x m cols)
+XStream pass1(const prmf_handle* h) {
+    return {h->x32 ? (const void*)h->Xt32 : h->Xt, h->x32, h->x32 ? h->ldxt32 : h->ldxt, h->n, h->m, h->Vbuf[h->vcur],
+            h->Apart, h->plan.pass1};
+}
+
+// pass 2: B partials = X^T . U_new   (M = X: m rows x n cols)
+XStream pass2(const prmf_handle* h) {
+    return {h->x32 ? (const void*)h->X32 : h->X, h->x32, h->x32 ? h->ldx32 : h->ldx, h->m, h->n, h->U, h->Bpart,
+            h->plan.pass2};
+}
+
+// the k <= 10 kernel of a pass with fused tail `epi`: call with KT = 1, it recurses to KT = k
+template <int KT>
+const void* tma_kernel(int k, bool f32, int epi) {
+    if constexpr (KT < 10)
+        if (k != KT) return tma_kernel<KT + 1>(k, f32, epi);
+    switch (epi) {
+        case 0: return f32 ? (const void*)skinny_tma_f32_kernel<KT, kTmaRS, 0> : (const void*)skinny_tma_kernel<KT, kTmaRS, 0>;
+        case 1: return f32 ? (const void*)skinny_tma_f32_kernel<KT, kTmaRS, 1> : (const void*)skinny_tma_kernel<KT, kTmaRS, 1>;
+        case 2: return f32 ? (const void*)skinny_tma_f32_kernel<KT, kTmaRS, 2> : (const void*)skinny_tma_kernel<KT, kTmaRS, 2>;
+        // no pack on fp32 storage: the f32 mode is single-rank (prmf_p2p_attach), the tf32 mode uses tc_rowdot_kernel
+        case 3: return f32 ? nullptr : (const void*)skinny_tma_kernel<KT, kTmaRS, 3>;
+    }
+    return nullptr;
+}
+
+// the k > 10 kernel of a pass (no fused tail)
+const void* gen_kernel(const prmf_xstream_plan& plan, bool f32) {
+#define GEN_CASE(KT_, FG_)                                                                                   \
+    if (plan.kt == KT_ && plan.fg == FG_)                                                                    \
+        return f32 ? (const void*)skinny_tma_gen_f32_kernel<KT_, FG_, kTmaRS> : (const void*)skinny_tma_gen_kernel<KT_, FG_, kTmaRS>;
+    GEN_CASE(12, 1) GEN_CASE(16, 1) GEN_CASE(8, 2) GEN_CASE(12, 2) GEN_CASE(16, 2) GEN_CASE(8, 4) GEN_CASE(12, 4)
+    GEN_CASE(16, 4) GEN_CASE(8, 8) GEN_CASE(12, 8) GEN_CASE(16, 8)
+#undef GEN_CASE
+    return nullptr;
+}
 
 // every launch of a pass on a fused-tail handle requests the tail's shared memory
 size_t pass_smem(const prmf_handle* h, const prmf_xstream_pass& p) { return h->use_epi ? p.tail_smem : p.ring_smem; }
 
-template <int KT, typename T>
-int launch_skinny_tma_t(prmf_handle* h, const T* M, int64_t ldm, int64_t rows, int64_t cols, const double* W,
-                        const prmf_xstream_pass& p, double* out) {
-    dim3 grid(p.panels, p.chunks);
-    EpiParams none{};
-    none.dbg_slot = -1;
-    none.err = h->err_word; none.timeout_ns = h->spin_timeout_ns;
-    const auto fn = tma_kernel<KT, 0>(M);
-    const size_t smem = pass_smem(h, p);
-    CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    fn<<<grid, kTmaThreads, smem, h->stream>>>(M, ldm, rows, cols, W, p.panel_w, p.rows_per_chunk, h->plan.stages, out,
-                                               none);
-    return PRMF_OK;
+// EpiParams of an X-stream launch without a fused tail; the fused-tail launchers fill in the rest
+EpiParams plain_epi(const prmf_handle* h) {
+    EpiParams ep{};
+    ep.dbg_slot = -1;
+    ep.err = h->err_word; ep.timeout_ns = h->spin_timeout_ns;
+    return ep;
 }
 
-// X-stream kernel with a fused tail (EPI 1: U update, 2: V update, 3: pack for the exchange over ranks).  The CTAs
-// of a panel wait for each other, so the launch is cooperative (all CTAs co-resident or the launch fails).
-template <int KT, typename T>
-int launch_skinny_epi_t(prmf_handle* h, int epi, const T* M, int64_t ldm, int64_t rows, int64_t cols,
-                        const double* W, const prmf_xstream_pass& p, double* out, const EpiParams& ep_in) {
-    dim3 grid(p.panels, p.chunks);
-    EpiParams ep = ep_in;
-    int panel_w = (int)p.panel_w, stages = (int)h->plan.stages;     // the kernel's parameter types
-    const size_t smem = pass_smem(h, p);
-    void* args[] = {(void*)&M, (void*)&ldm, (void*)&rows, (void*)&cols, (void*)&W, (void*)&panel_w,
-                    (void*)&p.rows_per_chunk, (void*)&stages, (void*)&out, (void*)&ep};
+// Launches pass `x` with fused tail `epi` (0: none, 1: U update, 2: V update, 3: pack for the exchange over ranks).
+// The storage of M and k choose the kernel once: skinny_tma_kernel<k,kTmaRS,EPI> at k <= 10,
+// skinny_tma_gen_kernel<KT,FG,kTmaRS> (no fused tail) above, or their _f32_ twins.  The CTAs of a panel with a fused
+// tail wait for each other, so that launch is cooperative (all CTAs co-resident or the launch fails).
+int launch_xstream(prmf_handle* h, const XStream& x, int epi, const EpiParams& ep_in) {
+    const bool gen = h->k > 10;
     const void* fn = nullptr;
-    switch (epi) {
-        case 1: fn = (const void*)tma_kernel<KT, 1>(M); break;
-        case 2: fn = (const void*)tma_kernel<KT, 2>(M); break;
-        case 3: if constexpr (sizeof(T) == sizeof(double)) fn = (const void*)skinny_tma_kernel<KT, kTmaRS, 3>; break;
-    }
-    if (!fn) return fail(h, PRMF_ERR_STATE, "bad fused-tail id %d", epi);
-    CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    // always cooperative: the CTAs of a panel wait for each other, so co-residency must be guaranteed by the driver
-    CU(cudaLaunchCooperativeKernel(fn, grid, dim3(kTmaThreads), args, smem, h->stream));
-    return PRMF_OK;
-}
-
-template <int KT, int FG>
-auto gen_kernel(const double*) { return skinny_tma_gen_kernel<KT, FG, kTmaRS>; }
-template <int KT, int FG>
-auto gen_kernel(const float*) { return skinny_tma_gen_f32_kernel<KT, FG, kTmaRS>; }
-
-template <int KT, int FG, typename T>
-int launch_skinny_gen_t(prmf_handle* h, const T* M, int64_t ldm, int64_t rows, int64_t cols, const double* W,
-                        const prmf_xstream_pass& p, double* out) {
-    dim3 grid(p.panels, p.chunks);
-    const auto fn = gen_kernel<KT, FG>(M);
+    if (!gen) fn = tma_kernel<1>(h->k, x.f32, epi);
+    else if (epi == 0) fn = gen_kernel(h->plan, x.f32);
+    if (!fn)
+        return fail(h, PRMF_ERR_STATE, "no X-stream kernel for k=%d (KT=%d FG=%d), fused tail %d, %s storage", h->k,
+                    (int)h->plan.kt, (int)h->plan.fg, epi, x.f32 ? "fp32" : "fp64");
+    const prmf_xstream_pass& p = x.p;
+    EpiParams ep = ep_in;
+    int k = h->k, panel_w = (int)p.panel_w, stages = (int)h->plan.stages;     // the kernels' parameter types
+    void* tma_args[] = {(void*)&x.M, (void*)&x.ldm, (void*)&x.rows, (void*)&x.cols, (void*)&x.W, (void*)&panel_w,
+                        (void*)&p.rows_per_chunk, (void*)&stages, (void*)&x.out, (void*)&ep};
+    void* gen_args[] = {(void*)&x.M, (void*)&x.ldm, (void*)&x.rows, (void*)&x.cols, (void*)&x.W, (void*)&k,
+                        (void*)&panel_w, (void*)&p.rows_per_chunk, (void*)&stages, (void*)&x.out};
+    const dim3 grid(p.panels, p.chunks);
     const size_t smem = pass_smem(h, p);
     CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    fn<<<grid, kTmaThreads, smem, h->stream>>>(M, ldm, rows, cols, W, h->k, p.panel_w, p.rows_per_chunk, h->plan.stages,
-                                               out);
+    if (epi != 0)
+        CU(cudaLaunchCooperativeKernel(fn, grid, dim3(kTmaThreads), tma_args, smem, h->stream));
+    else   // as with <<<>>>, a failure is left for the caller's LAUNCH_CHECK
+        cudaLaunchKernel(fn, grid, dim3(kTmaThreads), gen ? gen_args : tma_args, smem, h->stream);
     return PRMF_OK;
 }
-
-template <typename T>
-int launch_skinny_gen(prmf_handle* h, const T* M, int64_t ldm, int64_t rows, int64_t cols, const double* W,
-                      const prmf_xstream_pass& p, double* out) {
-#define GEN_CASE(KT_, FG_) \
-    if (h->plan.kt == KT_ && h->plan.fg == FG_) return launch_skinny_gen_t<KT_, FG_>(h, M, ldm, rows, cols, W, p, out);
-    GEN_CASE(12, 1) GEN_CASE(16, 1) GEN_CASE(8, 2) GEN_CASE(12, 2) GEN_CASE(16, 2) GEN_CASE(8, 4) GEN_CASE(12, 4)
-    GEN_CASE(16, 4) GEN_CASE(8, 8) GEN_CASE(12, 8) GEN_CASE(16, 8)
-#undef GEN_CASE
-    return fail(h, PRMF_ERR_STATE, "no general-k kernel for KT=%d FG=%d", (int)h->plan.kt, (int)h->plan.fg);
-}
-
-#define KT_SWITCH_RC(kt, rc, FN, ...)          \
-    switch (kt) {                              \
-        case 1: rc = FN<1>(__VA_ARGS__); break;   \
-        case 2: rc = FN<2>(__VA_ARGS__); break;   \
-        case 3: rc = FN<3>(__VA_ARGS__); break;   \
-        case 4: rc = FN<4>(__VA_ARGS__); break;   \
-        case 5: rc = FN<5>(__VA_ARGS__); break;   \
-        case 6: rc = FN<6>(__VA_ARGS__); break;   \
-        case 7: rc = FN<7>(__VA_ARGS__); break;   \
-        case 8: rc = FN<8>(__VA_ARGS__); break;   \
-        case 9: rc = FN<9>(__VA_ARGS__); break;   \
-        default: rc = FN<10>(__VA_ARGS__); break; \
-    }
 
 // number of per-chunk partials the passes leave in Apart / Bpart
 int a_chunks(const prmf_handle* h) { return (int)(h->x_tc ? h->plan.tc_chunks1 : h->plan.pass1.chunks); }
@@ -420,29 +419,18 @@ int refresh_wt(prmf_handle* h, const double* W, int64_t rows, float* Wt, int64_t
     return PRMF_OK;
 }
 
-// pass 1: A partials = Xt^T . V   (M = Xt: n rows x m cols)
+// pass 1 without a fused tail
 int launch_xv(prmf_handle* h) {
     if (h->m == 0) return PRMF_OK;
     if (h->x_tc)
         return launch_tc(h, h->tm_X, h->tm_Vt, h->tc1, h->plan.tc_tiles1, h->plan.tc_chunks1, "tc_rowdot_kernel(pass 1)");
-    const prmf_xstream_pass& p = h->plan.pass1;
-    const double* V = h->Vbuf[h->vcur];
-    int rc = 0;
-    if (h->x32 && h->k > 10) {
-        rc = launch_skinny_gen(h, h->Xt32, h->ldxt32, h->n, h->m, V, p, h->Apart);
-    } else if (h->x32) {
-        KT_SWITCH_RC(h->k, rc, launch_skinny_tma_t, h, h->Xt32, h->ldxt32, h->n, h->m, V, p, h->Apart);
-    } else if (h->k > 10) {
-        rc = launch_skinny_gen(h, h->Xt, h->ldxt, h->n, h->m, V, p, h->Apart);
-    } else {
-        KT_SWITCH_RC(h->k, rc, launch_skinny_tma_t, h, h->Xt, h->ldxt, h->n, h->m, V, p, h->Apart);
-    }
+    int rc = launch_xstream(h, pass1(h), 0, plain_epi(h));
     if (rc) return rc;
     LAUNCH_CHECK("skinny_tma_kernel(pass 1)");
     return PRMF_OK;
 }
 
-// pass 2: B partials = X^T . U_new   (M = X: m rows x n cols)
+// pass 2 without a fused tail
 int launch_xtu(prmf_handle* h) {
     if (h->m == 0) {
         CU(cudaMemsetAsync(h->Bpart, 0, sizeof(double) * b_chunks(h) * h->n * h->k, h->stream));
@@ -453,17 +441,7 @@ int launch_xtu(prmf_handle* h) {
         if (rc) return rc;
         return launch_tc(h, h->tm_Xt, h->tm_Ut, h->tc2, h->plan.tc_tiles2, h->plan.tc_chunks2, "tc_rowdot_kernel(pass 2)");
     }
-    const prmf_xstream_pass& p = h->plan.pass2;
-    int rc = 0;
-    if (h->x32 && h->k > 10) {
-        rc = launch_skinny_gen(h, h->X32, h->ldx32, h->m, h->n, h->U, p, h->Bpart);
-    } else if (h->x32) {
-        KT_SWITCH_RC(h->k, rc, launch_skinny_tma_t, h, h->X32, h->ldx32, h->m, h->n, h->U, p, h->Bpart);
-    } else if (h->k > 10) {
-        rc = launch_skinny_gen(h, h->X, h->ldx, h->m, h->n, h->U, p, h->Bpart);
-    } else {
-        KT_SWITCH_RC(h->k, rc, launch_skinny_tma_t, h, h->X, h->ldx, h->m, h->n, h->U, p, h->Bpart);
-    }
+    int rc = launch_xstream(h, pass2(h), 0, plain_epi(h));
     if (rc) return rc;
     LAUNCH_CHECK("skinny_tma_kernel(pass 2)");
     return PRMF_OK;
@@ -670,9 +648,14 @@ int ensure_pos(prmf_handle* h) {
 }
 
 // ---- fused-tail path (use_epi): two X-stream launches per inner step do the U and V updates as well ----
+// Where a sharded step packs its [X^T U | U^T U] for the sum over ranks: this rank's peer-buffer slot of the step's
+// parity, which the V update pulls from every rank, or h->red for ncclAllReduce
+double* exchange_dst(const prmf_handle* h) {
+    return h->p2p_ready ? h->p2p_buf + (size_t)h->p2p_parity * h->p2p_red_count : h->red;
+}
+
 int launch_xv_epi(prmf_handle* h, const double* gv_src = nullptr, int gv_parts = 1) {
-    EpiParams ep{};
-    ep.err = h->err_word; ep.timeout_ns = h->spin_timeout_ns;
+    EpiParams ep = plain_epi(h);
     ep.arrive = h->epi_counters;
     ep.done = h->epi_counters + h->plan.pass1.panels + h->plan.pass2.panels;
     ep.seq = ++h->epi_seq1;
@@ -684,24 +667,16 @@ int launch_xv_epi(prmf_handle* h, const double* gv_src = nullptr, int gv_parts =
     ep.Gv = gv_src ? gv_src : h->Gv;
     ep.gv_parts = gv_src ? gv_parts : 1;
     ep.Gu_part = h->Gu_part;
-    int rc = 0;
-    if (h->x32) {
-        KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, 1, h->Xt32, h->ldxt32, h->n, h->m, h->Vbuf[h->vcur],
-                     h->plan.pass1, h->Apart, ep);
-    } else {
-        KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, 1, h->Xt, h->ldxt, h->n, h->m, h->Vbuf[h->vcur], h->plan.pass1,
-                     h->Apart, ep);
-    }
+    const int rc = launch_xstream(h, pass1(h), 1, ep);
     if (rc) { h->failed = true; return rc; }     // the panel counters expect this launch: no further steps on this handle
     LAUNCH_CHECK("skinny_tma_kernel(pass 1 + U update)");
     std::swap(h->U, h->U2);
     return PRMF_OK;
 }
 
-// mode 2: V update (one GPU); 3: pack into `packed_dst` for the sum over ranks (sharded)
-int launch_xtu_epi(prmf_handle* h, int mode, double* packed_dst, int hist_slot = -1) {
-    EpiParams ep{};
-    ep.err = h->err_word; ep.timeout_ns = h->spin_timeout_ns;
+// mode 2: V update (one GPU); 3: pack into exchange_dst(h) for the sum over ranks (sharded)
+int launch_xtu_epi(prmf_handle* h, int mode, int hist_slot = -1) {
+    EpiParams ep = plain_epi(h);
     const int64_t panels1 = h->plan.pass1.panels, panels2 = h->plan.pass2.panels;
     ep.arrive = h->epi_counters + panels1;
     ep.done = h->epi_counters + panels1 + panels2 + panels1;
@@ -712,7 +687,7 @@ int launch_xtu_epi(prmf_handle* h, int mode, double* packed_dst, int hist_slot =
     ep.Gu_part_in = h->Gu_part;
     ep.gu_parts = (int)panels1;
     if (mode == 3) {
-        ep.red = packed_dst;
+        ep.red = exchange_dst(h);
     } else {
         ep.Vold = h->Vbuf[h->vcur];
         ep.Vnew = h->Vbuf[h->vcur ^ 1];
@@ -731,13 +706,7 @@ int launch_xtu_epi(prmf_handle* h, int mode, double* packed_dst, int hist_slot =
             ep.doff = h->as_off;
         }
     }
-    int rc = 0;
-    if (h->x32) {
-        KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, mode, h->X32, h->ldx32, h->m, h->n, h->U, h->plan.pass2, h->Bpart,
-                     ep);
-    } else {
-        KT_SWITCH_RC(h->k, rc, launch_skinny_epi_t, h, mode, h->X, h->ldx, h->m, h->n, h->U, h->plan.pass2, h->Bpart, ep);
-    }
+    const int rc = launch_xstream(h, pass2(h), mode, ep);
     if (rc) { h->failed = true; return rc; }
     LAUNCH_CHECK(mode == 3 ? "skinny_tma_kernel(pass 2 + pack)" : "skinny_tma_kernel(pass 2 + V update)");
     if (mode != 3) h->vcur ^= 1;
@@ -858,13 +827,43 @@ void cancel_ahead(prmf_handle* h) {
     h->ahead = 0;
 }
 
+// The launch sequence of a block of inner steps (one steps_* function each, below)
+enum class StepPath {
+    Persistent,        // block_kernel runs the whole block, then objective_deferred_kernel
+    FusedDeferred,     // per step: pass 1 + U update, pass 2 + V update; objective_deferred_kernel after the block
+    FusedPerStep,      // per step: pass 1 + U update, pass 2 + V update, objective_parts_kernel
+    FusedSharded,      // per step: pass 1 + U update, pass 2 + pack, [ncclAllReduce], V update + objective (+ pull)
+    Unfused,           // per step: pass 1, U update, pass 2, [pack, exchange], V update + objective
+};
+
+// The one place that chooses the path of a block of steps.  Call after ensure_pos (it reads the active set's size).
+int step_path(prmf_handle* h, double tradeoff, StepPath* path) {
+    // the objective of every step can wait for one launch after the block when
+    const bool defer = h->defer_ok                       // the per-step history is allocated (PRMF_DEFER_OBJ != 0),
+                       && h->use_epi                     // the fused V update fills it,
+                       && (!sharded(h) || h->blk_xchg)   // every rank evaluates the same numbers (sharded: block_kernel),
+                       && tradeoff < 0.0                 // gamma and delta stay fixed (--tradeoff updates them every step),
+                       && !h->profiling                  // the objective is not timed as a phase of each step,
+                       && h->as.n_diag <= kVhCap;        // and the active set's values of V_new fit a history slot
+    if (block_path(h) && defer) *path = StepPath::Persistent;
+    else if (sharded(h) && !h->comm)                     // without NCCL only block_kernel exchanges between ranks
+        return fail(h, PRMF_ERR_STATE, "without an NCCL communicator a sharded handle can only run the persistent step kernel "
+                                       "(k <= 10, fixed gamma / delta, no per-phase profiling); call prmf_comm_init for this configuration");
+    else if (!h->use_epi) *path = StepPath::Unfused;
+    else if (defer) *path = StepPath::FusedDeferred;
+    else *path = sharded(h) ? StepPath::FusedSharded : StepPath::FusedPerStep;
+    return PRMF_OK;
+}
+
+// Pass 1 (+ U update) of the next block's first step, by the kernel step_path picks for that block when its objective
+// is deferred.  The block's tradeoff and active set are not known yet, so only step_path's tests of the handle decide.
 int prefetch_pass1(prmf_handle* h) {
     if (h->ahead || h->profiling || h->m == 0) return PRMF_OK;
     if (!h->have_X || !h->have_U || !h->have_V) return PRMF_OK;
     int rc = 0;
     if (h->failed) return PRMF_OK;
     if (block_path(h)) {
-        if ((rc = launch_block(h, 0, 1))) return rc;        // pass 1 + U update of the next block's first step
+        if ((rc = launch_block(h, 0, 1))) return rc;
         h->ahead = 2;
     } else if (h->use_epi) {
         if ((rc = launch_xv_epi(h))) return rc;
@@ -903,14 +902,6 @@ int ensure_obj_capacity(prmf_handle* h, int n_steps) {
     return fail(h, PRMF_ERR_ARG, "at most %d inner steps per prmf_step call", h->obj_capacity);
 }
 
-cudaEvent_t get_event(prmf_handle* h, int* idx) {
-    cudaEvent_t e;
-    cudaEventCreate(&e);
-    h->ev_pool.push_back(e);
-    *idx = (int)h->ev_pool.size() - 1;
-    return e;
-}
-
 void harvest_events(prmf_handle* h) {
     for (auto& pr : h->ev_pairs) {
         float ms = 0.f;
@@ -924,6 +915,114 @@ void harvest_events(prmf_handle* h) {
     h->ev_pairs.clear();
 }
 
+// phase timing (profiling mode only): an event pair around each phase of the step
+void tic(prmf_handle* h, int phase) {
+    if (!h->profiling) return;
+    cudaEvent_t e[2];
+    cudaEventCreate(&e[0]);
+    cudaEventCreate(&e[1]);
+    h->ev_pairs.push_back({phase, (int)h->ev_pool.size()});
+    h->ev_pool.insert(h->ev_pool.end(), e, e + 2);
+    cudaEventRecord(e[0], h->stream);
+}
+
+void toc(prmf_handle* h) {
+    if (!h->profiling) return;
+    cudaEventRecord(h->ev_pool[h->ev_pairs.back().second + 1], h->stream);
+}
+
+// the objective of every step of a block from the history slots its V updates filled: one thread block per step
+int launch_deferred_objective(prmf_handle* h, int n_steps) {
+    objective_deferred_kernel<<<n_steps, kTailThreads, obj_smem(h), h->stream>>>(
+        h->k, h->hist_Gu, h->hist_Gvp, h->hist_VBp, h->plan.pass2.panels, h->hist_vh, kVhCap, h->normX_sq, h->as, h->Gv,
+        h->gd, h->obj, h->obj_capacity);
+    LAUNCH_CHECK("objective_deferred_kernel");
+    return PRMF_OK;
+}
+
+// ---- the launch sequence of each StepPath.  pass1_done: prmf_block_end already enqueued pass 1 (+ U update) of the
+// first step (prefetch_pass1).
+
+int steps_persistent(prmf_handle* h, int n_steps, bool pass1_done) {
+    const int h0 = pass1_done ? 1 : 0;
+    int rc = launch_block(h, h0, 2 * n_steps - h0);
+    if (rc) return rc;
+    return launch_deferred_objective(h, n_steps);
+}
+
+int steps_fused_deferred(prmf_handle* h, int n_steps, bool pass1_done) {
+    const size_t kk2 = (size_t)h->k * h->k;
+    const int64_t panels2 = h->plan.pass2.panels;
+    for (int s = 0; s < n_steps; ++s) {
+        int rc = 0;
+        // pass 1 of a later step reads V^T V as the panel partials the previous step's V update left in its slot
+        if (s > 0) rc = launch_xv_epi(h, h->hist_Gvp + (size_t)(s - 1) * panels2 * kk2, (int)panels2);
+        else if (!pass1_done) rc = launch_xv_epi(h);
+        if (rc) return rc;
+        if ((rc = launch_xtu_epi(h, 2, s))) return rc;
+    }
+    return launch_deferred_objective(h, n_steps);
+}
+
+int steps_fused_per_step(prmf_handle* h, int n_steps, bool pass1_done, double tradeoff) {
+    for (int s = 0; s < n_steps; ++s) {
+        int rc = 0;
+        if (s > 0 || !pass1_done) { tic(h, 0); rc = launch_xv_epi(h); toc(h); }
+        if (rc) return rc;
+        tic(h, 2); rc = launch_xtu_epi(h, 2); toc(h);                  // + V update
+        if (rc) return rc;
+        tic(h, 5); rc = launch_objective(h, tradeoff, h->Gu_part, h->plan.pass1.panels); toc(h);
+        if (rc) return rc;
+    }
+    return PRMF_OK;
+}
+
+int steps_fused_sharded(prmf_handle* h, int n_steps, bool pass1_done, double tradeoff) {
+    const size_t red_count = (size_t)h->n * h->k + (size_t)h->k * h->k + 2;
+    for (int s = 0; s < n_steps; ++s) {
+        int rc = 0;
+        if (s > 0 || !pass1_done) { tic(h, 0); rc = launch_xv_epi(h); toc(h); }
+        if (rc) return rc;
+        tic(h, 2); rc = launch_xtu_epi(h, 3); toc(h);                  // + pack
+        if (rc) return rc;
+        if (!h->p2p_ready) {                                            // else: pulled inside the V update
+            tic(h, 3); rc = allreduce(h, h->red, red_count); toc(h);
+            if (rc) return rc;
+        }
+        tic(h, 4); rc = launch_v_update_objective(h, true, tradeoff); toc(h);
+        if (rc) return rc;
+    }
+    return PRMF_OK;
+}
+
+int steps_unfused(prmf_handle* h, int n_steps, bool pass1_done, double tradeoff) {
+    const bool is_sharded = sharded(h);
+    const int64_t nk = h->n * h->k;
+    const int kk2 = h->k * h->k;
+    for (int s = 0; s < n_steps; ++s) {
+        int rc = 0;
+        if (s > 0 || !pass1_done) { tic(h, 0); rc = launch_xv(h); toc(h); }
+        if (rc) return rc;
+        tic(h, 1); rc = launch_u_update(h); toc(h);
+        if (rc) return rc;
+        tic(h, 2); rc = launch_xtu(h); toc(h);
+        if (rc) return rc;
+        if (is_sharded) {
+            tic(h, 3);
+            reduce_pack_kernel<<<(unsigned)((nk + kk2 + 2 + 255) / 256), 256, 0, h->stream>>>(
+                h->Bpart, b_chunks(h), nk, h->Gu_part, h->uu_grid, h->k, exchange_dst(h));
+            LAUNCH_CHECK("reduce_pack_kernel");
+            if (!h->p2p_ready) rc = allreduce(h, h->red, (size_t)nk + kk2 + 2);      // else: pulled inside the V update
+            toc(h);
+            if (rc) return rc;
+        }
+        tic(h, 4); rc = launch_v_update_objective(h, is_sharded, tradeoff); toc(h);
+        if (rc) return rc;
+    }
+    return PRMF_OK;
+}
+
+// Enqueues a block of n_steps inner steps: the launch sequence of the StepPath that step_path chooses.
 int enqueue_steps(prmf_handle* h, int n_steps, double gamma, double delta, double tradeoff) {
     if (!h->have_X || !h->have_U || !h->have_V || !h->have_pw || !h->have_active)
         return fail(h, PRMF_ERR_STATE, "prmf_step needs X, U/V, pathways and the active set first");
@@ -936,101 +1035,18 @@ int enqueue_steps(prmf_handle* h, int n_steps, double gamma, double delta, doubl
     const double gdh[2] = {gamma, delta};
     CU(cudaMemcpyAsync(h->gd, gdh, sizeof gdh, cudaMemcpyHostToDevice, h->stream));
     CU(cudaMemsetAsync(h->step_counter, 0, sizeof(int), h->stream));
-    const int64_t nk = h->n * h->k;
-    const int kk2 = h->k * h->k;
-    const size_t red_count = (size_t)nk + kk2 + 2;
-    // phase timing (profiling mode only): an event pair around each phase of the step
-    auto tic = [&](int phase) {
-        if (!h->profiling) return;
-        int i0 = 0, i1 = 0;
-        cudaEvent_t e0 = get_event(h, &i0);
-        get_event(h, &i1);
-        cudaEventRecord(e0, h->stream);
-        h->ev_pairs.push_back({phase, i0});
-    };
-    auto toc = [&]() {
-        if (!h->profiling) return;
-        cudaEventRecord(h->ev_pool[h->ev_pairs.back().second + 1], h->stream);
-    };
-    // deferred objective: one GPU, or sharded with the persistent step kernel (every rank evaluates the same numbers)
-    const bool defer = h->defer_ok && h->use_epi && (!sharded(h) || h->blk_xchg) && tradeoff < 0.0 &&
-                       !h->profiling && h->as.n_diag <= kVhCap;
-    if (defer && block_path(h)) {
-        // the whole block in ONE persistent launch (block.cuh) + the deferred objective
-        const int h0 = h->ahead != 0 ? 1 : 0;               // pass 1 + U update of step 0 already done by prmf_block_end
-        h->ahead = 0;
-        if ((rc = launch_block(h, h0, 2 * n_steps - h0))) return rc;
-        objective_deferred_kernel<<<n_steps, kTailThreads, obj_smem(h), h->stream>>>(
-            h->k, h->hist_Gu, h->hist_Gvp, h->hist_VBp, h->plan.pass2.panels, h->hist_vh, kVhCap, h->normX_sq, h->as, h->Gv,
-            h->gd, h->obj, h->obj_capacity);
-        LAUNCH_CHECK("objective_deferred_kernel");
-        return PRMF_OK;
+    StepPath path;
+    if ((rc = step_path(h, tradeoff, &path))) return rc;
+    const bool pass1_done = h->ahead != 0;
+    h->ahead = 0;
+    switch (path) {
+        case StepPath::Persistent: return steps_persistent(h, n_steps, pass1_done);
+        case StepPath::FusedDeferred: return steps_fused_deferred(h, n_steps, pass1_done);
+        case StepPath::FusedPerStep: return steps_fused_per_step(h, n_steps, pass1_done, tradeoff);
+        case StepPath::FusedSharded: return steps_fused_sharded(h, n_steps, pass1_done, tradeoff);
+        case StepPath::Unfused: return steps_unfused(h, n_steps, pass1_done, tradeoff);
     }
-    if (sharded(h) && !h->comm)
-        return fail(h, PRMF_ERR_STATE, "without an NCCL communicator a sharded handle can only run the persistent step kernel "
-                                       "(k <= 10, fixed gamma / delta, no per-phase profiling); call prmf_comm_init for this configuration");
-    for (int s = 0; s < n_steps; ++s) {
-        const bool skip_pass1 = s == 0 && h->ahead != 0;      // already enqueued by prmf_block_end
-        if (skip_pass1) h->ahead = 0;
-        if (h->use_epi && defer) {
-            // one GPU, fixed gamma / delta: the objective of every step is evaluated by ONE launch after the block
-            if (!skip_pass1) {
-                const size_t kk2s = (size_t)h->k * h->k;
-                const int64_t panels2 = h->plan.pass2.panels;
-                rc = s == 0 ? launch_xv_epi(h) : launch_xv_epi(h, h->hist_Gvp + (size_t)(s - 1) * panels2 * kk2s, (int)panels2);
-                if (rc) return rc;
-            }
-            if ((rc = launch_xtu_epi(h, 2, nullptr, s))) return rc;
-            if (s == n_steps - 1) {
-                objective_deferred_kernel<<<n_steps, kTailThreads, obj_smem(h), h->stream>>>(
-                    h->k, h->hist_Gu, h->hist_Gvp, h->hist_VBp, h->plan.pass2.panels, h->hist_vh, kVhCap, h->normX_sq, h->as, h->Gv,
-                    h->gd, h->obj, h->obj_capacity);
-                LAUNCH_CHECK("objective_deferred_kernel");
-            }
-            continue;
-        }
-        if (h->use_epi) {
-            if (!skip_pass1) { tic(0); rc = launch_xv_epi(h); toc(); }
-            if (rc) return rc;
-            if (!sharded(h)) {
-                tic(2); rc = launch_xtu_epi(h, 2, nullptr); toc();               // + V update
-                if (rc) return rc;
-                tic(5); rc = launch_objective(h, tradeoff, h->Gu_part, h->plan.pass1.panels); toc();
-                if (rc) return rc;
-            } else {
-                double* dst = h->p2p_ready ? h->p2p_buf + (size_t)h->p2p_parity * h->p2p_red_count : h->red;
-                tic(2); rc = launch_xtu_epi(h, 3, dst); toc();
-                if (rc) return rc;
-                if (!h->p2p_ready) {
-                    tic(3); rc = allreduce(h, h->red, red_count); toc();
-                    if (rc) return rc;
-                }
-                tic(4); rc = launch_v_update_objective(h, true, tradeoff); toc();
-                if (rc) return rc;
-            }
-            continue;
-        }
-        if (!skip_pass1) { tic(0); rc = launch_xv(h); toc(); }
-        if (rc) return rc;
-        tic(1); rc = launch_u_update(h); toc();
-        if (rc) return rc;
-        tic(2); rc = launch_xtu(h); toc();
-        if (rc) return rc;
-        const bool is_sharded = sharded(h);
-        if (is_sharded) {
-            tic(3);
-            double* dst = h->p2p_ready ? h->p2p_buf + (size_t)h->p2p_parity * h->p2p_red_count : h->red;
-            reduce_pack_kernel<<<(unsigned)((nk + kk2 + 2 + 255) / 256), 256, 0, h->stream>>>(
-                h->Bpart, b_chunks(h), nk, h->Gu_part, h->uu_grid, h->k, dst);
-            LAUNCH_CHECK("reduce_pack_kernel");
-            if (!h->p2p_ready) rc = allreduce(h, h->red, red_count);      // else: summed inside the V update
-            toc();
-            if (rc) return rc;
-        }
-        tic(4); rc = launch_v_update_objective(h, is_sharded, tradeoff); toc();
-        if (rc) return rc;
-    }
-    return PRMF_OK;
+    return fail(h, PRMF_ERR_STATE, "unknown step path");
 }
 
 int check_err_word(prmf_handle* h, unsigned int errw) {
