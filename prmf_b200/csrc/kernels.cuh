@@ -773,10 +773,24 @@ __device__ __forceinline__ void epi_pack(const EpiParams& ep, int panel, int64_t
 
 
 // ----------------------------------------------------------------------------------------------------
-// X-stream kernels (k <= 10).  The body is shared by the fp64 storage mode (T = double) and the fp32 storage mode
-// (T = float, skinny_tma_f32_kernel): an fp32 element is widened to fp64 exactly before its DFMA, so every column runs
-// the same fma chain in the same row order on the same values, and the fp32 kernel returns, bit for bit, what the
-// fp64 kernel returns on the widened matrix under the same launch plan.
+// X-stream kernels: out[chunk][j][0:k] = sum over the rows i of the chunk of M[i][j] * W[i][0:k].  One CTA streams the
+// rows of its chunk through a TMA ring: the producer warp bulk-copies a stage of RS rows of its column panel of M and
+// the RS matching rows of W, and each of the 256 consumer threads accumulates 4 columns x KT factors in registers.
+//
+// One body serves every kernel; a single compile-time fact, FIXED_K, separates the two families:
+//  - FIXED_K (skinny_tma_kernel<K,RS,EPI>, k = K <= 10): the wrapper passes k = KT, so the W row stride, the W slot and
+//    the store are compile-time; one factor group; an unrolled branch for full stages; the fused tails EPI 1 / 2 / 3
+//    run behind the store.
+//  - run-time k (skinny_tma_gen_kernel<KT,FG,RS>, 10 < k <= 128, no fused tail): the consumers split into FG factor
+//    groups of 256/FG threads.  A thread owns 4 columns of a (1024/FG)-column panel and KT consecutive factors of its
+//    group, so the X tile is fetched from HBM once and re-read from shared memory by every group -- at k = 64 the
+//    kernel is FP64-FMA bound (16 flop per byte of X), not HBM bound.  Factors >= k are computed on in-bounds garbage
+//    and never written.  A group reads W indices up to f0 + (RS-1) k + KT - 1, which for f0 < k is <= RS k + KT - 2,
+//    inside the RS k + KT doubles of the W slot; groups with f0 >= k read group 0's columns instead.
+//
+// T is the storage of X: double, or float for the fp32 storage mode (the _f32_ kernels).  An fp32 element is widened to
+// fp64 exactly before its DFMA, so every column runs the same fma chain in the same row order on the same values, and
+// the fp32 kernel returns, bit for bit, what the fp64 kernel returns on the widened matrix under the same launch plan.
 // ----------------------------------------------------------------------------------------------------
 // the two consecutive elements i = 2p, 2p + 1 of a shared-memory row, as fp64
 __device__ __forceinline__ double2 x_pair(const double* row, int p) { return reinterpret_cast<const double2*>(row)[p]; }
@@ -785,178 +799,25 @@ __device__ __forceinline__ double2 x_pair(const float* row, int p) {
     return make_double2((double)v.x, (double)v.y);
 }
 
-template <typename T, int KT, int RS, int EPI>
+template <typename T, bool FIXED_K, int KT, int FG, int RS, int EPI>
 __device__ __forceinline__ void
 skinny_tma_body(const T* __restrict__ M, int64_t ldm, int64_t rows_total, int64_t cols,
-                const double* __restrict__ W, int panel_w, int64_t rows_per_chunk, int stages,
+                const double* __restrict__ W, int k, int panel_w, int64_t rows_per_chunk, int stages,
                 double* __restrict__ OutPart, const EpiParams& ep, unsigned tid) {
+    static_assert(!FIXED_K || FG == 1, "a fixed k <= 10 runs one factor group");
+    static_assert(FIXED_K || EPI == 0, "the fused tails need k fixed at compile time");
     extern __shared__ __align__(128) unsigned char smem_raw[];
     constexpr uint32_t XB = (uint32_t)sizeof(T);                          // bytes per stored element of X
+    constexpr int TG = 256 / FG;                                          // threads per factor group
+    constexpr uint32_t W_SLACK = FIXED_K ? 0 : KT;                        // doubles behind a stage's W rows
     const int panel = blockIdx.x;
     const int64_t chunk = blockIdx.y;
     const int64_t c0 = (int64_t)panel * panel_w;                          // first column of the panel
     const int width = (int)min((int64_t)panel_w, ldm - c0);               // columns held (multiple of 4)
     const uint32_t row_bytes = (uint32_t)width * XB;
     const uint32_t x_stage_bytes = (uint32_t)RS * (uint32_t)panel_w * XB;
-    const uint32_t w_bytes = (uint32_t)RS * KT * 8u;
-    const uint32_t stage_bytes = x_stage_bytes + ((w_bytes + 127u) & ~127u);
-    uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem_raw + (size_t)stages * stage_bytes);
-    uint64_t* empty_bar = full_bar + stages;
-    const int64_t rbeg = chunk * rows_per_chunk;
-    const int64_t rend = min(rows_total, rbeg + rows_per_chunk);
-    const int nstage_iters = rend > rbeg ? (int)((rend - rbeg + RS - 1) / RS) : 0;
-    const int warp = tid >> 5, lane = tid & 31;
-    KT_STAMP_MIN(ep.dbg_slot, 0);
-
-    if (tid == 0) {
-        for (int s2 = 0; s2 < stages; ++s2) {
-            mbar_init(&full_bar[s2], 1);
-            mbar_init(&empty_bar[s2], kTmaConsumerWarps);
-        }
-        fence_mbar_init();
-    }
-    __syncthreads();
-
-    if (warp == kTmaConsumerWarps) {
-        // ===== producer warp: lanes 0..RS-1 copy one row piece each, lane 0 also copies the W rows =====
-        const uint64_t pol_x = l2_policy_evict_first();
-        const uint64_t pol_w = l2_policy_evict_last();
-        int s2 = 0;
-        uint32_t phase = 0;
-        for (int it = 0; it < nstage_iters; ++it) {
-            const int64_t r0 = rbeg + (int64_t)it * RS;
-            const int rows = (int)min((int64_t)RS, rend - r0);
-            if (lane == 0) mbar_wait(&empty_bar[s2], phase ^ 1u);
-            __syncwarp();
-            unsigned char* sx = smem_raw + (size_t)s2 * stage_bytes;
-            if (lane == 0) {
-                mbar_arrive_expect_tx(&full_bar[s2], (uint32_t)rows * row_bytes + w_bytes);
-                bulk_g2s(sx + x_stage_bytes, W + r0 * KT, w_bytes, &full_bar[s2], pol_w);
-            }
-            __syncwarp();
-            if (lane < rows)
-                bulk_g2s(sx + (size_t)lane * panel_w * XB, M + (r0 + lane) * ldm + c0, row_bytes, &full_bar[s2], pol_x);
-            if (++s2 == stages) { s2 = 0; phase ^= 1u; }
-        }
-        return;
-    }
-
-    // ===== consumer warps =====
-    const int H = panel_w >> 2;                        // double2 columns per half panel
-    const int t = tid;                         // 0..255
-    const bool active = t < H && (2 * t) < width;      // first pair inside the held columns
-    const bool active2 = t < H && (2 * (t + H)) < width;
-    double acc[4][KT];
-#pragma unroll
-    for (int g = 0; g < 4; ++g)
-#pragma unroll
-        for (int c = 0; c < KT; ++c) acc[g][c] = 0.0;
-    int s2 = 0;
-    uint32_t phase = 0;
-    for (int it = 0; it < nstage_iters; ++it) {
-        const int rows = (int)min((int64_t)RS, rend - (rbeg + (int64_t)it * RS));
-        mbar_wait(&full_bar[s2], phase);
-        const unsigned char* sx = smem_raw + (size_t)s2 * stage_bytes;
-        const double* sw = reinterpret_cast<const double*>(sx + x_stage_bytes);
-        if (rows == RS) {
-#pragma unroll
-            for (int r = 0; r < RS; ++r) {
-                const T* xrow = reinterpret_cast<const T*>(sx + (size_t)r * panel_w * XB);
-                const double2 xa = active ? x_pair(xrow, t) : make_double2(0.0, 0.0);
-                const double2 xb = active2 ? x_pair(xrow, t + H) : make_double2(0.0, 0.0);
-#pragma unroll
-                for (int c = 0; c < KT; ++c) {
-                    const double u = sw[r * KT + c];
-                    acc[0][c] = fma(xa.x, u, acc[0][c]);
-                    acc[1][c] = fma(xa.y, u, acc[1][c]);
-                    acc[2][c] = fma(xb.x, u, acc[2][c]);
-                    acc[3][c] = fma(xb.y, u, acc[3][c]);
-                }
-            }
-        } else {
-            for (int r = 0; r < rows; ++r) {
-                const T* xrow = reinterpret_cast<const T*>(sx + (size_t)r * panel_w * XB);
-                const double2 xa = active ? x_pair(xrow, t) : make_double2(0.0, 0.0);
-                const double2 xb = active2 ? x_pair(xrow, t + H) : make_double2(0.0, 0.0);
-#pragma unroll
-                for (int c = 0; c < KT; ++c) {
-                    const double u = sw[r * KT + c];
-                    acc[0][c] = fma(xa.x, u, acc[0][c]);
-                    acc[1][c] = fma(xa.y, u, acc[1][c]);
-                    acc[2][c] = fma(xb.x, u, acc[2][c]);
-                    acc[3][c] = fma(xb.y, u, acc[3][c]);
-                }
-            }
-        }
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&empty_bar[s2]);
-        if (++s2 == stages) { s2 = 0; phase ^= 1u; }
-    }
-    // columns owned: c0 + 2t, c0 + 2t + 1, c0 + 2(t+H), c0 + 2(t+H) + 1
-#pragma unroll
-    for (int g = 0; g < 4; ++g) {
-        const int64_t j = c0 + 2 * (int64_t)(g < 2 ? t : t + H) + (g & 1);
-        const bool ok = (g < 2 ? active : active2) && j < cols;
-        if (ok) {
-            double* out = OutPart + ((int64_t)chunk * cols + j) * KT;
-#pragma unroll
-            for (int c = 0; c < KT; ++c) out[c] = acc[g][c];
-        }
-    }
-    KT_STAMP_MAX(ep.dbg_slot, 1);
-    if constexpr (EPI != 0) {
-        __shared__ int s_last;
-        if constexpr (EPI == 1) epi_u_update<KT>(ep, smem_raw, &s_last, panel, c0, width, cols, OutPart);
-        if constexpr (EPI == 2) epi_v_update<KT>(ep, smem_raw, &s_last, panel, c0, width, cols, OutPart);
-        if constexpr (EPI == 3) epi_pack<KT>(ep, panel, c0, width, cols, OutPart);
-    }
-    KT_STAMP_MAX(ep.dbg_slot, 2);
-}
-
-// fp64 X (PRMF_X_F64)
-template <int KT, int RS, int EPI>
-__global__ void __launch_bounds__(kTmaThreads, 1)
-skinny_tma_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_total, int64_t cols,
-                  const double* __restrict__ W, int panel_w, int64_t rows_per_chunk, int stages,
-                  double* __restrict__ OutPart, const EpiParams ep) {
-    skinny_tma_body<double, KT, RS, EPI>(M, ldm, rows_total, cols, W, panel_w, rows_per_chunk, stages, OutPart, ep, threadIdx.x);
-}
-
-// fp32 X (PRMF_X_F32); single rank, so the fused tails are the U update (EPI 1) and the V update (EPI 2) only
-template <int KT, int RS, int EPI>
-__global__ void __launch_bounds__(kTmaThreads, 1)
-skinny_tma_f32_kernel(const float* __restrict__ M, int64_t ldm, int64_t rows_total, int64_t cols,
-                      const double* __restrict__ W, int panel_w, int64_t rows_per_chunk, int stages,
-                      double* __restrict__ OutPart, const EpiParams ep) {
-    static_assert(EPI <= 2, "the fp32 storage mode has no sharded tails");
-    skinny_tma_body<float, KT, RS, EPI>(M, ldm, rows_total, cols, W, panel_w, rows_per_chunk, stages, OutPart, ep, threadIdx.x);
-}
-
-// ----------------------------------------------------------------------------------------------------
-// General-k TMA X-stream kernel (k > 10: BASELINE configs 4 and 5).  Same pipeline as skinny_tma_kernel; the
-// 256 consumer threads are split into FG factor groups of 256/FG threads.  A thread owns 4 columns of a
-// (1024/FG)-column panel and KT consecutive factors of its group, so the X tile is fetched from HBM once and
-// re-read from shared memory by every group -- at k = 64 the kernel is FP64-FMA bound (16 flop per byte of X),
-// not HBM bound.  k is a run-time value: factors >= k are computed on in-bounds garbage and never written.  A group
-// reads W indices up to f0 + (RS-1) k + KT - 1, which for f0 < k is <= RS k + KT - 2, inside the RS k + KT doubles
-// of the W slot; groups with f0 >= k read group 0's columns instead.
-// ----------------------------------------------------------------------------------------------------
-template <typename T, int KT, int FG, int RS>
-__device__ __forceinline__ void
-skinny_tma_gen_body(const T* __restrict__ M, int64_t ldm, int64_t rows_total, int64_t cols,
-                    const double* __restrict__ W, int k, int panel_w, int64_t rows_per_chunk, int stages,
-                    double* __restrict__ OutPart, unsigned tid) {
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    constexpr uint32_t XB = (uint32_t)sizeof(T);
-    constexpr int TG = 256 / FG;                                          // threads per factor group
-    const int panel = blockIdx.x;
-    const int64_t chunk = blockIdx.y;
-    const int64_t c0 = (int64_t)panel * panel_w;
-    const int width = (int)min((int64_t)panel_w, ldm - c0);
-    const uint32_t row_bytes = (uint32_t)width * XB;
-    const uint32_t x_stage_bytes = (uint32_t)RS * (uint32_t)panel_w * XB;
     const uint32_t w_bytes = (uint32_t)RS * (uint32_t)k * 8u;
-    const uint32_t w_slot = (((uint32_t)RS * (uint32_t)k + KT) * 8u + 127u) & ~127u;   // + KT doubles of slack
+    const uint32_t w_slot = (((uint32_t)RS * (uint32_t)k + W_SLACK) * 8u + 127u) & ~127u;
     const uint32_t stage_bytes = x_stage_bytes + w_slot;
     uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem_raw + (size_t)stages * stage_bytes);
     uint64_t* empty_bar = full_bar + stages;
@@ -964,6 +825,7 @@ skinny_tma_gen_body(const T* __restrict__ M, int64_t ldm, int64_t rows_total, in
     const int64_t rend = min(rows_total, rbeg + rows_per_chunk);
     const int nstage_iters = rend > rbeg ? (int)((rend - rbeg + RS - 1) / RS) : 0;
     const int warp = tid >> 5, lane = tid & 31;
+    if constexpr (FIXED_K) KT_STAMP_MIN(ep.dbg_slot, 0);
 
     if (tid == 0) {
         for (int s2 = 0; s2 < stages; ++s2) {
@@ -973,11 +835,13 @@ skinny_tma_gen_body(const T* __restrict__ M, int64_t ldm, int64_t rows_total, in
         fence_mbar_init();
     }
     // the slack behind every W slot is read (and discarded) by the last factor group: keep it finite
-    for (int s2 = tid; s2 < stages * KT; s2 += blockDim.x)
-        reinterpret_cast<double*>(smem_raw + (size_t)(s2 / KT) * stage_bytes + x_stage_bytes + w_bytes)[s2 % KT] = 0.0;
+    if constexpr (W_SLACK > 0)
+        for (int s2 = tid; s2 < stages * KT; s2 += blockDim.x)
+            reinterpret_cast<double*>(smem_raw + (size_t)(s2 / KT) * stage_bytes + x_stage_bytes + w_bytes)[s2 % KT] = 0.0;
     __syncthreads();
 
     if (warp == kTmaConsumerWarps) {
+        // ===== producer warp: lanes 0..RS-1 copy one row piece each, lane 0 also copies the W rows =====
         const uint64_t pol_x = l2_policy_evict_first();
         const uint64_t pol_w = l2_policy_evict_last();
         int s2 = 0;
@@ -1000,14 +864,15 @@ skinny_tma_gen_body(const T* __restrict__ M, int64_t ldm, int64_t rows_total, in
         return;
     }
 
-    const int H = panel_w >> 2;
-    const int fg = tid / TG, t = tid % TG;
-    const int f0 = fg * KT;                                               // first factor of this thread
+    // ===== consumer warps =====
+    const int H = panel_w >> 2;                        // double2 columns per half panel
+    const int fg = FIXED_K ? 0 : tid / TG, t = FIXED_K ? tid : tid % TG;   // factor group, thread within it
+    const int f0 = fg * KT;                            // first factor of this thread
     // groups whose factors all lie at or beyond k (k = 33..36, 65..84, 97..112) read group 0's columns, since their
     // own can lie past the W slot; what they compute is never written.  A branch around their loop instead measured
     // 1 % slower on the k = 64 stream, where no group is idle (B200, 1000 W).
     const int fr = f0 < k ? f0 : 0;
-    const bool active = t < H && (2 * t) < width;
+    const bool active = t < H && (2 * t) < width;      // first pair inside the held columns
     const bool active2 = t < H && (2 * (t + H)) < width;
     double acc[4][KT];
 #pragma unroll
@@ -1021,24 +886,43 @@ skinny_tma_gen_body(const T* __restrict__ M, int64_t ldm, int64_t rows_total, in
         mbar_wait(&full_bar[s2], phase);
         const unsigned char* sx = smem_raw + (size_t)s2 * stage_bytes;
         const double* sw = reinterpret_cast<const double*>(sx + x_stage_bytes) + fr;
-        for (int r = 0; r < rows; ++r) {
-            const T* xrow = reinterpret_cast<const T*>(sx + (size_t)r * panel_w * XB);
-            const double2 xa = active ? x_pair(xrow, t) : make_double2(0.0, 0.0);
-            const double2 xb = active2 ? x_pair(xrow, t + H) : make_double2(0.0, 0.0);
-            const double* wr = sw + r * k;
+        // the same row step twice: unrolled over a full stage at fixed k, a plain loop otherwise (a helper function or
+        // lambda for the step changes the fixed-k kernels' SASS)
+        if (FIXED_K && rows == RS) {
 #pragma unroll
-            for (int c = 0; c < KT; ++c) {
-                const double u = wr[c];
-                acc[0][c] = fma(xa.x, u, acc[0][c]);
-                acc[1][c] = fma(xa.y, u, acc[1][c]);
-                acc[2][c] = fma(xb.x, u, acc[2][c]);
-                acc[3][c] = fma(xb.y, u, acc[3][c]);
+            for (int r = 0; r < RS; ++r) {
+                const T* xrow = reinterpret_cast<const T*>(sx + (size_t)r * panel_w * XB);
+                const double2 xa = active ? x_pair(xrow, t) : make_double2(0.0, 0.0);
+                const double2 xb = active2 ? x_pair(xrow, t + H) : make_double2(0.0, 0.0);
+#pragma unroll
+                for (int c = 0; c < KT; ++c) {
+                    const double u = sw[r * k + c];
+                    acc[0][c] = fma(xa.x, u, acc[0][c]);
+                    acc[1][c] = fma(xa.y, u, acc[1][c]);
+                    acc[2][c] = fma(xb.x, u, acc[2][c]);
+                    acc[3][c] = fma(xb.y, u, acc[3][c]);
+                }
+            }
+        } else {
+            for (int r = 0; r < rows; ++r) {
+                const T* xrow = reinterpret_cast<const T*>(sx + (size_t)r * panel_w * XB);
+                const double2 xa = active ? x_pair(xrow, t) : make_double2(0.0, 0.0);
+                const double2 xb = active2 ? x_pair(xrow, t + H) : make_double2(0.0, 0.0);
+#pragma unroll
+                for (int c = 0; c < KT; ++c) {
+                    const double u = sw[r * k + c];
+                    acc[0][c] = fma(xa.x, u, acc[0][c]);
+                    acc[1][c] = fma(xa.y, u, acc[1][c]);
+                    acc[2][c] = fma(xb.x, u, acc[2][c]);
+                    acc[3][c] = fma(xb.y, u, acc[3][c]);
+                }
             }
         }
         __syncwarp();
         if (lane == 0) mbar_arrive(&empty_bar[s2]);
         if (++s2 == stages) { s2 = 0; phase ^= 1u; }
     }
+    // columns owned: c0 + 2t, c0 + 2t + 1, c0 + 2(t+H), c0 + 2(t+H) + 1
 #pragma unroll
     for (int g = 0; g < 4; ++g) {
         const int64_t j = c0 + 2 * (int64_t)(g < 2 ? t : t + H) + (g & 1);
@@ -1050,22 +934,58 @@ skinny_tma_gen_body(const T* __restrict__ M, int64_t ldm, int64_t rows_total, in
                 if (f0 + c < k) out[c] = acc[g][c];
         }
     }
+    if constexpr (FIXED_K) {
+        KT_STAMP_MAX(ep.dbg_slot, 1);
+        if constexpr (EPI != 0) {
+            __shared__ int s_last;
+            if constexpr (EPI == 1) epi_u_update<KT>(ep, smem_raw, &s_last, panel, c0, width, cols, OutPart);
+            if constexpr (EPI == 2) epi_v_update<KT>(ep, smem_raw, &s_last, panel, c0, width, cols, OutPart);
+            if constexpr (EPI == 3) epi_pack<KT>(ep, panel, c0, width, cols, OutPart);
+        }
+        KT_STAMP_MAX(ep.dbg_slot, 2);
+    }
 }
 
+// The four kernels share one parameter list; a fixed-k kernel ignores `k`, a general-k kernel ignores `ep`.
+// fp64 X (PRMF_X_F64), k = KT <= 10
+template <int KT, int RS, int EPI>
+__global__ void __launch_bounds__(kTmaThreads, 1)
+skinny_tma_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_total, int64_t cols,
+                  const double* __restrict__ W, int k, int panel_w, int64_t rows_per_chunk, int stages,
+                  double* __restrict__ OutPart, const EpiParams ep) {
+    skinny_tma_body<double, true, KT, 1, RS, EPI>(M, ldm, rows_total, cols, W, KT, panel_w, rows_per_chunk, stages,
+                                                 OutPart, ep, threadIdx.x);
+}
+
+// fp32 X (PRMF_X_F32), k = KT <= 10; single rank, so the fused tails are the U update (EPI 1) and the V update (EPI 2)
+template <int KT, int RS, int EPI>
+__global__ void __launch_bounds__(kTmaThreads, 1)
+skinny_tma_f32_kernel(const float* __restrict__ M, int64_t ldm, int64_t rows_total, int64_t cols,
+                      const double* __restrict__ W, int k, int panel_w, int64_t rows_per_chunk, int stages,
+                      double* __restrict__ OutPart, const EpiParams ep) {
+    static_assert(EPI <= 2, "the fp32 storage mode has no sharded tails");
+    skinny_tma_body<float, true, KT, 1, RS, EPI>(M, ldm, rows_total, cols, W, KT, panel_w, rows_per_chunk, stages,
+                                                OutPart, ep, threadIdx.x);
+}
+
+// fp64 X, 10 < k <= 128 (BASELINE configs 4 and 5)
 template <int KT, int FG, int RS>
 __global__ void __launch_bounds__(kTmaThreads, 1)
 skinny_tma_gen_kernel(const double* __restrict__ M, int64_t ldm, int64_t rows_total, int64_t cols,
                       const double* __restrict__ W, int k, int panel_w, int64_t rows_per_chunk, int stages,
-                      double* __restrict__ OutPart) {
-    skinny_tma_gen_body<double, KT, FG, RS>(M, ldm, rows_total, cols, W, k, panel_w, rows_per_chunk, stages, OutPart, threadIdx.x);
+                      double* __restrict__ OutPart, const EpiParams ep) {
+    skinny_tma_body<double, false, KT, FG, RS, 0>(M, ldm, rows_total, cols, W, k, panel_w, rows_per_chunk, stages,
+                                                 OutPart, ep, threadIdx.x);
 }
 
+// fp32 X, 10 < k <= 128
 template <int KT, int FG, int RS>
 __global__ void __launch_bounds__(kTmaThreads, 1)
 skinny_tma_gen_f32_kernel(const float* __restrict__ M, int64_t ldm, int64_t rows_total, int64_t cols,
                           const double* __restrict__ W, int k, int panel_w, int64_t rows_per_chunk, int stages,
-                          double* __restrict__ OutPart) {
-    skinny_tma_gen_body<float, KT, FG, RS>(M, ldm, rows_total, cols, W, k, panel_w, rows_per_chunk, stages, OutPart, threadIdx.x);
+                          double* __restrict__ OutPart, const EpiParams ep) {
+    skinny_tma_body<float, false, KT, FG, RS, 0>(M, ldm, rows_total, cols, W, k, panel_w, rows_per_chunk, stages,
+                                                OutPart, ep, threadIdx.x);
 }
 
 // Xt[j][i] = X[i][j] : the factor of 2 in HBM capacity buys a coalesced, reduction-free pass 1.

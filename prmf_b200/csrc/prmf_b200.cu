@@ -1,8 +1,9 @@
 // libprmf_b200.so -- C ABI (include/prmf_b200.h) over the sm_100a kernels in kernels.cuh, block.cuh and tf32.cuh.
 // Host orchestration of one PRMF inner step (reference prmf_runner.py:419-449).  Both passes over X are TMA X-stream
 // launches: skinny_tma_kernel<k,kTmaRS,EPI> at k <= 10, skinny_tma_gen_kernel<KT,FG,kTmaRS> at k > 10 (their _f32_
-// twins when X is stored in fp32, PRMF_X_F32), or tc_rowdot_kernel in tf32 mode.  step_path chooses which of the
-// sequences below a block of steps runs (StepPath).
+// twins when X is stored in fp32, PRMF_X_F32), or tc_rowdot_kernel in tf32 mode.  The four DFMA kernels wrap one device
+// body (skinny_tma_body, kernels.cuh) and one lookup picks among them (xstream_kernel).  step_path chooses which of
+// the sequences below a block of steps runs (StepPath).
 //
 // k <= 10, fp64 (fused tails, launch_xv_epi / launch_xtu_epi):
 //   skinny_tma_kernel<k,8,1>   A partials = Xt^T.V, then U <- U*A/(U.Gv+U) and Gu in the last CTA of each panel   (:420-422)
@@ -331,29 +332,28 @@ XStream pass2(const prmf_handle* h) {
             h->plan.pass2};
 }
 
-// the k <= 10 kernel of a pass with fused tail `epi`: call with KT = 1, it recurses to KT = k
-template <int KT>
-const void* tma_kernel(int k, bool f32, int epi) {
-    if constexpr (KT < 10)
-        if (k != KT) return tma_kernel<KT + 1>(k, f32, epi);
-    switch (epi) {
-        case 0: return f32 ? (const void*)skinny_tma_f32_kernel<KT, kTmaRS, 0> : (const void*)skinny_tma_kernel<KT, kTmaRS, 0>;
-        case 1: return f32 ? (const void*)skinny_tma_f32_kernel<KT, kTmaRS, 1> : (const void*)skinny_tma_kernel<KT, kTmaRS, 1>;
-        case 2: return f32 ? (const void*)skinny_tma_f32_kernel<KT, kTmaRS, 2> : (const void*)skinny_tma_kernel<KT, kTmaRS, 2>;
-        // no pack on fp32 storage: the f32 mode is single-rank (prmf_p2p_attach), the tf32 mode uses tc_rowdot_kernel
-        case 3: return f32 ? nullptr : (const void*)skinny_tma_kernel<KT, kTmaRS, 3>;
-    }
-    return nullptr;
-}
-
-// the k > 10 kernel of a pass (no fused tail)
-const void* gen_kernel(const prmf_xstream_plan& plan, bool f32) {
+// The X-stream kernel of a pass with fused tail `epi`, or nullptr: skinny_tma_kernel<k,kTmaRS,EPI> at k <= 10,
+// skinny_tma_gen_kernel<KT,FG,kTmaRS> (no fused tail) at the plan's (KT, FG) above, or their _f32_ twins.  It
+// instantiates exactly the kernels prmf_plan_xstream can select.  Call with K = 1: it recurses to K = k.
+template <int K = 1>
+const void* xstream_kernel(int k, const prmf_xstream_plan& plan, bool f32, int epi) {
+    if constexpr (K <= 10) {
+        if (k != K) return xstream_kernel<K + 1>(k, plan, f32, epi);
+        switch (epi) {
+            case 0: return f32 ? (const void*)skinny_tma_f32_kernel<K, kTmaRS, 0> : (const void*)skinny_tma_kernel<K, kTmaRS, 0>;
+            case 1: return f32 ? (const void*)skinny_tma_f32_kernel<K, kTmaRS, 1> : (const void*)skinny_tma_kernel<K, kTmaRS, 1>;
+            case 2: return f32 ? (const void*)skinny_tma_f32_kernel<K, kTmaRS, 2> : (const void*)skinny_tma_kernel<K, kTmaRS, 2>;
+            // no pack on fp32 storage: the f32 mode is single-rank (prmf_p2p_attach), the tf32 mode uses tc_rowdot_kernel
+            case 3: return f32 ? nullptr : (const void*)skinny_tma_kernel<K, kTmaRS, 3>;
+        }
+    } else if (epi == 0) {
 #define GEN_CASE(KT_, FG_)                                                                                   \
-    if (plan.kt == KT_ && plan.fg == FG_)                                                                    \
-        return f32 ? (const void*)skinny_tma_gen_f32_kernel<KT_, FG_, kTmaRS> : (const void*)skinny_tma_gen_kernel<KT_, FG_, kTmaRS>;
-    GEN_CASE(12, 1) GEN_CASE(16, 1) GEN_CASE(8, 2) GEN_CASE(12, 2) GEN_CASE(16, 2) GEN_CASE(8, 4) GEN_CASE(12, 4)
-    GEN_CASE(16, 4) GEN_CASE(8, 8) GEN_CASE(12, 8) GEN_CASE(16, 8)
+        if (plan.kt == KT_ && plan.fg == FG_)                                                                \
+            return f32 ? (const void*)skinny_tma_gen_f32_kernel<KT_, FG_, kTmaRS> : (const void*)skinny_tma_gen_kernel<KT_, FG_, kTmaRS>;
+        GEN_CASE(12, 1) GEN_CASE(16, 1) GEN_CASE(12, 2) GEN_CASE(16, 2) GEN_CASE(12, 4) GEN_CASE(16, 4) GEN_CASE(12, 8)
+        GEN_CASE(16, 8)
 #undef GEN_CASE
+    }
     return nullptr;
 }
 
@@ -369,31 +369,25 @@ EpiParams plain_epi(const prmf_handle* h) {
 }
 
 // Launches pass `x` with fused tail `epi` (0: none, 1: U update, 2: V update, 3: pack for the exchange over ranks).
-// The storage of M and k choose the kernel once: skinny_tma_kernel<k,kTmaRS,EPI> at k <= 10,
-// skinny_tma_gen_kernel<KT,FG,kTmaRS> (no fused tail) above, or their _f32_ twins.  The CTAs of a panel with a fused
-// tail wait for each other, so that launch is cooperative (all CTAs co-resident or the launch fails).
+// The storage of M, k and the plan choose the kernel once (xstream_kernel).  The CTAs of a panel with a fused tail wait
+// for each other, so that launch is cooperative (all CTAs co-resident or the launch fails).
 int launch_xstream(prmf_handle* h, const XStream& x, int epi, const EpiParams& ep_in) {
-    const bool gen = h->k > 10;
-    const void* fn = nullptr;
-    if (!gen) fn = tma_kernel<1>(h->k, x.f32, epi);
-    else if (epi == 0) fn = gen_kernel(h->plan, x.f32);
+    const void* fn = xstream_kernel(h->k, h->plan, x.f32, epi);
     if (!fn)
         return fail(h, PRMF_ERR_STATE, "no X-stream kernel for k=%d (KT=%d FG=%d), fused tail %d, %s storage", h->k,
                     (int)h->plan.kt, (int)h->plan.fg, epi, x.f32 ? "fp32" : "fp64");
     const prmf_xstream_pass& p = x.p;
     EpiParams ep = ep_in;
     int k = h->k, panel_w = (int)p.panel_w, stages = (int)h->plan.stages;     // the kernels' parameter types
-    void* tma_args[] = {(void*)&x.M, (void*)&x.ldm, (void*)&x.rows, (void*)&x.cols, (void*)&x.W, (void*)&panel_w,
-                        (void*)&p.rows_per_chunk, (void*)&stages, (void*)&x.out, (void*)&ep};
-    void* gen_args[] = {(void*)&x.M, (void*)&x.ldm, (void*)&x.rows, (void*)&x.cols, (void*)&x.W, (void*)&k,
-                        (void*)&panel_w, (void*)&p.rows_per_chunk, (void*)&stages, (void*)&x.out};
+    void* args[] = {(void*)&x.M, (void*)&x.ldm, (void*)&x.rows, (void*)&x.cols, (void*)&x.W, (void*)&k, (void*)&panel_w,
+                    (void*)&p.rows_per_chunk, (void*)&stages, (void*)&x.out, (void*)&ep};
     const dim3 grid(p.panels, p.chunks);
     const size_t smem = pass_smem(h, p);
     CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     if (epi != 0)
-        CU(cudaLaunchCooperativeKernel(fn, grid, dim3(kTmaThreads), tma_args, smem, h->stream));
+        CU(cudaLaunchCooperativeKernel(fn, grid, dim3(kTmaThreads), args, smem, h->stream));
     else   // as with <<<>>>, a failure is left for the caller's LAUNCH_CHECK
-        cudaLaunchKernel(fn, grid, dim3(kTmaThreads), gen ? gen_args : tma_args, smem, h->stream);
+        cudaLaunchKernel(fn, grid, dim3(kTmaThreads), args, smem, h->stream);
     return PRMF_OK;
 }
 
@@ -1378,7 +1372,7 @@ int prmf_plan_xstream(int64_t m_local, int64_t n, int k, int x_dtype, int sm_cou
         const int groups = (k + 15) / 16;
         p.fg = groups <= 1 ? 1 : groups <= 2 ? 2 : groups <= 4 ? 4 : 8;
         const int64_t per = (k + p.fg - 1) / p.fg;
-        p.kt = per <= 8 ? 8 : per <= 12 ? 12 : 16;
+        p.kt = per <= 12 ? 12 : 16;
     }
     const int64_t max_panel = 1024 / p.fg;
     auto plan = [&](int64_t cols, int64_t rows, prmf_xstream_pass& q) {

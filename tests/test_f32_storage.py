@@ -15,7 +15,7 @@ import pytest
 
 from conftest import load_golden
 from helpers import run_product, xstream_plan
-from test_sass import _longest_dfma_region, _sass_by_function
+from test_sass import _instantiations, _longest_dfma_region, _sass_by_function
 from test_xstream_exact import (K_GEN, K_SKINNY, RING_LIMIT, RS, SHAPES, _instance, _run_products, b200,  # noqa: F401
                                 fg_kt)
 
@@ -48,6 +48,9 @@ def test_f32_stream_kernels_sass():
             assert sum(op.startswith("DFMA") for op in loop) >= 8 * 4 * k, pattern
             assert not any(op.startswith(("LDL", "STL")) for op in loop), pattern
     gen = {(kt, fg) for fg, kt in (fg_kt(k) for k in range(11, 129))}
+    # the library holds the fp32 kernels the planner can select, and no others
+    assert _instantiations(funcs, "skinny_tma_f32_kernel") == {(k, 8, epi) for k in range(1, 11) for epi in range(3)}
+    assert _instantiations(funcs, "skinny_tma_gen_f32_kernel") == {(kt, fg, 8) for kt, fg in gen}
     for kt, fg in gen:
         pattern = "skinny_tma_gen_f32_kernelILi%dELi%dELi8E" % (kt, fg)
         names = [n for n in funcs if pattern in n]

@@ -9,6 +9,7 @@ import subprocess
 import pytest
 
 from conftest import ROOT
+from test_xstream_exact import fg_kt
 
 LIB = os.path.join(ROOT, "prmf_b200", "libprmf_b200.so")
 
@@ -78,3 +79,17 @@ def test_stream_kernel_main_loops_are_clean():
         moves = sum(op.startswith(("IMAD.MOV", "MOV")) for op in loop)
         assert moves <= n_dfma // 8, "register-move storm inside the main loop of %s: %d moves for %d DFMA" % (pattern, moves, n_dfma)
         assert sum(op.startswith("LDS.128") for op in loop) >= 8 * (2 + (k // 2 if k % 2 == 0 else 0)) - 16, pattern
+
+
+def _instantiations(funcs, kernel):
+    """The template arguments of every instantiation of the three-argument kernel template `kernel` in the library."""
+    found = (re.search(kernel + r"ILi(\d+)ELi(\d+)ELi(\d+)E", n) for n in funcs)
+    return {tuple(int(v) for v in m.groups()) for m in found if m}
+
+
+def test_stream_kernel_instantiations_are_the_reachable_set():
+    """The library holds the fp64 X-stream kernels the launch planner can select, and no others: skinny_tma_kernel at
+    k = 1..10 with every fused tail (EPI 0..3), skinny_tma_gen_kernel at every (KT, FG) that k = 11..128 reaches."""
+    funcs = _sass_by_function()
+    assert _instantiations(funcs, "skinny_tma_kernel") == {(k, 8, epi) for k in range(1, 11) for epi in range(4)}
+    assert _instantiations(funcs, "skinny_tma_gen_kernel") == {(kt, fg, 8) for fg, kt in (fg_kt(k) for k in range(11, 129))}

@@ -135,7 +135,7 @@ def test_general_k_choices_reach_idle_and_ragged_factor_groups():
     assert fg_kt(33) == (4, 12) and 3 * 12 >= 33
     assert fg_kt(66) == (8, 12) and sum(g * 12 >= 66 for g in range(8)) == 2
     assert fg_kt(98) == (8, 16) and 7 * 16 >= 98
-    # every (FG, KT) that k = 11..128 can select; the KT = 8 instantiations are compiled but unreachable
+    # every (FG, KT) that k = 11..128 can select: the library instantiates exactly these (tests/test_sass.py)
     assert {fg_kt(k) for k in range(11, 129)} == {(1, 12), (1, 16), (2, 12), (2, 16), (4, 12), (4, 16), (8, 12), (8, 16)}
 
 
